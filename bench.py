@@ -10,6 +10,7 @@ are all-gathered once per step (the only collective).
 
   python bench.py [--gpus N --steps K --warmup W]          our arm (CUDA engine through the C ABI)
   python bench.py --impl reference [...]                   the reference's CPU path (oracle port) on the host cores
+  python bench.py --dump-outputs DIR [...]                 also write the last timed step's spectra as DIR/<name>.npy
 """
 import argparse
 import json
@@ -30,6 +31,8 @@ UNIT = "pairs/s"
 WORKLOAD = "cfg2: mixed H2O+CO2+CH4+O3 gas cell, 0-3000 cm-1 @ 0.001 cm-1 per GPU (3.0M points, ~500k lines, W=5000)"
 SM_COUNT = 148
 SM_MAX_MHZ_DEFAULT = 1965.0
+DUMP_MAX_BYTES = 64_000_000
+DUMP_SAMPLE_SEED = 20240601
 
 
 def load_traffic(key):
@@ -189,6 +192,42 @@ def gather_parity(e, plan_chunks, nc, rank, world, dist):
     return "bitwise" if int(flag.item()) == 0 else "MISMATCH on %d rank(s)" % int(flag.item())
 
 
+def step_outputs(e, n_chunk, world, dist, range_min):
+    """What a caller of the timed step receives from its last run: the float32 radiance and transmittance spectra
+    (prb_atmosphere_read_f32), over the whole grid at N > 1 (every rank's chunk, in rank order).  Collective.
+
+    The transmittance is whole.  The radiance leaves out a grid point at 0 cm-1: Planck's law as the reference
+    evaluates it is 0/0 there, so the radiance is NaN by design (tests/test_gpu_parity.py holds the kernels to that)."""
+    rad, tr = np.empty(n_chunk, dtype=np.float32), np.empty(n_chunk, dtype=np.float32)
+    e.atmosphere_read_f32(rad, tr)
+    out = {"radiance": rad, "transmittance": tr}
+    if world > 1:
+        import torch
+        for name, mine in out.items():
+            every = torch.empty(world * n_chunk, dtype=torch.float32, device="cuda")
+            dist.all_gather_into_tensor(every, torch.from_numpy(mine).cuda())
+            out[name] = every.cpu().numpy()
+    if range_min == 0.0:
+        out["radiance"] = out["radiance"][1:]
+    return out
+
+
+def dump_outputs(directory, arrays, max_bytes=DUMP_MAX_BYTES):
+    """Write every array as directory/<name>.npy.  When they hold more than max_bytes together, each is cut to a sorted
+    sample of its positions drawn with a fixed seed: the sample depends only on the array's length (arrays of one
+    length share it), so runs with the same arguments write the same elements."""
+    total = sum(a.nbytes for a in arrays.values())
+    budget = max_bytes - 4096 * len(arrays)                   # room for the .npy headers
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        a = a.ravel()
+        if total > budget:
+            keep = a.size * budget // total
+            a = a[np.sort(np.random.default_rng(DUMP_SAMPLE_SEED).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 # ---------------------------------------------------------------------------------------------- CPU side
 def _oracle_window(args):
     """One bounded sample of the cfg2 workload on one core: the oracle's slice-add restatement of
@@ -294,7 +333,15 @@ def main():
     ap.add_argument("--no-farfield", action="store_true", help="skip the secondary far-field (PRB_K2_FARFIELD) measurements")
     ap.add_argument("--atm-layers", type=int, default=100)
     ap.add_argument("--atm-lines", type=int, default=5_000_000)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the transmittance and radiance spectra of the last timed step (the radiance above 0 cm-1, "
+                         "where Planck's law is 0/0) as DIR/<name>.npy (float32; a fixed seeded sample of positions when "
+                         "they exceed 64 MB), to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm keeps no outputs (it measures a rate on sample windows)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     out = claim_stdout()
     if args.impl == "reference":
@@ -392,6 +439,10 @@ def main():
         b.record(ext)
     sync_all()
     wall = time.perf_counter() - wall0
+    if args.dump_outputs:
+        outputs = step_outputs(e, n_chunk, world, dist, w["range_min"])   # before anything overwrites the result buffers
+        if rank == 0:
+            dump_outputs(args.dump_outputs, outputs)
     dev_ms = sum(a.elapsed_time(b) for a, b in evs)
     launches_per_step = e.atmosphere_launches()
     headline_parity = None

@@ -26,6 +26,7 @@ The harness never modifies reference files and never copies them.
 import contextlib
 import importlib
 import io
+import json
 import os
 import sys
 
@@ -148,6 +149,38 @@ class Reference:
         """BASE_RESOLUTION is a module constant (pyradUtilities.py:804-805); 0.001 grids
         require overriding it after import and dynamicResolution=False (SURVEY 8(a) a11)."""
         self.utils.BASE_RESOLUTION = res
+
+
+def reference_id_tables():
+    """MOLECULE_ID and HITRAN_GLOBAL_ISO as the dict literals of the reference source (pyradClasses.py:951-1022), read
+    without importing it; None where the sources are absent."""
+    path = os.path.join(REFERENCE_DIR, "pyradClasses.py")
+    if not os.path.isfile(path):
+        return None
+    with open(path) as f:
+        src = f.read()
+    ns = {}
+    for name in ("HITRAN_GLOBAL_ISO", "MOLECULE_ID"):
+        i = src.index(name + " = {")
+        depth, j = 0, i
+        while True:                                    # the dict literal: up to its matching brace
+            ch = src[j]
+            depth += ch == "{"
+            depth -= ch == "}"
+            j += 1
+            if ch == "}" and depth == 0:
+                break
+        exec(src[i:j], ns)
+    return {"MOLECULE_ID": ns["MOLECULE_ID"], "HITRAN_GLOBAL_ISO": ns["HITRAN_GLOBAL_ISO"]}
+
+
+def id_tables_json(tables):
+    """The layout of tests/golden/hitran_id_tables.json: the name table on one line, one isotopologue row per line."""
+    rows = list(tables["HITRAN_GLOBAL_ISO"].items())
+    out = ["{", ' "MOLECULE_ID": ' + json.dumps(tables["MOLECULE_ID"]) + ",", ' "HITRAN_GLOBAL_ISO": {']
+    for k, (mol, isos) in enumerate(rows):
+        out.append('  "%d": %s%s' % (mol, json.dumps({str(i): g for i, g in isos.items()}), "," if k < len(rows) - 1 else ""))
+    return "\n".join(out + [" }", "}"]) + "\n"
 
 
 @contextlib.contextmanager

@@ -259,11 +259,19 @@ def case_kat(name):
     print(name, {k: (v if np.ndim(v) == 0 else "...") for k, v in out.items()})
 
 
+def case_hitran_id_tables(name):
+    """MOLECULE_ID and HITRAN_GLOBAL_ISO read from the reference source's dict literals (pyradClasses.py:951-1022)."""
+    with open(os.path.join(OUT, name + ".json"), "w") as f:
+        f.write(rh.id_tables_json(rh.reference_id_tables()))
+    print(name, "written")
+
+
 if __name__ == "__main__":
     if not rh.available():
         raise SystemExit("the reference is not mounted at %s" % rh.REFERENCE_DIR)
     if len(sys.argv) > 1:                                          # regenerate only the named late additions
-        {"xsc_files": case_xsc_files, "cfg3_mini": case_cfg3_mini}[sys.argv[1]](sys.argv[1])
+        {"xsc_files": case_xsc_files, "cfg3_mini": case_cfg3_mini,
+         "hitran_id_tables": case_hitran_id_tables}[sys.argv[1]](sys.argv[1])
         raise SystemExit(0)
     case_kat("kat")
     case_gas_cell("cell_co2_1atm", ["co2"], [400e-6], 1500, 600.0, 700.0, 296, 1013.0, 10.0, 101)
@@ -276,3 +284,4 @@ if __name__ == "__main__":
     case_xsc("xsc_coarse_res", 0.05, 830.0, 860.0, 800.0, 900.0, 707)
     case_xsc_files("xsc_files")
     case_cfg3_mini("cfg3_mini")
+    case_hitran_id_tables("hitran_id_tables")

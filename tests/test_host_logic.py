@@ -156,8 +156,11 @@ def test_xsc_file_name_parser_matches_the_oracle():
 
 def test_hitran_id_tables_equal_the_reference_tables():
     """MOLECULE_ID and HITRAN_GLOBAL_ISO (pyradClasses.py:951-1022) carried in full: all 49 molecules and every
-    isotopologue row, compared with the reference source when it is mounted (the build container), and pinned by
-    count and spot values everywhere else."""
+    isotopologue row, pinned by count and spot values, equal to tests/golden/hitran_id_tables.json on every run, and
+    equal to the reference source's dict literals whenever the sources are present.  The committed JSON was written
+    from pyrad_b200/hitran_tables.py (the tables this test holds equal to the reference source); make_golden.py
+    hitran_id_tables rewrites it from the source itself."""
+    from oracle import ref_harness as rh
     from pyrad_b200 import classes as C
     assert len(C.MOLECULE_ID) == 49 and sorted(C.MOLECULE_ID.values()) == list(range(1, 50))
     assert set(C.HITRAN_GLOBAL_ISO) == set(range(1, 50))
@@ -165,23 +168,30 @@ def test_hitran_id_tables_equal_the_reference_tables():
     assert C.MOLECULE_ID["so2"] == 9 and C.MOLECULE_ID["nh3"] == 11 and C.MOLECULE_ID["cocl2"] == 49
     assert C.getGlobalIsotope(C.MOLECULE_ID["so2"], 2) == [42, 43]
     assert C.getGlobalIsotope(2, 12)[-1] == 122 and C.getGlobalIsotope(16, 2) == [19, 11]      # the reference's rows, sic
-    ref = "/root/reference/pyradClasses.py"
-    if os.path.isfile(ref):
-        src = open(ref).read()
-        ns = {}
-        for name in ("HITRAN_GLOBAL_ISO", "MOLECULE_ID"):
-            i = src.index(name + " = {")
-            depth, j = 0, i
-            while True:                                    # the dict literal: up to its matching brace
-                ch = src[j]
-                depth += ch == "{"
-                depth -= ch == "}"
-                j += 1
-                if ch == "}" and depth == 0:
-                    break
-            exec(src[i:j], ns)
-        assert ns["HITRAN_GLOBAL_ISO"] == C.HITRAN_GLOBAL_ISO
-        assert ns["MOLECULE_ID"] == C.MOLECULE_ID
+    with open(os.path.join(ROOT, "tests", "golden", "hitran_id_tables.json")) as f:
+        g = json.load(f)
+    assert g["MOLECULE_ID"] == C.MOLECULE_ID
+    assert {int(m): {int(i): gid for i, gid in row.items()} for m, row in g["HITRAN_GLOBAL_ISO"].items()} == C.HITRAN_GLOBAL_ISO
+    ref = rh.reference_id_tables()
+    if ref is not None:
+        assert ref["HITRAN_GLOBAL_ISO"] == C.HITRAN_GLOBAL_ISO
+        assert ref["MOLECULE_ID"] == C.MOLECULE_ID
+
+
+def test_reference_id_table_reader_and_golden_writer(tmp_path, monkeypatch):
+    """The reader make_golden.py and the test above use on pyradClasses.py (dict literals found by brace matching,
+    nested rows included) and the JSON layout of tests/golden/hitran_id_tables.json, on a stand-in source file."""
+    from oracle import ref_harness as rh
+    from pyrad_b200 import classes as C
+    monkeypatch.setattr(rh, "REFERENCE_DIR", str(tmp_path))
+    assert rh.reference_id_tables() is None
+    with open(str(tmp_path / "pyradClasses.py"), "w") as f:
+        f.write("import numpy as np\nx = {'a': {1: 2}}\nHITRAN_GLOBAL_ISO = %r\n\ndef f():\n    return {}\n\nMOLECULE_ID = %r\n"
+                % (C.HITRAN_GLOBAL_ISO, C.MOLECULE_ID))
+    tables = rh.reference_id_tables()
+    assert tables == {"MOLECULE_ID": C.MOLECULE_ID, "HITRAN_GLOBAL_ISO": C.HITRAN_GLOBAL_ISO}
+    with open(os.path.join(ROOT, "tests", "golden", "hitran_id_tables.json")) as f:
+        assert rh.id_tables_json(tables) == f.read()
 
 
 def test_isotope_lines_are_views_over_soa_columns(tmp_path, monkeypatch):

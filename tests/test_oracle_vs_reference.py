@@ -1,6 +1,8 @@
-"""CPU test, build container only: the oracle against the REAL reference executed live through
-oracle/ref_harness.py.  Skipped where /root/reference is absent (the GPU box); the committed golden vectors
-(tests/test_oracle.py) carry the same pin there."""
+"""CPU tests: the oracle against the REAL reference executed live through oracle/ref_harness.py, from the sources
+PYRAD_REFERENCE_DIR points to; skipped where they are absent.  Without them only part of this pin remains: the committed
+golden vectors (tests/test_oracle.py) hold the oracle to the reference's outputs on fixed gas cells, xsc tables, the xsc
+file utilities and known answers, but nothing stored covers what these tests check -- mergeArray on random ranges, the
+layer mutation model, the text readers and random cells at dynamic and 0.002 base resolution."""
 import numpy as np
 import pytest
 
