@@ -20,6 +20,7 @@
  *   pyradUtilities.py:173-189,421-448 HITRAN-online CSV rows -> line arrays -> prb_ingest_hitran_csv
  *   pyradClasses.py:409-428,26-29 line survey, integrateSpectrum            -> prb_line_survey, prb_integrate_spectrum
  *   (absent upstream, SURVEY 3.5) multi-layer fold of Layer.transmission   -> prb_atmosphere
+ *   (absent upstream) hemispheric fluxes, downwelling and slant radiances of the column -> prb_atmosphere_fluxes
  *
  * Conventions: every entry point is extern "C", returns int (0 = PRB_OK, < 0 = error) unless
  * noted, takes plain pointers and sizes.  Pointers named *_host / unmarked are caller-owned host
@@ -258,6 +259,18 @@ int prb_atmosphere_timing(prb_engine *e, float *k1_ms, float *k2_ms, float *k3_m
 int prb_atmosphere_layer_timing(prb_engine *e, int32_t n_layers, float *k1_ms, float *k2_ms);   /* per layer */
 int prb_atmosphere_kmatrix_dev(prb_engine *e, void **kmat_dev, int64_t *ld);                 /* float[L][ld] */
 int prb_atmosphere_launches(prb_engine *e);              /* kernels launched by the last prb_atmosphere */
+/* Hemispheric fluxes and slant radiances of the last column (prb_atmosphere or prb_gas_cell_host), on the owned chunk,
+ * from its device-resident k matrix.  For every node i of an angular quadrature (mu[i] in (0, 1], weight[i] > 0,
+ * 1 <= n_mu <= 4) the fold I <- T I + (1 - T) B(nu, t[l]), T = exp(-k_l depth_l / mu[i]), runs up from B(nu, t_surface)
+ * and down from 0 (no cosmic background, no solar source).  Level j is the boundary below layer j: 0 = surface, L = top.
+ * flux_up / flux_down: L+1 doubles each, F[j] = 2 pi sum_i weight[i] mu[i] sum_nu I_i(nu, level j) res over this chunk
+ * (NaN -- the 0 cm^-1 point -- counts as 0, as in integrateSpectrum, and so does +-inf: next to 0 cm^-1 the reference's
+ * negative Doppler widths can make k < 0 and the FP32 transmittance overflow; with wavenumber chunks the ranks' values add up).
+ * rad_up_top / rad_down_surface: n_mu x chunk floats each, row-major: the radiance leaving the top along mu[i], and the
+ * radiance reaching the surface along mu[i].  Any output may be NULL.  Planck is evaluated as in the column's fold, so
+ * mu = 1 reproduces prb_atmosphere's radiance bit for bit.  Under a peer connection the call stays local. */
+int prb_atmosphere_fluxes(prb_engine *e, int32_t n_mu, const double *mu, const double *weight,
+                          double *flux_up, double *flux_down, float *rad_up_top, float *rad_down_surface);
 int prb_set_option(prb_engine *e, int option, int64_t value);
 
 /* ---- section 8(f) rows beside the hot path -------------------------------------------------------

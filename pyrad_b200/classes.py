@@ -866,6 +866,34 @@ class Atmosphere(list):
         without one host round trip per layer and isotope; needs layers that share range and base resolution and carry
         the same line-by-line molecules in the same order.  xsc molecules (up to eight distinct tables over the column)
         stay resident on the device and enter every layer's k(nu) inside the line-sum kernel (prb_xsc_resident)."""
+        return self._column(surfaceTemperature, lambda e: e.atmosphere_read())
+
+    def columnFluxes(self, surfaceTemperature, mu=None, weights=None):
+        """Hemispheric fluxes, heating rates and slant radiances of the column (prb_atmosphere, then
+        prb_atmosphere_fluxes on its device-resident k matrix; same requirements on the layers as columnSpectrum).
+        For every node mu_i of the angular quadrature (default: 3-node Gauss-Legendre on [0, 1]; at most 4 nodes) the
+        fold runs up from B(nu, surfaceTemperature) and down from 0 (no cosmic background, no sun) with
+        T = exp(-k_l depth_l / mu_i); level j is the boundary below layer j (0 = surface, len(self) = top), and
+        F[j] = 2 pi sum_i w_i mu_i integrateSpectrum(I_i(level j), 1, res).  A column with opaque bands is not
+        isotropic, so F_up at the top differs from the pi x nadir radiance of integrateSpectrum(columnSpectrum(...)[0]).
+        Returns a dict: flux_up, flux_down, net (= up - down) per level in W m-2; heating_rate per layer in K/day
+        (heatingRate); rad_up_top and rad_down_surface, float32 (n_mu, n_points) -- the radiance leaving the top and
+        reaching the surface along every mu_i; mu and weights."""
+        if mu is None and weights is None:
+            x, w = np.polynomial.legendre.leggauss(3)
+            mu, weights = (x + 1) / 2, w / 2
+        mu, weights = np.atleast_1d(np.asarray(mu, dtype=np.float64)), np.atleast_1d(np.asarray(weights, dtype=np.float64))
+        if mu.shape != weights.shape or not 1 <= mu.size <= 4:
+            raise ValueError("columnFluxes needs 1 to 4 quadrature nodes, as many weights as mu")
+        up, down, ru, rd = self._column(surfaceTemperature, lambda e: e.atmosphere_fluxes(mu, weights, rows=True))
+        layers = list(self)
+        return {"flux_up": up, "flux_down": down, "net": up - down,
+                "heating_rate": heatingRate(up, down, [l.depth for l in layers], [l.T for l in layers],
+                                            [l.P for l in layers]),
+                "rad_up_top": ru, "rad_down_surface": rd, "mu": mu, "weights": weights}
+
+    def _column(self, surfaceTemperature, result):
+        """Run the column on the device (prb_atmosphere) and return result(engine) while its state is in place."""
         layers = list(self)
         if not layers:
             raise ValueError("atmosphere has no layers")
@@ -923,10 +951,30 @@ class Atmosphere(list):
             e.atmosphere([l.depth for l in layers], [l.T for l in layers], [l.P for l in layers], conc,
                          [iso.molmass for iso in isos] or [1.0], q_t, [iso.q296 for iso in isos] or [1.0], window,
                          surfaceTemperature, ref.rangeMax)
-            return e.atmosphere_read()
+            return result(e)
         finally:
             e.xsc_clear()
             e.set_layer_line_range()
+
+
+#: dry air: molar mass (kg/mol), isobaric specific heat (J kg-1 K-1); molar gas constant (J mol-1 K-1, CODATA 2018 exact)
+M_DRY_AIR = 0.0289647
+CP_DRY_AIR = 1004.64
+R_GAS = 8.314462618
+
+
+def heatingRate(flux_up, flux_down, depth_cm, T, P):
+    """Radiative heating rate of every layer in K/day from the level fluxes (L+1 values, level 0 = surface, W m-2):
+    Q_l = -(F_net[l+1] - F_net[l]) / (rho_l c_p dz_l) * 86400 s/day with F_net = F_up - F_down, the layer's thickness
+    dz_l = depth_cm / 100 m and its density rho_l = 100 P_l M_d / (R T_l) (ideal dry air; P in hPa as Layer holds it,
+    T in K).  Constants: M_DRY_AIR, CP_DRY_AIR, R_GAS above.  Negative values are cooling."""
+    net = np.asarray(flux_up, dtype=np.float64) - np.asarray(flux_down, dtype=np.float64)
+    T, P = np.asarray(T, dtype=np.float64), np.asarray(P, dtype=np.float64)
+    dz = np.asarray(depth_cm, dtype=np.float64) / 100
+    if net.shape != (T.size + 1,) or T.shape != P.shape or dz.shape != T.shape:
+        raise ValueError("heatingRate needs L+1 level fluxes and L depths, temperatures and pressures")
+    rho = 100 * P * M_DRY_AIR / (R_GAS * T)
+    return -(net[1:] - net[:-1]) / (rho * CP_DRY_AIR * dz) * 86400
 
 
 def getGlobalIsotope(ID, isotopeDepth):

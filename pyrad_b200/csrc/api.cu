@@ -210,6 +210,13 @@ struct prb_engine {
     DevBuf<FoldLayer> fold;
     int64_t kmat_ld = 0;
     int atm_layers = 0;
+    // the last column's layer constants and fold policy, for prb_atmosphere_fluxes
+    std::vector<double> atm_depth, atm_t;
+    double atm_t_surface = 0, atm_range_max = 0;
+    float atm_nu_interp_min = 1e30f;                  // Planck interpolated above this (k3_fold_tma), else per point
+    DevBuf<FluxLayer> flux_layers;
+    DevBuf<double> flux_part, flux_out;
+    DevBuf<float> flux_rows;
     // optional stage timing of prb_atmosphere (CUDA events on the engine stream)
     bool timing = false;
     std::vector<cudaEvent_t> ev;
@@ -304,6 +311,7 @@ extern "C" int prb_destroy(prb_engine *e) {
     e->out64.release(); e->scratch_a.release(); e->scratch_b.release(); e->scratch_c.release();
     e->scratch_d.release(); e->scratch_w.release();
     e->kmat.release(); e->rad.release(); e->trans.release(); e->fold.release();
+    e->flux_layers.release(); e->flux_part.release(); e->flux_out.release(); e->flux_rows.release();
     e->k2tab.release(); e->ring_d.release(); e->peer_err.release();
     if (e->blk_h) cudaFreeHost(e->blk_h);
     if (e->read_stage) cudaFreeHost(e->read_stage);
@@ -1491,6 +1499,11 @@ static int atmosphere_impl(prb_engine *e, int32_t n_layers, int32_t n_groups, co
         CK(cudaMemsetAsync(e->kmat.p, 0, sizeof(float) * e->kmat_ld * n_layers, e->stream));
         e->atm_layers = n_layers;
     }
+    e->atm_depth.assign(depth_cm, depth_cm + n_layers);
+    e->atm_t.assign(t_layer, t_layer + n_layers);
+    e->atm_t_surface = t_surface;
+    e->atm_range_max = range_max;
+    e->atm_nu_interp_min = 1e30f;                                // per-point Planck unless k3_fold_tma runs below
 
     // Launch plan.  Layers are processed widest window first, in batches of `slots` layers whose records are
     // resident together (36 B per line per layer): ONE K1 launch per batch, then ONE K2 launch per kernel class
@@ -1663,6 +1676,7 @@ static int atmosphere_impl(prb_engine *e, int32_t n_layers, int32_t n_groups, co
             for (int l = 0; l < n_layers; ++l) { t_max = std::max(t_max, t_layer[l]); t_min = std::min(t_min, t_layer[l]); }
             double nu_min = std::max(3 * dx * std::sqrt(6.0 / 8e-7), 0.26 * t_max / c2);
             if ((3 * dx) * (3 * dx) / 8 * (c2 / t_min) * (c2 / t_min) > 1e-7) nu_min = 1e30;      // grid too coarse: never
+            e->atm_nu_interp_min = (float)nu_min;
             k3_fold_tma<<<grid, K3T_THREADS, sizeof(K3TSmem), e->stream>>>(e->kmat.p, e->kmat_ld, n_layers, fold_dev, nc,
                                                                           e->i_begin, e->n_total, e->range_min, dx, range_max,
                                                                           (float)(c2 / t_surface), (float)nu_min, dst);
@@ -1778,6 +1792,95 @@ extern "C" int prb_atmosphere_read_f32(prb_engine *e, float *radiance_host, floa
     if (radiance_host) CK(cudaMemcpyAsync(radiance_host, e->res_rad, sizeof(float) * nc, cudaMemcpyDeviceToHost, e->stream));
     if (transmittance_host)
         CK(cudaMemcpyAsync(transmittance_host, e->res_trans, sizeof(float) * nc, cudaMemcpyDeviceToHost, e->stream));
+    CK(cudaStreamSynchronize(e->stream));
+    return PRB_OK;
+}
+
+// One flux pass (k3_flux_tma) over the resident k matrix; its per-CTA level sums go to a.part.
+template <int NMU, bool DOWN>
+static cudaError_t launch_flux(prb_engine *e, int grid, size_t smem, double dx, const K3FArgs &a) {
+    const auto fn = k3_flux_tma<NMU, DOWN>;
+    cudaError_t ce = cudaFuncSetAttribute((const void *)fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (ce != cudaSuccess) return ce;
+    const double c2 = 100 * hPlanck * cLight / kBoltz;
+    fn<<<grid, K3T_THREADS, smem, e->stream>>>(e->kmat.p, e->kmat_ld, e->atm_layers, e->flux_layers.p, chunk_len(e),
+                                               e->i_begin, e->n_total, e->range_min, dx, e->atm_range_max,
+                                               (float)(c2 / e->atm_t_surface), e->atm_nu_interp_min, a);
+    return cudaGetLastError();
+}
+
+template <int NMU>
+static cudaError_t launch_flux_pair(prb_engine *e, int grid, size_t smem, double dx, const K3FArgs &up, const K3FArgs &down) {
+    cudaError_t ce = launch_flux<NMU, false>(e, grid, smem, dx, up);
+    return ce != cudaSuccess ? ce : launch_flux<NMU, true>(e, grid, smem, dx, down);
+}
+
+extern "C" int prb_atmosphere_fluxes(prb_engine *e, int32_t n_mu, const double *mu, const double *weight, double *flux_up,
+                                     double *flux_down, float *rad_up_top, float *rad_down_surface) {
+    if (!e || !e->atm_layers) return fail(PRB_ERR_STATE, "prb_atmosphere_fluxes: run prb_atmosphere first");
+    if (n_mu < 1 || n_mu > 4 || !mu || !weight) return fail(PRB_ERR_ARG, "prb_atmosphere_fluxes: need 1 <= n_mu <= 4, mu and weight");
+    for (int i = 0; i < n_mu; ++i)
+        if (!(mu[i] > 0 && mu[i] <= 1) || !(weight[i] > 0 && std::isfinite(weight[i])))
+            return fail(PRB_ERR_ARG, "prb_atmosphere_fluxes: every mu must lie in (0, 1] and every weight be finite and > 0");
+    CK(cudaSetDevice(e->device));
+    const int L = e->atm_layers, n_levels = L + 1;
+    const int64_t nc = chunk_len(e);
+    const size_t smem = k3f_smem_bytes(L);
+    if (smem > (size_t)e->prop.sharedMemPerBlockOptin)
+        return fail(PRB_ERR_RANGE, "prb_atmosphere_fluxes: too many layers for the per-level accumulators in shared memory");
+    if (nc == 0) {                                              // an empty chunk contributes nothing
+        if (flux_up) std::fill(flux_up, flux_up + n_levels, 0.0);
+        if (flux_down) std::fill(flux_down, flux_down + n_levels, 0.0);
+        return PRB_OK;
+    }
+    // per layer: c2 / T_l and -depth_l log2(e) / mu_i, rounded as the fold rounds them (mu = 1 gives its very constants)
+    const double c2 = 100 * hPlanck * cLight / kBoltz;
+    std::vector<FluxLayer> hl(L);
+    for (int l = 0; l < L; ++l) {
+        hl[l].c2_over_t = (float)(c2 / e->atm_t[l]);
+        for (int i = 0; i < 4; ++i) hl[l].nd[i] = i < n_mu ? (float)(-e->atm_depth[l] * 1.4426950408889634 / mu[i]) : 0.f;
+    }
+    const int64_t n_strips = (nc + K3T_STRIP - 1) / K3T_STRIP;
+    const int grid = (int)std::min<int64_t>(n_strips, k3f_minb(n_mu) * (int64_t)e->prop.multiProcessorCount);
+    const bool rows = rad_up_top || rad_down_surface;
+    CK(e->flux_layers.ensure(L));
+    CK(e->flux_part.ensure((size_t)2 * grid * n_levels));
+    CK(e->flux_out.ensure((size_t)2 * n_levels));
+    if (rows) CK(e->flux_rows.ensure((size_t)2 * 4 * e->kmat_ld));
+    CK(cudaMemcpyAsync(e->flux_layers.p, hl.data(), sizeof(FluxLayer) * L, cudaMemcpyHostToDevice, e->stream));
+    K3FArgs up{}, down{};
+    for (int i = 0; i < n_mu; ++i) up.wmu[i] = down.wmu[i] = (float)(weight[i] * mu[i]);
+    up.ld_rows = down.ld_rows = e->kmat_ld;
+    up.rows = rows ? e->flux_rows.p : nullptr;
+    down.rows = rows ? e->flux_rows.p + (size_t)4 * e->kmat_ld : nullptr;
+    up.part = e->flux_part.p;
+    down.part = e->flux_part.p + (size_t)grid * n_levels;
+    const double dx = e->n_total > 1 ? (e->atm_range_max - e->range_min) / (double)(e->n_total - 1) : 0.0;
+    cudaError_t ce;
+    switch (n_mu) {
+        case 1: ce = launch_flux_pair<1>(e, grid, smem, dx, up, down); break;
+        case 2: ce = launch_flux_pair<2>(e, grid, smem, dx, up, down); break;
+        case 3: ce = launch_flux_pair<3>(e, grid, smem, dx, up, down); break;
+        default: ce = launch_flux_pair<4>(e, grid, smem, dx, up, down); break;
+    }
+    if (ce != cudaSuccess) return fail(PRB_ERR_CUDA, std::string("k3_flux_tma launch failed: ") + cudaGetErrorString(ce));
+    // F[j] = 2 pi sum_i w_i mu_i sum_nu I_i(nu, j) res  (integrateSpectrum's res and NaN rule, pyradClasses.py:26-29)
+    const double scale = 2 * 3.141592653589793 * e->res;
+    const unsigned sum_blocks = (unsigned)((n_levels + 255) / 256);
+    k3_flux_sum<<<sum_blocks, 256, 0, e->stream>>>(up.part, grid, n_levels, scale, e->flux_out.p);
+    k3_flux_sum<<<sum_blocks, 256, 0, e->stream>>>(down.part, grid, n_levels, scale, e->flux_out.p + n_levels);
+    CK(cudaGetLastError());
+    if (flux_up) CK(cudaMemcpyAsync(flux_up, e->flux_out.p, sizeof(double) * n_levels, cudaMemcpyDeviceToHost, e->stream));
+    if (flux_down)
+        CK(cudaMemcpyAsync(flux_down, e->flux_out.p + n_levels, sizeof(double) * n_levels, cudaMemcpyDeviceToHost, e->stream));
+    for (int i = 0; i < n_mu; ++i) {
+        if (rad_up_top)
+            CK(cudaMemcpyAsync(rad_up_top + (size_t)i * nc, up.rows + (size_t)i * e->kmat_ld, sizeof(float) * nc,
+                               cudaMemcpyDeviceToHost, e->stream));
+        if (rad_down_surface)
+            CK(cudaMemcpyAsync(rad_down_surface + (size_t)i * nc, down.rows + (size_t)i * e->kmat_ld, sizeof(float) * nc,
+                               cudaMemcpyDeviceToHost, e->stream));
+    }
     CK(cudaStreamSynchronize(e->stream));
     return PRB_OK;
 }

@@ -283,6 +283,31 @@ constexpr int K3T_LAYERS = PRB_K3T_LAYERS;             // rows per ring slot
 constexpr int K3T_SLOTS = PRB_K3T_SLOTS;
 constexpr int K3T_MINB = PRB_K3T_MINB;                 // resident CTAs per SM the shared memory is sized for
 
+// B(nu, T_l) at a thread's four consecutive points for one layer.  interp: evaluated at the first and last point only,
+// the two between by linear interpolation (relative error < 1e-7 above the host's nu_interp_min, chosen from the grid
+// spacing; one path decision per thread instead of per point); otherwise per point.  Shared by k3_fold_tma and
+// k3_flux_tma, so a flux pass with mu = 1 reproduces the fold bit for bit.
+__device__ __forceinline__ void k3_planck4(const float (&nu)[4], const float (&a3)[4], float c2_over_t, bool interp,
+                                           float (&b)[4]) {
+    if (interp) {
+        const float xa = c2_over_t * nu[0], xb = c2_over_t * nu[3];
+        float ba, bb;
+        if (xa > 8.5f) {
+            const float ya = k3_ex2(xa * -1.4426950408889634f), yb = k3_ex2(xb * -1.4426950408889634f);
+            ba = a3[0] * fmaf(ya, ya, ya);
+            bb = a3[3] * fmaf(yb, yb, yb);
+        } else {
+            ba = a3[0] * k3_rcp(k3_ex2(xa * 1.4426950408889634f) - 1.0f);
+            bb = a3[3] * k3_rcp(k3_ex2(xb * 1.4426950408889634f) - 1.0f);
+        }
+        const float db = bb - ba;
+        b[0] = ba; b[1] = fmaf(db, 1.0f / 3.0f, ba); b[2] = fmaf(db, 2.0f / 3.0f, ba); b[3] = bb;
+    } else {
+#pragma unroll
+        for (int q = 0; q < 4; ++q) b[q] = planck_f32(a3[q], c2_over_t * nu[q]);
+    }
+}
+
 struct K3TSmem {
     float k[K3T_SLOTS][K3T_LAYERS][K3T_STRIP];
     float2 tau[4][K3T_THREADS];            // (hi, lo) optical-depth accumulators of every thread's four points
@@ -363,26 +388,7 @@ k3_fold_tma(const float *__restrict__ kmat, int64_t ld, int n_layers, const Fold
                     const FoldLayer fl = layers[g * K3T_LAYERS + r];
                     const float kk[4] = {k4.x, k4.y, k4.z, k4.w};
                     float b[4];
-                    if (interp) {
-                        // B(nu, T_l) at the thread's first and last point, the two between by linear interpolation
-                        // (relative error < 1e-7 above nu_interp_min, chosen by the host from the grid spacing); one
-                        // path decision per thread instead of per point
-                        const float xa = fl.c2_over_t * nu[0], xb = fl.c2_over_t * nu[3];
-                        float ba, bb;
-                        if (xa > 8.5f) {
-                            const float ya = k3_ex2(xa * -1.4426950408889634f), yb = k3_ex2(xb * -1.4426950408889634f);
-                            ba = a3[0] * fmaf(ya, ya, ya);
-                            bb = a3[3] * fmaf(yb, yb, yb);
-                        } else {
-                            ba = a3[0] * k3_rcp(k3_ex2(xa * 1.4426950408889634f) - 1.0f);
-                            bb = a3[3] * k3_rcp(k3_ex2(xb * 1.4426950408889634f) - 1.0f);
-                        }
-                        const float db = bb - ba;
-                        b[0] = ba; b[1] = fmaf(db, 1.0f / 3.0f, ba); b[2] = fmaf(db, 2.0f / 3.0f, ba); b[3] = bb;
-                    } else {
-#pragma unroll
-                        for (int q = 0; q < 4; ++q) b[q] = planck_f32(a3[q], fl.c2_over_t * nu[q]);
-                    }
+                    k3_planck4(nu, a3, fl.c2_over_t, interp, b);
                     {
                         const float2 nd = make_float2(fl.neg_depth_log2e, fl.neg_depth_log2e);
                         const float2 e01 = __fmul2_rn(make_float2(kk[0], kk[1]), nd), e23 = __fmul2_rn(make_float2(kk[2], kk[3]), nd);
@@ -418,6 +424,187 @@ k3_fold_tma(const float *__restrict__ kmat, int64_t ld, int n_layers, const Fold
                 }
             }
         }
+    }
+}
+
+// ---- flux fold: hemispheric fluxes and slant radiances over the resident k matrix --------------------------------
+// For every node mu_i (NMU of them, 1..4) of a caller's angular quadrature, the fold I <- T I + (1 - T) B(nu, T_l) with
+// T = exp(-k_l depth_l / mu_i) runs upward from I = B(nu, T_surface) at level 0 (DOWN = false), or downward from I = 0 at
+// level L (DOWN = true).  Level j is the boundary below layer j: 0 = surface, L = top of the atmosphere.  The strips, the
+// TMA ring and the Planck policy are k3_fold_tma's; B(nu, T_l) is evaluated once per point and layer and serves every
+// node.  At each level a thread forms sum_i w_i mu_i sum_q I_i(nu_q) over its four points in FP32 (a value that is not
+// finite counts as 0, see `partial`), a fixed xor-butterfly adds the warp's 32 values, and lane 0 adds the result into a per-(warp,
+// level) FP64 accumulator in shared memory that lives for all of the CTA's strips.  The CTA then writes its per-level
+// partials (warps in order) and k3_flux_sum adds them in CTA order: the result is deterministic, with no atomics.
+struct FluxLayer {
+    float c2_over_t;         // 100 h c / kB / T_layer
+    float nd[4];             // -depth log2(e) / mu_i: T_i = exp2(k * nd[i])
+};
+
+struct K3FArgs {
+    float wmu[4];            // w_i mu_i
+    float *rows;             // [NMU][ld_rows]: radiance leaving the column at the last level of the pass (NULL: none)
+    int64_t ld_rows;
+    double *part;            // [gridDim.x][n_layers + 1] per-CTA level sums
+};
+
+constexpr int K3F_WARPS = K3T_THREADS / 32;
+struct K3FSmem {
+    float k[K3T_SLOTS][K3T_LAYERS][K3T_STRIP];
+    uint64_t full[K3T_SLOTS];
+};                                                     // followed by double acc[K3F_WARPS][n_layers + 1]
+
+// Resident CTAs per SM, from the register count without spills (-Xptxas -v, 256 threads): one and two nodes fit 64
+// registers (4 CTAs; one node spills at the 48 of 5 CTAs), three and four nodes take 78-80 (3 CTAs).
+__host__ __device__ constexpr int k3f_minb(int nmu) { return nmu <= 2 ? 4 : 3; }
+
+__host__ __device__ constexpr size_t k3f_smem_bytes(int n_layers) {
+    return sizeof(K3FSmem) + sizeof(double) * K3F_WARPS * (size_t)(n_layers + 1);
+}
+
+template <int NMU, bool DOWN>
+__global__ void __launch_bounds__(K3T_THREADS, k3f_minb(NMU))
+k3_flux_tma(const float *__restrict__ kmat, int64_t ld, int n_layers, const FluxLayer *__restrict__ layers,
+            int64_t n_chunk, int64_t i_begin, int64_t n_total, double x0, double dx, double x_last,
+            float c2_over_tsurf, float nu_interp_min, const K3FArgs a) {
+    extern __shared__ __align__(128) unsigned char k3_smem_raw[];
+    K3FSmem &sm = *reinterpret_cast<K3FSmem *>(k3_smem_raw);
+    double *acc = reinterpret_cast<double *>(k3_smem_raw + sizeof(K3FSmem));
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int n_levels = n_layers + 1;
+    const int64_t n_strips = (n_chunk + K3T_STRIP - 1) / K3T_STRIP;
+    const int groups = (n_layers + K3T_LAYERS - 1) / K3T_LAYERS;
+    const int64_t my_strips = blockIdx.x < n_strips ? (n_strips - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
+    const int64_t n_steps = my_strips * groups;
+    for (int j = tid; j < K3F_WARPS * n_levels; j += K3T_THREADS) acc[j] = 0.0;
+    if (tid == 0) {
+        for (int s = 0; s < K3T_SLOTS; ++s) mbar_init(&sm.full[s], 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    }
+    __syncthreads();
+    // step s of the CTA covers row group s % groups of its strip, counted from the top for the downward pass
+    auto group_of = [&](int64_t step) { const int g = (int)(step % groups); return DOWN ? groups - 1 - g : g; };
+    auto issue = [&](int64_t step) {                   // thread 0 only
+        const int slot = (int)(step % K3T_SLOTS);
+        const int64_t strip = blockIdx.x + (step / groups) * gridDim.x;
+        const int g = group_of(step);
+        const int64_t p0 = strip * K3T_STRIP;
+        const int64_t pts = min((int64_t)K3T_STRIP, ((n_chunk - p0) + 3) & ~int64_t(3));   // rows are padded to 4 floats
+        const int rows = min(K3T_LAYERS, n_layers - g * K3T_LAYERS);
+        mbar_expect_tx(&sm.full[slot], (uint32_t)(rows * pts * 4));
+        for (int r = 0; r < rows; ++r)
+            tma_bulk_g2s(sm.k[slot][r], kmat + (int64_t)(g * K3T_LAYERS + r) * ld + p0, (uint32_t)(pts * 4), &sm.full[slot]);
+    };
+    if (tid == 0)
+        for (int64_t s = 0; s < min(n_steps, (int64_t)(K3T_SLOTS - 1)); ++s) issue(s);
+
+    float nu[4], a3[4], rad[NMU][4];
+    bool interp = false;
+    int n_valid = 0;                                   // of the thread's four points, those inside the chunk
+    int64_t i0 = 0;
+    // sum_i w_i mu_i sum_q I_i(nu_q) over the thread's points inside the chunk.  A value that is not finite counts as 0:
+    // the NaN of the 0 cm^-1 point, and the +-inf of the few points next to it where the reference's negative Doppler
+    // widths make k < 0 and T = exp(-k u) overflows FP32.  The plain sum is checked once; the masked sum only runs for a
+    // ragged last strip or when the plain sum met such a value.
+    auto partial = [&]() {
+        float s = 0.f;
+        if (n_valid == 4) {
+#pragma unroll
+            for (int i = 0; i < NMU; ++i) {
+                const float2 p = __fadd2_rn(make_float2(rad[i][0], rad[i][1]), make_float2(rad[i][2], rad[i][3]));
+                s = fmaf(a.wmu[i], p.x + p.y, s);
+            }
+        }
+        if (n_valid < 4 || !isfinite(s)) {
+            s = 0.f;
+#pragma unroll
+            for (int i = 0; i < NMU; ++i) {
+                float t = 0.f;
+#pragma unroll
+                for (int q = 0; q < 4; ++q)
+                    if (q < n_valid && isfinite(rad[i][q])) t += rad[i][q];
+                s = fmaf(a.wmu[i], t, s);
+            }
+        }
+        return s;
+    };
+    auto level_add = [&](float v, int level) {         // every lane of the warp takes part
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+        if (lane == 0) acc[warp * n_levels + level] += (double)v;
+    };
+    for (int64_t step = 0; step < n_steps; ++step) {
+        const int slot = (int)(step % K3T_SLOTS);
+        const int g = group_of(step);
+        if (step % groups == 0) {                      // a new strip: the boundary radiance of the pass
+            const int64_t strip = blockIdx.x + (step / groups) * gridDim.x;
+            i0 = strip * K3T_STRIP + 4 * tid;
+            n_valid = (int)max((int64_t)0, min((int64_t)4, n_chunk - i0));
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+                const double x = axis_value(i_begin + i0 + q, n_total, x0, dx, x_last);
+                nu[q] = (float)x;
+                a3[q] = (float)(2E8 * hPlanck * (cLight * cLight) * (x * x * x));
+                const float r0 = DOWN ? 0.f : planck_f32(a3[q], c2_over_tsurf * nu[q]);
+#pragma unroll
+                for (int i = 0; i < NMU; ++i) rad[i][q] = r0;
+            }
+            interp = nu[0] >= nu_interp_min;
+            if (!DOWN) level_add(partial(), 0);        // (the downward pass starts from 0 at level L)
+        }
+        if (tid == 0 && step + K3T_SLOTS - 1 < n_steps) issue(step + K3T_SLOTS - 1);
+        mbar_wait(&sm.full[slot], (uint32_t)((step / K3T_SLOTS) & 1));
+        const int rows = min(K3T_LAYERS, n_layers - g * K3T_LAYERS);
+#pragma unroll
+        for (int rr = 0; rr < K3T_LAYERS; ++rr) {
+            if (rr < rows) {
+                const int r = DOWN ? rows - 1 - rr : rr;
+                const int l = g * K3T_LAYERS + r;
+                const float4 k4 = *reinterpret_cast<const float4 *>(&sm.k[slot][r][4 * tid]);
+                const FluxLayer fl = layers[l];
+                float b[4];
+                k3_planck4(nu, a3, fl.c2_over_t, interp, b);
+                const float2 b01 = make_float2(b[0], b[1]), b23 = make_float2(b[2], b[3]);
+#pragma unroll
+                for (int i = 0; i < NMU; ++i) {
+                    const float2 nd = make_float2(fl.nd[i], fl.nd[i]);
+                    const float2 e01 = __fmul2_rn(make_float2(k4.x, k4.y), nd), e23 = __fmul2_rn(make_float2(k4.z, k4.w), nd);
+                    const float2 r01 = k3_fold_step2(make_float2(rad[i][0], rad[i][1]), e01, b01);
+                    const float2 r23 = k3_fold_step2(make_float2(rad[i][2], rad[i][3]), e23, b23);
+                    rad[i][0] = r01.x; rad[i][1] = r01.y; rad[i][2] = r23.x; rad[i][3] = r23.y;
+                }
+                level_add(partial(), DOWN ? l : l + 1);
+            }
+        }
+        __syncthreads();                               // every thread is done with this slot: it may be refilled
+        if (step % groups == groups - 1 && a.rows && n_valid > 0) {
+#pragma unroll
+            for (int i = 0; i < NMU; ++i) {
+                float *dst = a.rows + (int64_t)i * a.ld_rows + i0;
+                if (n_valid == 4) *reinterpret_cast<float4 *>(dst) = make_float4(rad[i][0], rad[i][1], rad[i][2], rad[i][3]);
+                else
+#pragma unroll
+                    for (int q = 0; q < 4; ++q)
+                        if (q < n_valid) dst[q] = rad[i][q];
+            }
+        }
+    }
+    __syncthreads();
+    for (int j = tid; j < n_levels; j += K3T_THREADS) {
+        double s = 0.0;
+        for (int w = 0; w < K3F_WARPS; ++w) s += acc[w * n_levels + j];
+        a.part[(int64_t)blockIdx.x * n_levels + j] = s;
+    }
+}
+
+// out[j] = scale * sum over the n_parts CTAs, in CTA order, of their level-j partials.
+__global__ void __launch_bounds__(256)
+k3_flux_sum(const double *__restrict__ part, int n_parts, int n_levels, double scale, double *__restrict__ out) {
+    for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < n_levels; j += gridDim.x * blockDim.x) {
+        double s = 0.0;
+        for (int b = 0; b < n_parts; ++b) s += part[(int64_t)b * n_levels + j];
+        out[j] = s * scale;
     }
 }
 

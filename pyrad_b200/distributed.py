@@ -74,6 +74,24 @@ def assemble(gathered, plan):
     return torch.cat(parts) if parts else gathered.new_zeros(0)
 
 
+def sum_over_ranks(values, dist=None):
+    """Sum of a small float64 vector over the ranks -- e.g. the level fluxes of Engine.atmosphere_fluxes, of which every
+    rank holds its wavenumber chunk's share.  ONE all_gather, then the ranks' vectors added in rank order on every rank,
+    so the result is deterministic and the same everywhere (an all_reduce leaves the order to the backend)."""
+    import torch
+    v = torch.as_tensor(np.ascontiguousarray(values, dtype=np.float64))
+    if dist is None or dist.get_world_size() == 1:
+        return v.numpy().copy()
+    if dist.get_backend() == "nccl":
+        v = v.cuda()
+    parts = [torch.empty_like(v) for _ in range(dist.get_world_size())]
+    dist.all_gather(parts, v)
+    total = parts[0].clone()
+    for p in parts[1:]:
+        total += p
+    return total.cpu().numpy()
+
+
 def connect_peers(engine, rank, world, max_chunk_points, dist):
     """Set up the engine's peer-memory gather: allocate this rank's buffer, exchange the CUDA IPC handles
     with ONE all_gather of 64 bytes per rank (torch.distributed: plumbing), map every peer.  After this,

@@ -394,6 +394,7 @@ class Engine:
             rc = fn(h, L, g, *ptrs, ts, rm)
             if rc:
                 _lib.check(rc)
+            self.atm_layers = L
         call.keepalive = (keep, win)
         return call
 
@@ -424,6 +425,7 @@ class Engine:
             if rc:
                 _lib.check(rc)
             self.n_lines, self.n_groups = n, g
+            self.atm_layers = 1
             self.n_chunk = int(i_end) - int(i_begin)
             self.n_total = int(n_total)
             self.i_begin, self.i_end = int(i_begin), int(i_end)
@@ -451,6 +453,24 @@ class Engine:
         _lib.check(self._lib.prb_atmosphere_read_f32(
             self._h, rad.ctypes.data_as(fp) if rad is not None else None,
             tr.ctypes.data_as(fp) if tr is not None else None))
+
+    def atmosphere_fluxes(self, mu, weights, rows=False):
+        """Hemispheric fluxes of the last column (prb_atmosphere_fluxes) for the angular quadrature (mu, weights), 1 to 4
+        nodes: (flux_up, flux_down), float64 W m-2 per level (L+1: level 0 = surface, L = top; this chunk's share).  With
+        rows=True also (rad_up_top, rad_down_surface), float32 (n_mu, chunk): the radiance leaving the top and reaching
+        the surface along every mu."""
+        m, w = _f64(np.atleast_1d(mu)), _f64(np.atleast_1d(weights))
+        if m.ndim != 1 or m.shape != w.shape:
+            raise ValueError("atmosphere_fluxes: mu and weights must be 1-d arrays of one length")
+        L = int(getattr(self, "atm_layers", 0))
+        up, down = np.zeros(L + 1), np.zeros(L + 1)
+        fp = C.POINTER(C.c_float)
+        ru = np.empty((m.size, self.n_chunk), dtype=np.float32) if rows else None
+        rd = np.empty((m.size, self.n_chunk), dtype=np.float32) if rows else None
+        _lib.check(self._lib.prb_atmosphere_fluxes(self._h, m.size, _dp(m), _dp(w), _dp(up) if L else None,
+                                                   _dp(down) if L else None, ru.ctypes.data_as(fp) if rows else None,
+                                                   rd.ctypes.data_as(fp) if rows else None))
+        return (up, down, ru, rd) if rows else (up, down)
 
     def set_result_host(self, rad=None, tr=None):
         """Register pinned float32 host arrays that every following atmosphere() fills directly from the device

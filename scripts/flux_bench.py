@@ -1,0 +1,101 @@
+"""Time prb_atmosphere_fluxes on the cfg4 column (100 layers, ~5 M lines, 0-5000 cm-1 at 0.001 cm-1: 5 M points).
+
+Runs the column once through prb_atmosphere (far-field K2, as bench.py's atmosphere object), times it, then times the
+flux call for 1, 2, 3 and 4 angular nodes (Gauss-Legendre on [0, 1]) on the same resident k matrix: CUDA events on the
+engine stream around each call (the layer-table upload, the upward and downward k3_flux_tma passes, the two k3_flux_sum
+launches and the copy of the level fluxes), warm-up first, then --reps calls.  Also reports the algorithmic bytes (the
+k matrix read once per pass, L N 4 bytes, two passes) and their rate against prb_measure_peaks' copy bandwidth, and the
+device name and power limit read in the same run.  Prints one JSON line; writes nothing.
+
+    python scripts/flux_bench.py [--reps 30] [--warmup 3]
+"""
+import argparse
+import json
+import os
+import subprocess
+import sys
+
+import numpy as np
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+
+
+def device_power():
+    try:
+        out = subprocess.run(["nvidia-smi", "-i", "0", "--query-gpu=name,power.limit,clocks.max.sm",
+                              "--format=csv,noheader,nounits"], capture_output=True, text=True, timeout=20).stdout
+        name, limit, mhz = [x.strip() for x in out.strip().splitlines()[0].split(",")]
+        return {"nvidia_smi_name": name, "power_limit_w": float(limit), "sm_max_mhz": float(mhz)}
+    except Exception as ex:                                   # the timing stands without it; say why it is missing
+        return {"nvidia_smi_error": str(ex)}
+
+
+def timed(stream, fn, warmup, reps):
+    import torch
+    for _ in range(warmup):
+        fn()
+    ms = []
+    for _ in range(reps):
+        a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        a.record(stream)
+        fn()
+        b.record(stream)
+        b.synchronize()
+        ms.append(a.elapsed_time(b))
+    return ms
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--reps", type=int, default=30)
+    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--atm-reps", type=int, default=5)
+    args = ap.parse_args()
+    if args.reps < 20:
+        ap.error("--reps must be at least 20")
+    import torch
+    from pyrad_b200 import engine as eng
+    from pyrad_b200 import workloads
+
+    if not torch.cuda.is_available():
+        raise SystemExit("flux_bench: no CUDA device (there is no CPU measurement)")
+    w = workloads.atmosphere()
+    sp = w["species"]
+    L = len(w["T"])
+    e = eng.Engine(0)
+    n = eng.grid_len(w["range_min"], w["range_max"], w["res"])
+    e.upload_lines(w["lines"], n_groups=len(sp))
+    e.set_grid(w["range_min"], w["res"], n)
+    win = [eng.window_len(c, w["res"]) for c in w["cutoff"]]
+    qt = np.array([[s.q(T) for s in sp] for T in w["T"]])
+    column = e.atmosphere_call(w["depth_cm"], w["T"], w["P"], w["conc"], [s.molmass for s in sp], qt,
+                               [s.q296 for s in sp], win, w["t_surface"], w["range_max"])
+    stream = torch.cuda.ExternalStream(e.stream)
+    e.set_k2_variant(eng.K2_FARFIELD, 0)
+    atm_ms = timed(stream, column, 1, args.atm_reps)
+    peaks = e.measure_peaks()
+    pass_bytes = L * n * 4
+    out = {"workload": "cfg4: %d layers, %d lines, %d points, far-field K2" % (L, len(w["lines"]["nu"]), n),
+           "device": torch.cuda.get_device_name(0), **device_power(),
+           "atmosphere_ms_median": float(np.median(atm_ms)), "atmosphere_ms_runs": atm_ms,
+           "copy_bytes_per_s": peaks["copy_bytes_per_s"], "kmatrix_pass_bytes": pass_bytes, "fluxes": []}
+    for n_mu in (1, 2, 3, 4):
+        x, wt = np.polynomial.legendre.leggauss(n_mu)
+        mu, wt = (x + 1) / 2, wt / 2
+        ms = timed(stream, lambda: e.atmosphere_fluxes(mu, wt), args.warmup, args.reps)
+        med = float(np.median(ms))
+        up, down = e.atmosphere_fluxes(mu, wt)
+        out["fluxes"].append({
+            "n_mu": n_mu, "ms_median": med, "ms_min": float(np.min(ms)), "ms_max": float(np.max(ms)),
+            "ms_p10_p90": [float(np.percentile(ms, 10)), float(np.percentile(ms, 90))], "reps": args.reps,
+            "bytes_per_s": 2 * pass_bytes / (med * 1e-3),
+            "share_of_copy_bandwidth": 2 * pass_bytes / (med * 1e-3) / peaks["copy_bytes_per_s"],
+            "share_of_atmosphere": med / float(np.median(atm_ms)),
+            "olr_w_m2": float(up[-1]), "surface_down_w_m2": float(down[0])})
+    e.close()
+    print(json.dumps(out))
+
+
+if __name__ == "__main__":
+    main()
