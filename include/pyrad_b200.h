@@ -21,6 +21,7 @@
  *   pyradClasses.py:409-428,26-29 line survey, integrateSpectrum            -> prb_line_survey, prb_integrate_spectrum
  *   (absent upstream, SURVEY 3.5) multi-layer fold of Layer.transmission   -> prb_atmosphere
  *   (absent upstream) hemispheric fluxes, downwelling and slant radiances of the column -> prb_atmosphere_fluxes
+ *   (absent upstream) the column's fluxes per wavenumber band, at every level      -> prb_atmosphere_band_fluxes
  *
  * Conventions: every entry point is extern "C", returns int (0 = PRB_OK, < 0 = error) unless
  * noted, takes plain pointers and sizes.  Pointers named *_host / unmarked are caller-owned host
@@ -271,6 +272,16 @@ int prb_atmosphere_launches(prb_engine *e);              /* kernels launched by 
  * mu = 1 reproduces prb_atmosphere's radiance bit for bit.  Under a peer connection the call stays local. */
 int prb_atmosphere_fluxes(prb_engine *e, int32_t n_mu, const double *mu, const double *weight,
                           double *flux_up, double *flux_down, float *rad_up_top, float *rad_down_surface);
+/* The same fluxes as prb_atmosphere_fluxes (same column, quadrature rules, levels and non-finite rule), split by wavenumber
+ * band.  Grid point i belongs to band b when edges[b] <= x_i < edges[b+1], x the column's Planck axis
+ * (linspace(range_min, range_max, n_total)); points outside [edges[0], edges[n_bands]) count nowhere, and a band with no
+ * points gives zeros.  edges: n_bands + 1 finite values, strictly ascending (n_bands >= 1).  band_up / band_down:
+ * [n_bands][L+1] doubles each, this chunk's share, F_b[j] = 2 pi sum_i weight[i] mu[i] sum_{nu in b} I_i(nu, level j) res;
+ * either may be NULL.  Only the k-matrix strips that meet a band are read.  The sums are deterministic and independent of
+ * the launch grid: repeated calls give the same bits, and so does a band read from a chunk that holds it whole (chunks
+ * aligned to 128 points).  Under a peer connection the call stays local. */
+int prb_atmosphere_band_fluxes(prb_engine *e, int32_t n_mu, const double *mu, const double *weight,
+                               int32_t n_bands, const double *edges, double *band_up, double *band_down);
 int prb_set_option(prb_engine *e, int option, int64_t value);
 
 /* ---- section 8(f) rows beside the hot path -------------------------------------------------------

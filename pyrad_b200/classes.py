@@ -868,7 +868,7 @@ class Atmosphere(list):
         stay resident on the device and enter every layer's k(nu) inside the line-sum kernel (prb_xsc_resident)."""
         return self._column(surfaceTemperature, lambda e: e.atmosphere_read())
 
-    def columnFluxes(self, surfaceTemperature, mu=None, weights=None):
+    def columnFluxes(self, surfaceTemperature, mu=None, weights=None, bands=None):
         """Hemispheric fluxes, heating rates and slant radiances of the column (prb_atmosphere, then
         prb_atmosphere_fluxes on its device-resident k matrix; same requirements on the layers as columnSpectrum).
         For every node mu_i of the angular quadrature (default: 3-node Gauss-Legendre on [0, 1]; at most 4 nodes) the
@@ -878,19 +878,36 @@ class Atmosphere(list):
         isotropic, so F_up at the top differs from the pi x nadir radiance of integrateSpectrum(columnSpectrum(...)[0]).
         Returns a dict: flux_up, flux_down, net (= up - down) per level in W m-2; heating_rate per layer in K/day
         (heatingRate); rad_up_top and rad_down_surface, float32 (n_mu, n_points) -- the radiance leaving the top and
-        reaching the surface along every mu_i; mu and weights."""
+        reaching the surface along every mu_i; mu and weights.
+        bands: optional band edges in cm-1 (1-d, at least 2, finite, strictly ascending); a grid point nu belongs to band
+        b when bands[b] <= nu < bands[b+1] (prb_atmosphere_band_fluxes, on the same column run).  The dict then also holds
+        band_edges, band_flux_up and band_flux_down (n_bands, L+1), band_net, and band_heating_rate (n_bands, L): each
+        band's heating rate by heatingRate."""
         if mu is None and weights is None:
             x, w = np.polynomial.legendre.leggauss(3)
             mu, weights = (x + 1) / 2, w / 2
         mu, weights = np.atleast_1d(np.asarray(mu, dtype=np.float64)), np.atleast_1d(np.asarray(weights, dtype=np.float64))
         if mu.shape != weights.shape or not 1 <= mu.size <= 4:
             raise ValueError("columnFluxes needs 1 to 4 quadrature nodes, as many weights as mu")
-        up, down, ru, rd = self._column(surfaceTemperature, lambda e: e.atmosphere_fluxes(mu, weights, rows=True))
+        if bands is not None:
+            bands = np.asarray(bands, dtype=np.float64)
+            if bands.ndim != 1 or bands.size < 2 or not np.all(np.isfinite(bands)) or not np.all(np.diff(bands) > 0):
+                raise ValueError("columnFluxes: bands must be a 1-d array of at least 2 finite, strictly ascending edges")
+
+        def result(e):
+            return (e.atmosphere_fluxes(mu, weights, rows=True),
+                    e.atmosphere_band_fluxes(mu, weights, bands) if bands is not None else None)
+
+        (up, down, ru, rd), band = self._column(surfaceTemperature, result)
         layers = list(self)
-        return {"flux_up": up, "flux_down": down, "net": up - down,
-                "heating_rate": heatingRate(up, down, [l.depth for l in layers], [l.T for l in layers],
-                                            [l.P for l in layers]),
-                "rad_up_top": ru, "rad_down_surface": rd, "mu": mu, "weights": weights}
+        depth, T, P = [l.depth for l in layers], [l.T for l in layers], [l.P for l in layers]
+        out = {"flux_up": up, "flux_down": down, "net": up - down, "heating_rate": heatingRate(up, down, depth, T, P),
+               "rad_up_top": ru, "rad_down_surface": rd, "mu": mu, "weights": weights}
+        if band is not None:
+            bu, bd = band
+            out.update(band_edges=bands, band_flux_up=bu, band_flux_down=bd, band_net=bu - bd,
+                       band_heating_rate=np.array([heatingRate(u, d, depth, T, P) for u, d in zip(bu, bd)]))
+        return out
 
     def _column(self, surfaceTemperature, result):
         """Run the column on the device (prb_atmosphere) and return result(engine) while its state is in place."""

@@ -217,6 +217,8 @@ struct prb_engine {
     DevBuf<FluxLayer> flux_layers;
     DevBuf<double> flux_part, flux_out;
     DevBuf<float> flux_rows;
+    DevBuf<double> band_part, band_out;               // prb_atmosphere_band_fluxes: per-segment level sums, band totals
+    DevBuf<int32_t> band_tab;                         // its span, segment, band and strip tables
     // optional stage timing of prb_atmosphere (CUDA events on the engine stream)
     bool timing = false;
     std::vector<cudaEvent_t> ev;
@@ -312,6 +314,7 @@ extern "C" int prb_destroy(prb_engine *e) {
     e->scratch_d.release(); e->scratch_w.release();
     e->kmat.release(); e->rad.release(); e->trans.release(); e->fold.release();
     e->flux_layers.release(); e->flux_part.release(); e->flux_out.release(); e->flux_rows.release();
+    e->band_part.release(); e->band_out.release(); e->band_tab.release();
     e->k2tab.release(); e->ring_d.release(); e->peer_err.release();
     if (e->blk_h) cudaFreeHost(e->blk_h);
     if (e->read_stage) cudaFreeHost(e->read_stage);
@@ -1796,10 +1799,10 @@ extern "C" int prb_atmosphere_read_f32(prb_engine *e, float *radiance_host, floa
     return PRB_OK;
 }
 
-// One flux pass (k3_flux_tma) over the resident k matrix; its per-CTA level sums go to a.part.
-template <int NMU, bool DOWN>
+// One flux pass (k3_flux_tma) over the resident k matrix; its level sums (per CTA, or per segment for BAND) go to a.part.
+template <int NMU, bool DOWN, bool BAND = false>
 static cudaError_t launch_flux(prb_engine *e, int grid, size_t smem, double dx, const K3FArgs &a) {
-    const auto fn = k3_flux_tma<NMU, DOWN>;
+    const auto fn = k3_flux_tma<NMU, DOWN, BAND>;
     cudaError_t ce = cudaFuncSetAttribute((const void *)fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (ce != cudaSuccess) return ce;
     const double c2 = 100 * hPlanck * cLight / kBoltz;
@@ -1809,60 +1812,84 @@ static cudaError_t launch_flux(prb_engine *e, int grid, size_t smem, double dx, 
     return cudaGetLastError();
 }
 
-template <int NMU>
+template <int NMU, bool BAND = false>
 static cudaError_t launch_flux_pair(prb_engine *e, int grid, size_t smem, double dx, const K3FArgs &up, const K3FArgs &down) {
-    cudaError_t ce = launch_flux<NMU, false>(e, grid, smem, dx, up);
-    return ce != cudaSuccess ? ce : launch_flux<NMU, true>(e, grid, smem, dx, down);
+    cudaError_t ce = launch_flux<NMU, false, BAND>(e, grid, smem, dx, up);
+    return ce != cudaSuccess ? ce : launch_flux<NMU, true, BAND>(e, grid, smem, dx, down);
+}
+
+template <bool BAND>
+static cudaError_t launch_flux_passes(prb_engine *e, int n_mu, int grid, size_t smem, double dx, const K3FArgs &up,
+                                      const K3FArgs &down) {
+    switch (n_mu) {
+        case 1: return launch_flux_pair<1, BAND>(e, grid, smem, dx, up, down);
+        case 2: return launch_flux_pair<2, BAND>(e, grid, smem, dx, up, down);
+        case 3: return launch_flux_pair<3, BAND>(e, grid, smem, dx, up, down);
+        default: return launch_flux_pair<4, BAND>(e, grid, smem, dx, up, down);
+    }
+}
+
+// The checks shared by the flux calls: a column on the device, a quadrature of 1 to 4 nodes with mu in (0, 1] and finite
+// weights > 0, and few enough layers for k3_flux_tma's per-level accumulators.
+static int flux_check(prb_engine *e, const char *fn, int32_t n_mu, const double *mu, const double *weight) {
+    if (!e || !e->atm_layers) return fail(PRB_ERR_STATE, std::string(fn) + ": run prb_atmosphere first");
+    if (n_mu < 1 || n_mu > 4 || !mu || !weight) return fail(PRB_ERR_ARG, std::string(fn) + ": need 1 <= n_mu <= 4, mu and weight");
+    for (int i = 0; i < n_mu; ++i)
+        if (!(mu[i] > 0 && mu[i] <= 1) || !(weight[i] > 0 && std::isfinite(weight[i])))
+            return fail(PRB_ERR_ARG, std::string(fn) + ": every mu must lie in (0, 1] and every weight be finite and > 0");
+    if (k3f_smem_bytes(e->atm_layers) > (size_t)e->prop.sharedMemPerBlockOptin)
+        return fail(PRB_ERR_RANGE, std::string(fn) + ": too many layers for the per-level accumulators in shared memory");
+    return PRB_OK;
+}
+
+// Per layer: c2 / T_l and -depth_l log2(e) / mu_i, rounded as the fold rounds them (mu = 1 gives its very constants),
+// uploaded to e->flux_layers; and w_i mu_i into both passes' arguments.
+static cudaError_t flux_layers_upload(prb_engine *e, int32_t n_mu, const double *mu, const double *weight,
+                                      std::vector<FluxLayer> &hl, K3FArgs &up, K3FArgs &down) {
+    const int L = e->atm_layers;
+    const double c2 = 100 * hPlanck * cLight / kBoltz;
+    hl.resize(L);
+    for (int l = 0; l < L; ++l) {
+        hl[l].c2_over_t = (float)(c2 / e->atm_t[l]);
+        for (int i = 0; i < 4; ++i) hl[l].nd[i] = i < n_mu ? (float)(-e->atm_depth[l] * 1.4426950408889634 / mu[i]) : 0.f;
+    }
+    for (int i = 0; i < n_mu; ++i) up.wmu[i] = down.wmu[i] = (float)(weight[i] * mu[i]);
+    cudaError_t ce = e->flux_layers.ensure(L);
+    if (ce != cudaSuccess) return ce;
+    return cudaMemcpyAsync(e->flux_layers.p, hl.data(), sizeof(FluxLayer) * L, cudaMemcpyHostToDevice, e->stream);
+}
+
+static double flux_dx(const prb_engine *e) {
+    return e->n_total > 1 ? (e->atm_range_max - e->range_min) / (double)(e->n_total - 1) : 0.0;
 }
 
 extern "C" int prb_atmosphere_fluxes(prb_engine *e, int32_t n_mu, const double *mu, const double *weight, double *flux_up,
                                      double *flux_down, float *rad_up_top, float *rad_down_surface) {
-    if (!e || !e->atm_layers) return fail(PRB_ERR_STATE, "prb_atmosphere_fluxes: run prb_atmosphere first");
-    if (n_mu < 1 || n_mu > 4 || !mu || !weight) return fail(PRB_ERR_ARG, "prb_atmosphere_fluxes: need 1 <= n_mu <= 4, mu and weight");
-    for (int i = 0; i < n_mu; ++i)
-        if (!(mu[i] > 0 && mu[i] <= 1) || !(weight[i] > 0 && std::isfinite(weight[i])))
-            return fail(PRB_ERR_ARG, "prb_atmosphere_fluxes: every mu must lie in (0, 1] and every weight be finite and > 0");
+    if (int rc = flux_check(e, "prb_atmosphere_fluxes", n_mu, mu, weight)) return rc;
     CK(cudaSetDevice(e->device));
     const int L = e->atm_layers, n_levels = L + 1;
     const int64_t nc = chunk_len(e);
     const size_t smem = k3f_smem_bytes(L);
-    if (smem > (size_t)e->prop.sharedMemPerBlockOptin)
-        return fail(PRB_ERR_RANGE, "prb_atmosphere_fluxes: too many layers for the per-level accumulators in shared memory");
     if (nc == 0) {                                              // an empty chunk contributes nothing
         if (flux_up) std::fill(flux_up, flux_up + n_levels, 0.0);
         if (flux_down) std::fill(flux_down, flux_down + n_levels, 0.0);
         return PRB_OK;
     }
-    // per layer: c2 / T_l and -depth_l log2(e) / mu_i, rounded as the fold rounds them (mu = 1 gives its very constants)
-    const double c2 = 100 * hPlanck * cLight / kBoltz;
-    std::vector<FluxLayer> hl(L);
-    for (int l = 0; l < L; ++l) {
-        hl[l].c2_over_t = (float)(c2 / e->atm_t[l]);
-        for (int i = 0; i < 4; ++i) hl[l].nd[i] = i < n_mu ? (float)(-e->atm_depth[l] * 1.4426950408889634 / mu[i]) : 0.f;
-    }
+    std::vector<FluxLayer> hl;
+    K3FArgs up{}, down{};
+    CK(flux_layers_upload(e, n_mu, mu, weight, hl, up, down));
     const int64_t n_strips = (nc + K3T_STRIP - 1) / K3T_STRIP;
     const int grid = (int)std::min<int64_t>(n_strips, k3f_minb(n_mu) * (int64_t)e->prop.multiProcessorCount);
     const bool rows = rad_up_top || rad_down_surface;
-    CK(e->flux_layers.ensure(L));
     CK(e->flux_part.ensure((size_t)2 * grid * n_levels));
     CK(e->flux_out.ensure((size_t)2 * n_levels));
     if (rows) CK(e->flux_rows.ensure((size_t)2 * 4 * e->kmat_ld));
-    CK(cudaMemcpyAsync(e->flux_layers.p, hl.data(), sizeof(FluxLayer) * L, cudaMemcpyHostToDevice, e->stream));
-    K3FArgs up{}, down{};
-    for (int i = 0; i < n_mu; ++i) up.wmu[i] = down.wmu[i] = (float)(weight[i] * mu[i]);
     up.ld_rows = down.ld_rows = e->kmat_ld;
     up.rows = rows ? e->flux_rows.p : nullptr;
     down.rows = rows ? e->flux_rows.p + (size_t)4 * e->kmat_ld : nullptr;
     up.part = e->flux_part.p;
     down.part = e->flux_part.p + (size_t)grid * n_levels;
-    const double dx = e->n_total > 1 ? (e->atm_range_max - e->range_min) / (double)(e->n_total - 1) : 0.0;
-    cudaError_t ce;
-    switch (n_mu) {
-        case 1: ce = launch_flux_pair<1>(e, grid, smem, dx, up, down); break;
-        case 2: ce = launch_flux_pair<2>(e, grid, smem, dx, up, down); break;
-        case 3: ce = launch_flux_pair<3>(e, grid, smem, dx, up, down); break;
-        default: ce = launch_flux_pair<4>(e, grid, smem, dx, up, down); break;
-    }
+    const cudaError_t ce = launch_flux_passes<false>(e, n_mu, grid, smem, flux_dx(e), up, down);
     if (ce != cudaSuccess) return fail(PRB_ERR_CUDA, std::string("k3_flux_tma launch failed: ") + cudaGetErrorString(ce));
     // F[j] = 2 pi sum_i w_i mu_i sum_nu I_i(nu, j) res  (integrateSpectrum's res and NaN rule, pyradClasses.py:26-29)
     const double scale = 2 * 3.141592653589793 * e->res;
@@ -1881,6 +1908,116 @@ extern "C" int prb_atmosphere_fluxes(prb_engine *e, int32_t n_mu, const double *
             CK(cudaMemcpyAsync(rad_down_surface + (size_t)i * nc, down.rows + (size_t)i * e->kmat_ld, sizeof(float) * nc,
                                cudaMemcpyDeviceToHost, e->stream));
     }
+    CK(cudaStreamSynchronize(e->stream));
+    return PRB_OK;
+}
+
+// The first grid point i in [0, n] with axis_value(i) >= v (n if none): the axis is non-decreasing.
+static int64_t first_point_at_or_above(double v, int64_t n, double x0, double dx, double x_last) {
+    int64_t lo = 0, hi = n;
+    while (lo < hi) {
+        const int64_t mid = lo + (hi - lo) / 2;
+        if (axis_value(mid, n, x0, dx, x_last) >= v) hi = mid;
+        else lo = mid + 1;
+    }
+    return lo;
+}
+
+extern "C" int prb_atmosphere_band_fluxes(prb_engine *e, int32_t n_mu, const double *mu, const double *weight,
+                                          int32_t n_bands, const double *edges, double *band_up, double *band_down) {
+    if (int rc = flux_check(e, "prb_atmosphere_band_fluxes", n_mu, mu, weight)) return rc;
+    if (n_bands < 1 || !edges) return fail(PRB_ERR_ARG, "prb_atmosphere_band_fluxes: need n_bands >= 1 and n_bands + 1 edges");
+    for (int b = 0; b <= n_bands; ++b)
+        if (!std::isfinite(edges[b]) || (b > 0 && !(edges[b] > edges[b - 1])))
+            return fail(PRB_ERR_ARG, "prb_atmosphere_band_fluxes: the edges must be finite and strictly ascending");
+    CK(cudaSetDevice(e->device));
+    const int L = e->atm_layers, n_levels = L + 1;
+    const int64_t nc = chunk_len(e);
+    const size_t per_dir = (size_t)n_bands * n_levels;
+    auto zeros = [&]() {
+        if (band_up) std::fill(band_up, band_up + per_dir, 0.0);
+        if (band_down) std::fill(band_down, band_down + per_dir, 0.0);
+        return PRB_OK;
+    };
+    if (nc == 0) return zeros();                                // an empty chunk contributes nothing
+    constexpr int SPAN = 128;                                   // points per warp
+    const int64_t n_strips = (nc + K3T_STRIP - 1) / K3T_STRIP, n_spans = n_strips * K3F_WARPS;
+    if (n_spans + n_bands + 1 > INT32_MAX) return fail(PRB_ERR_RANGE, "prb_atmosphere_band_fluxes: chunk too long");
+    // Band b holds the points with edges[b] <= x_i < edges[b+1], x the Planck axis of the fold: the chunk-local points
+    // [p[b], p[b+1]), each p the first point at or above its edge by the device's own formula (exact at grid values).
+    const double dx = flux_dx(e);
+    std::vector<int64_t> p(n_bands + 1);
+    for (int b = 0; b <= n_bands; ++b)
+        p[b] = std::clamp<int64_t>(first_point_at_or_above(edges[b], e->n_total, e->range_min, dx, e->atm_range_max) -
+                                   e->i_begin, 0, nc);
+    // Segments (span x band) in position order; a band's segments are consecutive: band_seg[b] .. band_seg[b+1].
+    std::vector<K3FSpan> spans(n_spans, K3FSpan{0, 0});
+    std::vector<uint32_t> seg_range;
+    std::vector<int32_t> band_seg(n_bands + 1);
+    for (int b = 0; b < n_bands; ++b) {
+        band_seg[b] = (int32_t)seg_range.size();
+        if (p[b] >= p[b + 1]) continue;                         // a band with no points: no segments, zeros
+        for (int64_t s = p[b] / SPAN; s <= (p[b + 1] - 1) / SPAN; ++s) {
+            const int64_t s0 = s * SPAN, s1 = std::min(s0 + SPAN, nc);
+            const uint32_t lo = (uint32_t)(std::max(p[b], s0) - s0), hi = (uint32_t)(std::min(p[b + 1], s1) - s0);
+            if (spans[s].nseg == 0) spans[s].seg0 = (int32_t)seg_range.size();
+            spans[s].nseg++;
+            seg_range.push_back(lo | hi << 16);
+        }
+    }
+    const int64_t n_seg = (int64_t)seg_range.size();
+    band_seg[n_bands] = (int32_t)n_seg;
+    for (int64_t s = 0; s < n_spans; ++s)                       // one band over all of the span's points: the plain sum
+        if (spans[s].nseg == 1 && seg_range[spans[s].seg0] == (uint32_t)(std::min<int64_t>(SPAN, nc - s * SPAN) << 16))
+            spans[s].nseg = -1;
+    // the strips that meet a band, and the bands by the size of their sum (k3_flux_band_sum)
+    std::vector<int32_t> strips, small, big;
+    for (int64_t t = 0; t < n_strips; ++t)
+        for (int w = 0; w < K3F_WARPS; ++w)
+            if (spans[t * K3F_WARPS + w].nseg != 0) { strips.push_back((int32_t)t); break; }
+    if (strips.empty()) return zeros();                         // no band meets the chunk
+    for (int b = 0; b < n_bands; ++b) (band_seg[b + 1] - band_seg[b] > K3F_BAND_WARP_MAX ? big : small).push_back(b);
+    // one upload: spans | seg_range | band_seg | strips | small | big
+    std::vector<int32_t> tab(2 * n_spans + n_seg);
+    std::memcpy(tab.data(), spans.data(), sizeof(K3FSpan) * n_spans);
+    std::memcpy(tab.data() + 2 * n_spans, seg_range.data(), sizeof(uint32_t) * n_seg);
+    const size_t o_band = tab.size(), o_strips = o_band + band_seg.size(), o_small = o_strips + strips.size(),
+                 o_big = o_small + small.size();
+    for (const auto *v : {&band_seg, &strips, &small, &big}) tab.insert(tab.end(), v->begin(), v->end());
+    std::vector<FluxLayer> hl;
+    K3FArgs up{}, down{};
+    CK(flux_layers_upload(e, n_mu, mu, weight, hl, up, down));
+    CK(e->band_tab.ensure(tab.size()));
+    CK(cudaMemcpyAsync(e->band_tab.p, tab.data(), sizeof(int32_t) * tab.size(), cudaMemcpyHostToDevice, e->stream));
+    CK(e->band_part.ensure((size_t)2 * n_levels * n_seg));
+    CK(e->band_out.ensure(2 * per_dir));
+    const int32_t *d_tab = e->band_tab.p;
+    for (K3FArgs *a : {&up, &down}) {
+        a->strips = d_tab + o_strips;
+        a->n_list = (int64_t)strips.size();
+        a->spans = reinterpret_cast<const K3FSpan *>(d_tab);
+        a->seg_range = reinterpret_cast<const uint32_t *>(d_tab + 2 * n_spans);
+        a->ld_part = n_seg;
+    }
+    up.part = e->band_part.p;
+    down.part = e->band_part.p + (size_t)n_levels * n_seg;
+    const int grid = (int)std::min<int64_t>((int64_t)strips.size(), k3f_minb(n_mu) * (int64_t)e->prop.multiProcessorCount);
+    const cudaError_t ce = launch_flux_passes<true>(e, n_mu, grid, sizeof(K3FSmem), dx, up, down);
+    if (ce != cudaSuccess) return fail(PRB_ERR_CUDA, std::string("k3_flux_tma launch failed: ") + cudaGetErrorString(ce));
+    // F_b[j] = 2 pi sum_i w_i mu_i sum_{nu in band b} I_i(nu, j) res
+    const double scale = 2 * 3.141592653589793 * e->res;
+    if (!small.empty()) {
+        const int64_t items = 2 * (int64_t)small.size() * n_levels;
+        k3_flux_band_sum<32><<<(unsigned)((items + 7) / 8), 256, 0, e->stream>>>(
+            e->band_part.p, n_seg, n_levels, d_tab + o_small, (int)small.size(), d_tab + o_band, n_bands, scale, e->band_out.p);
+    }
+    if (!big.empty())
+        k3_flux_band_sum<256><<<(unsigned)(2 * big.size() * n_levels), 256, 0, e->stream>>>(
+            e->band_part.p, n_seg, n_levels, d_tab + o_big, (int)big.size(), d_tab + o_band, n_bands, scale, e->band_out.p);
+    CK(cudaGetLastError());
+    if (band_up) CK(cudaMemcpyAsync(band_up, e->band_out.p, sizeof(double) * per_dir, cudaMemcpyDeviceToHost, e->stream));
+    if (band_down)
+        CK(cudaMemcpyAsync(band_down, e->band_out.p + per_dir, sizeof(double) * per_dir, cudaMemcpyDeviceToHost, e->stream));
     CK(cudaStreamSynchronize(e->stream));
     return PRB_OK;
 }

@@ -15,10 +15,16 @@
 
 namespace prb {
 
-// nu_i of np.linspace(start, stop, n): i*step + start (two roundings, as numpy), last = stop.
-__device__ __forceinline__ double axis_value(int64_t i, int64_t n, double x0, double dx, double x_last) {
+// nu_i of np.linspace(start, stop, n): i*step + start (two roundings, as numpy), last = stop.  The host evaluates the
+// same two roundings (no FMA contraction) when it turns band edges into point indices.
+__host__ __device__ __forceinline__ double axis_value(int64_t i, int64_t n, double x0, double dx, double x_last) {
     if (i == n - 1) return x_last;
+#ifdef __CUDA_ARCH__
     return __dadd_rn(__dmul_rn((double)i, dx), x0);
+#else
+    volatile double p = (double)i * dx;                // a separate rounding of the product, as __dmul_rn
+    return p + x0;
+#endif
 }
 
 __device__ __forceinline__ double planck_f64(double nu, double temp) {
@@ -436,16 +442,36 @@ k3_fold_tma(const float *__restrict__ kmat, int64_t ld, int n_layers, const Fold
 // finite counts as 0, see `partial`), a fixed xor-butterfly adds the warp's 32 values, and lane 0 adds the result into a per-(warp,
 // level) FP64 accumulator in shared memory that lives for all of the CTA's strips.  The CTA then writes its per-level
 // partials (warps in order) and k3_flux_sum adds them in CTA order: the result is deterministic, with no atomics.
+//
+// Band pass (BAND = true, prb_atmosphere_band_fluxes): the same fold, but each warp's sums are kept apart by wavenumber
+// band instead of running over strips.  The 128 points of a warp (its span) meet zero or more bands; a segment is the
+// intersection of a span with a band, numbered in position order (so a band's segments are consecutive).  At each level a
+// span that lies inside one band forms exactly the sum above (partial() and the butterfly); a span that meets band edges
+// forms one masked sum per segment (same non-finite rule) with the same butterfly.  Lane 0 stores each as FP64 into
+// part[level][segment].  The CTA walks the host's list of strips that meet a band, and k3_flux_band_sum adds each band's
+// segments in position order with a tree whose shape depends only on their count: the result depends on the edges and
+// the span positions only, not on the launch grid.
 struct FluxLayer {
     float c2_over_t;         // 100 h c / kB / T_layer
     float nd[4];             // -depth log2(e) / mu_i: T_i = exp2(k * nd[i])
+};
+
+struct K3FSpan {
+    int32_t seg0;            // the span's first segment
+    int32_t nseg;            // how many segments it holds; -1: one, and the band covers all of the span's points
 };
 
 struct K3FArgs {
     float wmu[4];            // w_i mu_i
     float *rows;             // [NMU][ld_rows]: radiance leaving the column at the last level of the pass (NULL: none)
     int64_t ld_rows;
-    double *part;            // [gridDim.x][n_layers + 1] per-CTA level sums
+    double *part;            // [gridDim.x][n_layers + 1] per-CTA level sums; band pass: [n_layers + 1][ld_part]
+    // band pass only
+    const int32_t *strips;   // the n_list strips that meet a band, ascending
+    int64_t n_list;
+    const K3FSpan *spans;    // per span of the chunk, 8 per strip (a ragged last strip padded with empty spans)
+    const uint32_t *seg_range;   // per segment: its points within the span, [lo, hi) as lo | hi << 16 (0 <= lo < hi <= 128)
+    int64_t ld_part;         // the number of segments
 };
 
 constexpr int K3F_WARPS = K3T_THREADS / 32;
@@ -462,7 +488,7 @@ __host__ __device__ constexpr size_t k3f_smem_bytes(int n_layers) {
     return sizeof(K3FSmem) + sizeof(double) * K3F_WARPS * (size_t)(n_layers + 1);
 }
 
-template <int NMU, bool DOWN>
+template <int NMU, bool DOWN, bool BAND = false>
 __global__ void __launch_bounds__(K3T_THREADS, k3f_minb(NMU))
 k3_flux_tma(const float *__restrict__ kmat, int64_t ld, int n_layers, const FluxLayer *__restrict__ layers,
             int64_t n_chunk, int64_t i_begin, int64_t n_total, double x0, double dx, double x_last,
@@ -472,11 +498,12 @@ k3_flux_tma(const float *__restrict__ kmat, int64_t ld, int n_layers, const Flux
     double *acc = reinterpret_cast<double *>(k3_smem_raw + sizeof(K3FSmem));
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int n_levels = n_layers + 1;
-    const int64_t n_strips = (n_chunk + K3T_STRIP - 1) / K3T_STRIP;
+    const int64_t n_strips = BAND ? a.n_list : (n_chunk + K3T_STRIP - 1) / K3T_STRIP;
     const int groups = (n_layers + K3T_LAYERS - 1) / K3T_LAYERS;
     const int64_t my_strips = blockIdx.x < n_strips ? (n_strips - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
     const int64_t n_steps = my_strips * groups;
-    for (int j = tid; j < K3F_WARPS * n_levels; j += K3T_THREADS) acc[j] = 0.0;
+    if constexpr (!BAND)
+        for (int j = tid; j < K3F_WARPS * n_levels; j += K3T_THREADS) acc[j] = 0.0;
     if (tid == 0) {
         for (int s = 0; s < K3T_SLOTS; ++s) mbar_init(&sm.full[s], 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -485,9 +512,13 @@ k3_flux_tma(const float *__restrict__ kmat, int64_t ld, int n_layers, const Flux
     __syncthreads();
     // step s of the CTA covers row group s % groups of its strip, counted from the top for the downward pass
     auto group_of = [&](int64_t step) { const int g = (int)(step % groups); return DOWN ? groups - 1 - g : g; };
+    auto strip_of = [&](int64_t step) {
+        const int64_t s = blockIdx.x + (step / groups) * gridDim.x;
+        return BAND ? (int64_t)a.strips[s] : s;
+    };
     auto issue = [&](int64_t step) {                   // thread 0 only
         const int slot = (int)(step % K3T_SLOTS);
-        const int64_t strip = blockIdx.x + (step / groups) * gridDim.x;
+        const int64_t strip = strip_of(step);
         const int g = group_of(step);
         const int64_t p0 = strip * K3T_STRIP;
         const int64_t pts = min((int64_t)K3T_STRIP, ((n_chunk - p0) + 3) & ~int64_t(3));   // rows are padded to 4 floats
@@ -534,11 +565,57 @@ k3_flux_tma(const float *__restrict__ kmat, int64_t ld, int n_layers, const Flux
         for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
         if (lane == 0) acc[warp * n_levels + level] += (double)v;
     };
+    // band pass: one value per segment of the warp's span.  A span inside one band takes partial() and the butterfly
+    // above.  Otherwise each point's sum_i w_i mu_i I_i (a value that is not finite counts as 0) is formed once, and the
+    // segments are taken two at a time: each a masked sum over the thread's points in its range [lo, hi) of the span,
+    // both through one interleaved butterfly.
+    auto band_add = [&](int level) {                   // every lane of the warp takes part; the span is the warp's
+        const K3FSpan sp = a.spans[i0 >> 7];
+        double *dst = a.part + (int64_t)level * a.ld_part + sp.seg0;
+        if (sp.nseg < 0) {
+            float v = partial();
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+            if (lane == 0) dst[0] = (double)v;
+        } else if (sp.nseg > 0) {
+            float v[4];
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+                v[q] = 0.f;
+#pragma unroll
+                for (int i = 0; i < NMU; ++i)
+                    if (isfinite(rad[i][q])) v[q] = fmaf(a.wmu[i], rad[i][q], v[q]);
+            }
+            for (int s = 0; s < sp.nseg; s += 2) {
+                const uint32_t r0 = a.seg_range[sp.seg0 + s], r1 = s + 1 < sp.nseg ? a.seg_range[sp.seg0 + s + 1] : 0u;
+                float t0 = 0.f, t1 = 0.f;
+#pragma unroll
+                for (int q = 0; q < 4; ++q) {
+                    const uint32_t p = 4 * lane + q;
+                    if (p >= (r0 & 0xffffu) && p < (r0 >> 16)) t0 += v[q];
+                    if (p >= (r1 & 0xffffu) && p < (r1 >> 16)) t1 += v[q];
+                }
+#pragma unroll
+                for (int o = 16; o > 0; o >>= 1) {
+                    t0 += __shfl_xor_sync(0xffffffffu, t0, o);
+                    t1 += __shfl_xor_sync(0xffffffffu, t1, o);
+                }
+                if (lane == 0) {
+                    dst[s] = (double)t0;
+                    if (s + 1 < sp.nseg) dst[s + 1] = (double)t1;
+                }
+            }
+        }
+    };
+    auto add_level = [&](int level) {
+        if constexpr (BAND) band_add(level);
+        else level_add(partial(), level);
+    };
     for (int64_t step = 0; step < n_steps; ++step) {
         const int slot = (int)(step % K3T_SLOTS);
         const int g = group_of(step);
         if (step % groups == 0) {                      // a new strip: the boundary radiance of the pass
-            const int64_t strip = blockIdx.x + (step / groups) * gridDim.x;
+            const int64_t strip = strip_of(step);
             i0 = strip * K3T_STRIP + 4 * tid;
             n_valid = (int)max((int64_t)0, min((int64_t)4, n_chunk - i0));
 #pragma unroll
@@ -551,7 +628,8 @@ k3_flux_tma(const float *__restrict__ kmat, int64_t ld, int n_layers, const Flux
                 for (int i = 0; i < NMU; ++i) rad[i][q] = r0;
             }
             interp = nu[0] >= nu_interp_min;
-            if (!DOWN) level_add(partial(), 0);        // (the downward pass starts from 0 at level L)
+            if (!DOWN) add_level(0);                   // (the downward pass starts from 0 at level L)
+            else if (BAND) add_level(n_layers);        // (whose segment slots must still be written: zeros)
         }
         if (tid == 0 && step + K3T_SLOTS - 1 < n_steps) issue(step + K3T_SLOTS - 1);
         mbar_wait(&sm.full[slot], (uint32_t)((step / K3T_SLOTS) & 1));
@@ -574,7 +652,7 @@ k3_flux_tma(const float *__restrict__ kmat, int64_t ld, int n_layers, const Flux
                     const float2 r23 = k3_fold_step2(make_float2(rad[i][2], rad[i][3]), e23, b23);
                     rad[i][0] = r01.x; rad[i][1] = r01.y; rad[i][2] = r23.x; rad[i][3] = r23.y;
                 }
-                level_add(partial(), DOWN ? l : l + 1);
+                add_level(DOWN ? l : l + 1);
             }
         }
         __syncthreads();                               // every thread is done with this slot: it may be refilled
@@ -590,12 +668,45 @@ k3_flux_tma(const float *__restrict__ kmat, int64_t ld, int n_layers, const Flux
             }
         }
     }
-    __syncthreads();
-    for (int j = tid; j < n_levels; j += K3T_THREADS) {
-        double s = 0.0;
-        for (int w = 0; w < K3F_WARPS; ++w) s += acc[w * n_levels + j];
-        a.part[(int64_t)blockIdx.x * n_levels + j] = s;
+    if constexpr (!BAND) {
+        __syncthreads();
+        for (int j = tid; j < n_levels; j += K3T_THREADS) {
+            double s = 0.0;
+            for (int w = 0; w < K3F_WARPS; ++w) s += acc[w * n_levels + j];
+            a.part[(int64_t)blockIdx.x * n_levels + j] = s;
+        }
     }
+}
+
+// Band totals of the band pass: out[d][b][j] = scale * sum of band b's segments at level j of pass d (0 up, 1 down), for
+// the bands list[0 .. n_list).  G threads take one (d, b, j): thread t adds segments t, t + G, ... in order, then a fixed
+// xor butterfly over the warp and, for G = 256, the eight warps' values in a fixed tree.  The host picks G from the
+// band's segment count only (256 above K3F_BAND_WARP_MAX segments, else 32), so the order is a function of that count.
+constexpr int K3F_BAND_WARP_MAX = 1024;
+template <int G>
+__global__ void __launch_bounds__(256)
+k3_flux_band_sum(const double *__restrict__ part, int64_t ld_part, int n_levels, const int32_t *__restrict__ list,
+                 int n_list, const int32_t *__restrict__ band_seg, int n_bands, double scale, double *__restrict__ out) {
+    constexpr int PER = 256 / G;                       // (d, b, j) per block
+    const int64_t item = (int64_t)blockIdx.x * PER + threadIdx.x / G;
+    if (item >= 2 * (int64_t)n_list * n_levels) return;    // uniform over each group of G threads
+    const int t = threadIdx.x % G, lane = threadIdx.x & 31;
+    const int j = (int)(item % n_levels);
+    const int64_t r = item / n_levels;
+    const int d = (int)(r / n_list), b = list[r % n_list];
+    const int32_t s0 = band_seg[b], cnt = band_seg[b + 1] - s0;
+    const double *p = part + ((int64_t)d * n_levels + j) * ld_part + s0;
+    double s = 0.0;
+    for (int k = t; k < cnt; k += G) s += p[k];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+    if constexpr (G == 256) {
+        __shared__ double w[8];
+        if (lane == 0) w[threadIdx.x >> 5] = s;
+        __syncthreads();
+        s = ((w[0] + w[1]) + (w[2] + w[3])) + ((w[4] + w[5]) + (w[6] + w[7]));
+    }
+    if (t == 0) out[((int64_t)d * n_bands + b) * n_levels + j] = s * scale;
 }
 
 // out[j] = scale * sum over the n_parts CTAs, in CTA order, of their level-j partials.

@@ -75,9 +75,10 @@ def assemble(gathered, plan):
 
 
 def sum_over_ranks(values, dist=None):
-    """Sum of a small float64 vector over the ranks -- e.g. the level fluxes of Engine.atmosphere_fluxes, of which every
-    rank holds its wavenumber chunk's share.  ONE all_gather, then the ranks' vectors added in rank order on every rank,
-    so the result is deterministic and the same everywhere (an all_reduce leaves the order to the backend)."""
+    """Sum of a small float64 array of any shape over the ranks -- e.g. the level fluxes of Engine.atmosphere_fluxes or
+    the (n_bands, L+1) band fluxes of Engine.atmosphere_band_fluxes, of which every rank holds its wavenumber chunk's
+    share.  ONE all_gather, then the ranks' arrays added in rank order on every rank, so the result is deterministic and
+    the same everywhere (an all_reduce leaves the order to the backend)."""
     import torch
     v = torch.as_tensor(np.ascontiguousarray(values, dtype=np.float64))
     if dist is None or dist.get_world_size() == 1:

@@ -472,6 +472,22 @@ class Engine:
                                                    rd.ctypes.data_as(fp) if rows else None))
         return (up, down, ru, rd) if rows else (up, down)
 
+    def atmosphere_band_fluxes(self, mu, weights, edges):
+        """Band fluxes of the last column (prb_atmosphere_band_fluxes): the fluxes of atmosphere_fluxes split by the
+        wavenumber bands edges[b] <= nu < edges[b+1] (cm-1, strictly ascending; nu the column's linspace axis).  Returns
+        (band_up, band_down), float64 W m-2 of shape (n_bands, L+1): level 0 = surface, L = top; this chunk's share."""
+        m, w, ed = _f64(np.atleast_1d(mu)), _f64(np.atleast_1d(weights)), _f64(np.atleast_1d(edges))
+        if m.ndim != 1 or m.shape != w.shape:
+            raise ValueError("atmosphere_band_fluxes: mu and weights must be 1-d arrays of one length")
+        if ed.ndim != 1:
+            raise ValueError("atmosphere_band_fluxes: edges must be a 1-d array")
+        L = int(getattr(self, "atm_layers", 0))
+        nb = max(ed.size - 1, 0)
+        up, down = np.zeros((nb, L + 1)), np.zeros((nb, L + 1))
+        _lib.check(self._lib.prb_atmosphere_band_fluxes(self._h, m.size, _dp(m), _dp(w), ed.size - 1, _dp(ed),
+                                                        _dp(up) if up.size else None, _dp(down) if down.size else None))
+        return up, down
+
     def set_result_host(self, rad=None, tr=None):
         """Register pinned float32 host arrays that every following atmosphere() fills directly from the device
         kernels (zero-copy); call with no arguments to switch it off."""

@@ -5,7 +5,10 @@ flux call for 1, 2, 3 and 4 angular nodes (Gauss-Legendre on [0, 1]) on the same
 engine stream around each call (the layer-table upload, the upward and downward k3_flux_tma passes, the two k3_flux_sum
 launches and the copy of the level fluxes), warm-up first, then --reps calls.  Also reports the algorithmic bytes (the
 k matrix read once per pass, L N 4 bytes, two passes) and their rate against prb_measure_peaks' copy bandwidth, and the
-device name and power limit read in the same run.  Prints one JSON line; writes nothing.
+device name and power limit read in the same run.  Then times prb_atmosphere_band_fluxes with 3 nodes on the same
+k matrix, for four band sets -- one band over the whole grid, RRTMG's 16 longwave bands, 5000 bands of 1 cm-1 and the
+single band 630-700 cm-1 -- and reports each beside the 3-node total call of the same run.  Prints one JSON line;
+writes nothing.
 
     python scripts/flux_bench.py [--reps 30] [--warmup 3]
 """
@@ -93,6 +96,24 @@ def main():
             "share_of_copy_bandwidth": 2 * pass_bytes / (med * 1e-3) / peaks["copy_bytes_per_s"],
             "share_of_atmosphere": med / float(np.median(atm_ms)),
             "olr_w_m2": float(up[-1]), "surface_down_w_m2": float(down[0])})
+    x, wt = np.polynomial.legendre.leggauss(3)
+    mu, wt = (x + 1) / 2, wt / 2
+    total_ms = next(f["ms_median"] for f in out["fluxes"] if f["n_mu"] == 3)
+    band_sets = {"whole_grid": [w["range_min"], w["range_max"] + w["res"]],
+                 "rrtmg_lw_16": [10, 350, 500, 630, 700, 820, 980, 1080, 1180, 1390, 1480, 1800, 2080, 2250, 2380,
+                                 2600, 3250],
+                 "one_cm_5000": np.arange(0.0, 5001.0),
+                 "co2_630_700": [630.0, 700.0]}
+    out["band_fluxes"] = []
+    for name, edges in band_sets.items():
+        edges = np.asarray(edges, dtype=np.float64)
+        ms = timed(stream, lambda: e.atmosphere_band_fluxes(mu, wt, edges), args.warmup, args.reps)
+        med = float(np.median(ms))
+        bu, _ = e.atmosphere_band_fluxes(mu, wt, edges)
+        out["band_fluxes"].append({
+            "bands": name, "n_bands": len(edges) - 1, "n_mu": 3, "ms_median": med,
+            "ms_p10_p90": [float(np.percentile(ms, 10)), float(np.percentile(ms, 90))], "reps": args.reps,
+            "ratio_to_total_call": med / total_ms, "olr_w_m2": float(bu[:, -1].sum())})
     e.close()
     print(json.dumps(out))
 
