@@ -22,6 +22,7 @@
  *   (absent upstream, SURVEY 3.5) multi-layer fold of Layer.transmission   -> prb_atmosphere
  *   (absent upstream) hemispheric fluxes, downwelling and slant radiances of the column -> prb_atmosphere_fluxes
  *   (absent upstream) the column's fluxes per wavenumber band, at every level      -> prb_atmosphere_band_fluxes
+ *   (absent upstream) a grey or spectral surface and a warm top for both flux calls -> prb_set_flux_boundaries
  *
  * Conventions: every entry point is extern "C", returns int (0 = PRB_OK, < 0 = error) unless
  * noted, takes plain pointers and sizes.  Pointers named *_host / unmarked are caller-owned host
@@ -263,7 +264,8 @@ int prb_atmosphere_launches(prb_engine *e);              /* kernels launched by 
 /* Hemispheric fluxes and slant radiances of the last column (prb_atmosphere or prb_gas_cell_host), on the owned chunk,
  * from its device-resident k matrix.  For every node i of an angular quadrature (mu[i] in (0, 1], weight[i] > 0,
  * 1 <= n_mu <= 4) the fold I <- T I + (1 - T) B(nu, t[l]), T = exp(-k_l depth_l / mu[i]), runs up from B(nu, t_surface)
- * and down from 0 (no cosmic background, no solar source).  Level j is the boundary below layer j: 0 = surface, L = top.
+ * and down from 0 (a black surface, nothing from above, no solar source; prb_set_flux_boundaries changes the first two).
+ * Level j is the boundary below layer j: 0 = surface, L = top.
  * flux_up / flux_down: L+1 doubles each, F[j] = 2 pi sum_i weight[i] mu[i] sum_nu I_i(nu, level j) res over this chunk
  * (NaN -- the 0 cm^-1 point -- counts as 0, as in integrateSpectrum, and so does +-inf: next to 0 cm^-1 the reference's
  * negative Doppler widths can make k < 0 and the FP32 transmittance overflow; with wavenumber chunks the ranks' values add up).
@@ -282,6 +284,20 @@ int prb_atmosphere_fluxes(prb_engine *e, int32_t n_mu, const double *mu, const d
  * aligned to 128 points).  Under a peer connection the call stays local. */
 int prb_atmosphere_band_fluxes(prb_engine *e, int32_t n_mu, const double *mu, const double *weight,
                                int32_t n_bands, const double *edges, double *band_up, double *band_down);
+/* The two boundaries of every later prb_atmosphere_fluxes and prb_atmosphere_band_fluxes call, until changed (independent
+ * of the grid; prb_atmosphere keeps them).  Top (level L), every node: I = B(nu, t_top), 0 when t_top = 0.  Surface
+ * (level 0), node i: I = eps(nu) B(nu, t_surface) + (1 - eps(nu)) S_i, with eps(x) = np.interp(x, table_nu,
+ * table_emissivity) on the Planck axis x (FP64, rounded to FP32; one entry: a constant; n_table = 0: eps = 1 and the
+ * pointers may be NULL).  PRB_REFLECT_LAMBERTIAN: S_i = 2 sum_j weight[j] mu[j] I_down_j(nu, 0), the same for every
+ * node; PRB_REFLECT_SPECULAR: S_i = I_down_i(nu, 0).  Where eps = 1 the surface value is B(nu, t_surface) bit for bit,
+ * and with t_top = 0 the downward results are those without boundaries bit for bit.  (0, NULL, NULL, 0, 0.0) restores
+ * a black surface and 0 at the top.  table_nu must be finite and strictly ascending, every emissivity finite and in
+ * [0, 1], reflection one of the two constants, t_top finite and >= 0; otherwise PRB_ERR_ARG and the previous setting
+ * stays.  prb_atmosphere's own nadir radiance is not affected: its fold always starts from a black surface. */
+#define PRB_REFLECT_LAMBERTIAN 0
+#define PRB_REFLECT_SPECULAR   1
+int prb_set_flux_boundaries(prb_engine *e, int64_t n_table, const double *table_nu, const double *table_emissivity,
+                            int32_t reflection, double t_top);
 int prb_set_option(prb_engine *e, int option, int64_t value);
 
 /* ---- section 8(f) rows beside the hot path -------------------------------------------------------

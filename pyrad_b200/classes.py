@@ -868,7 +868,8 @@ class Atmosphere(list):
         stay resident on the device and enter every layer's k(nu) inside the line-sum kernel (prb_xsc_resident)."""
         return self._column(surfaceTemperature, lambda e: e.atmosphere_read())
 
-    def columnFluxes(self, surfaceTemperature, mu=None, weights=None, bands=None):
+    def columnFluxes(self, surfaceTemperature, mu=None, weights=None, bands=None, surfaceEmissivity=None,
+                     reflection="lambertian", topTemperature=0.0):
         """Hemispheric fluxes, heating rates and slant radiances of the column (prb_atmosphere, then
         prb_atmosphere_fluxes on its device-resident k matrix; same requirements on the layers as columnSpectrum).
         For every node mu_i of the angular quadrature (default: 3-node Gauss-Legendre on [0, 1]; at most 4 nodes) the
@@ -882,7 +883,13 @@ class Atmosphere(list):
         bands: optional band edges in cm-1 (1-d, at least 2, finite, strictly ascending); a grid point nu belongs to band
         b when bands[b] <= nu < bands[b+1] (prb_atmosphere_band_fluxes, on the same column run).  The dict then also holds
         band_edges, band_flux_up and band_flux_down (n_bands, L+1), band_net, and band_heating_rate (n_bands, L): each
-        band's heating rate by heatingRate."""
+        band's heating rate by heatingRate.
+        surfaceEmissivity, reflection, topTemperature: the column's boundaries for this call (Engine.set_flux_boundaries).
+        surfaceEmissivity is None (black), a scalar, or a pair (nu, eps) of 1-d arrays interpolated onto the grid (np.interp);
+        the surface then emits eps B(nu, surfaceTemperature) and reflects 1 - eps of the downward radiance, diffusely
+        ("lambertian") or along the same mu ("specular").  topTemperature > 0 sends B(nu, topTemperature) down from the top
+        (2.725 for the cosmic background).  The defaults give the result described above, bit for bit."""
+        _eng.flux_boundary_args(surfaceEmissivity, reflection, topTemperature)      # ValueError before the column runs
         if mu is None and weights is None:
             x, w = np.polynomial.legendre.leggauss(3)
             mu, weights = (x + 1) / 2, w / 2
@@ -895,8 +902,12 @@ class Atmosphere(list):
                 raise ValueError("columnFluxes: bands must be a 1-d array of at least 2 finite, strictly ascending edges")
 
         def result(e):
-            return (e.atmosphere_fluxes(mu, weights, rows=True),
-                    e.atmosphere_band_fluxes(mu, weights, bands) if bands is not None else None)
+            e.set_flux_boundaries(surfaceEmissivity, reflection, topTemperature)
+            try:
+                return (e.atmosphere_fluxes(mu, weights, rows=True),
+                        e.atmosphere_band_fluxes(mu, weights, bands) if bands is not None else None)
+            finally:
+                e.set_flux_boundaries()
 
         (up, down, ru, rd), band = self._column(surfaceTemperature, result)
         layers = list(self)

@@ -219,6 +219,12 @@ struct prb_engine {
     DevBuf<float> flux_rows;
     DevBuf<double> band_part, band_out;               // prb_atmosphere_band_fluxes: per-segment level sums, band totals
     DevBuf<int32_t> band_tab;                         // its span, segment, band and strip tables
+    // the flux calls' boundaries (prb_set_flux_boundaries); an empty table and t_top = 0: a black surface, 0 at the top
+    std::vector<double> bnd_tab;                      // table_nu | table_emissivity
+    int bnd_reflection = PRB_REFLECT_LAMBERTIAN;
+    double bnd_t_top = 0;
+    DevBuf<double> bnd_tab_dev;
+    DevBuf<float> flux_eps;                           // the emissivity on the owned chunk
     // optional stage timing of prb_atmosphere (CUDA events on the engine stream)
     bool timing = false;
     std::vector<cudaEvent_t> ev;
@@ -315,6 +321,7 @@ extern "C" int prb_destroy(prb_engine *e) {
     e->kmat.release(); e->rad.release(); e->trans.release(); e->fold.release();
     e->flux_layers.release(); e->flux_part.release(); e->flux_out.release(); e->flux_rows.release();
     e->band_part.release(); e->band_out.release(); e->band_tab.release();
+    e->bnd_tab_dev.release(); e->flux_eps.release();
     e->k2tab.release(); e->ring_d.release(); e->peer_err.release();
     if (e->blk_h) cudaFreeHost(e->blk_h);
     if (e->read_stage) cudaFreeHost(e->read_stage);
@@ -1800,9 +1807,9 @@ extern "C" int prb_atmosphere_read_f32(prb_engine *e, float *radiance_host, floa
 }
 
 // One flux pass (k3_flux_tma) over the resident k matrix; its level sums (per CTA, or per segment for BAND) go to a.part.
-template <int NMU, bool DOWN, bool BAND = false>
+template <int NMU, bool DOWN, bool BAND = false, bool BOUND = false>
 static cudaError_t launch_flux(prb_engine *e, int grid, size_t smem, double dx, const K3FArgs &a) {
-    const auto fn = k3_flux_tma<NMU, DOWN, BAND>;
+    const auto fn = k3_flux_tma<NMU, DOWN, BAND, BOUND>;
     cudaError_t ce = cudaFuncSetAttribute((const void *)fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (ce != cudaSuccess) return ce;
     const double c2 = 100 * hPlanck * cLight / kBoltz;
@@ -1812,21 +1819,62 @@ static cudaError_t launch_flux(prb_engine *e, int grid, size_t smem, double dx, 
     return cudaGetLastError();
 }
 
-template <int NMU, bool BAND = false>
+template <int NMU, bool BAND = false, bool BOUND = false>
 static cudaError_t launch_flux_pair(prb_engine *e, int grid, size_t smem, double dx, const K3FArgs &up, const K3FArgs &down) {
+    if constexpr (BOUND) {                             // the upward pass reflects the downward pass's surface rows
+        cudaError_t ce = launch_flux<NMU, true, BAND, true>(e, grid, smem, dx, down);
+        return ce != cudaSuccess ? ce : launch_flux<NMU, false, BAND, true>(e, grid, smem, dx, up);
+    }
     cudaError_t ce = launch_flux<NMU, false, BAND>(e, grid, smem, dx, up);
     return ce != cudaSuccess ? ce : launch_flux<NMU, true, BAND>(e, grid, smem, dx, down);
 }
 
+template <bool BAND, bool BOUND>
+static cudaError_t launch_flux_nodes(prb_engine *e, int n_mu, int grid, size_t smem, double dx, const K3FArgs &up,
+                                     const K3FArgs &down) {
+    switch (n_mu) {
+        case 1: return launch_flux_pair<1, BAND, BOUND>(e, grid, smem, dx, up, down);
+        case 2: return launch_flux_pair<2, BAND, BOUND>(e, grid, smem, dx, up, down);
+        case 3: return launch_flux_pair<3, BAND, BOUND>(e, grid, smem, dx, up, down);
+        default: return launch_flux_pair<4, BAND, BOUND>(e, grid, smem, dx, up, down);
+    }
+}
+
+// A black surface and nothing from the top: the plain passes.
+static bool flux_bounded(const prb_engine *e) { return !e->bnd_tab.empty() || e->bnd_t_top > 0; }
+
 template <bool BAND>
 static cudaError_t launch_flux_passes(prb_engine *e, int n_mu, int grid, size_t smem, double dx, const K3FArgs &up,
                                       const K3FArgs &down) {
-    switch (n_mu) {
-        case 1: return launch_flux_pair<1, BAND>(e, grid, smem, dx, up, down);
-        case 2: return launch_flux_pair<2, BAND>(e, grid, smem, dx, up, down);
-        case 3: return launch_flux_pair<3, BAND>(e, grid, smem, dx, up, down);
-        default: return launch_flux_pair<4, BAND>(e, grid, smem, dx, up, down);
-    }
+    return flux_bounded(e) ? launch_flux_nodes<BAND, true>(e, n_mu, grid, smem, dx, up, down)
+                           : launch_flux_nodes<BAND, false>(e, n_mu, grid, smem, dx, up, down);
+}
+
+// With boundaries set: the emissivity on the chunk (k3_flux_emissivity, every call: the table is tiny), the downward
+// pass's surface rows whether or not the caller reads them, and the boundary fields of both passes' arguments.
+static cudaError_t flux_boundaries_prepare(prb_engine *e, double dx, K3FArgs &up, K3FArgs &down) {
+    if (!flux_bounded(e)) return cudaSuccess;
+    const int64_t nc = chunk_len(e);
+    const std::vector<double> black{0.0, 1.0};        // no table: eps = 1 everywhere
+    const std::vector<double> &tab = e->bnd_tab.empty() ? black : e->bnd_tab;
+    const int64_t n_tab = (int64_t)tab.size() / 2;
+    cudaError_t ce;
+    if ((ce = e->flux_rows.ensure((size_t)2 * 4 * e->kmat_ld)) != cudaSuccess) return ce;
+    if ((ce = e->flux_eps.ensure((size_t)e->kmat_ld)) != cudaSuccess) return ce;
+    if ((ce = e->bnd_tab_dev.ensure(tab.size())) != cudaSuccess) return ce;
+    ce = cudaMemcpyAsync(e->bnd_tab_dev.p, tab.data(), sizeof(double) * tab.size(), cudaMemcpyHostToDevice, e->stream);
+    if (ce != cudaSuccess) return ce;
+    const unsigned blocks = (unsigned)std::min<int64_t>((nc + 255) / 256, 8 * (int64_t)e->prop.multiProcessorCount);
+    k3_flux_emissivity<<<blocks, 256, 0, e->stream>>>(nc, e->i_begin, e->n_total, e->range_min, dx, e->atm_range_max,
+                                                      e->bnd_tab_dev.p, n_tab, e->flux_eps.p);
+    if ((ce = cudaGetLastError()) != cudaSuccess) return ce;
+    down.rows = e->flux_rows.p + (size_t)4 * e->kmat_ld;
+    down.ld_rows = up.ld_rows = e->kmat_ld;
+    down.c2_over_ttop = e->bnd_t_top > 0 ? (float)(100 * hPlanck * cLight / kBoltz / e->bnd_t_top) : 0.f;
+    up.eps = e->flux_eps.p;
+    up.surf_down = down.rows;
+    up.specular = e->bnd_reflection == PRB_REFLECT_SPECULAR;
+    return cudaSuccess;
 }
 
 // The checks shared by the flux calls: a column on the device, a quadrature of 1 to 4 nodes with mu in (0, 1] and finite
@@ -1889,6 +1937,7 @@ extern "C" int prb_atmosphere_fluxes(prb_engine *e, int32_t n_mu, const double *
     down.rows = rows ? e->flux_rows.p + (size_t)4 * e->kmat_ld : nullptr;
     up.part = e->flux_part.p;
     down.part = e->flux_part.p + (size_t)grid * n_levels;
+    CK(flux_boundaries_prepare(e, flux_dx(e), up, down));
     const cudaError_t ce = launch_flux_passes<false>(e, n_mu, grid, smem, flux_dx(e), up, down);
     if (ce != cudaSuccess) return fail(PRB_ERR_CUDA, std::string("k3_flux_tma launch failed: ") + cudaGetErrorString(ce));
     // F[j] = 2 pi sum_i w_i mu_i sum_nu I_i(nu, j) res  (integrateSpectrum's res and NaN rule, pyradClasses.py:26-29)
@@ -2001,6 +2050,7 @@ extern "C" int prb_atmosphere_band_fluxes(prb_engine *e, int32_t n_mu, const dou
     }
     up.part = e->band_part.p;
     down.part = e->band_part.p + (size_t)n_levels * n_seg;
+    CK(flux_boundaries_prepare(e, dx, up, down));
     const int grid = (int)std::min<int64_t>((int64_t)strips.size(), k3f_minb(n_mu) * (int64_t)e->prop.multiProcessorCount);
     const cudaError_t ce = launch_flux_passes<true>(e, n_mu, grid, sizeof(K3FSmem), dx, up, down);
     if (ce != cudaSuccess) return fail(PRB_ERR_CUDA, std::string("k3_flux_tma launch failed: ") + cudaGetErrorString(ce));
@@ -2019,6 +2069,28 @@ extern "C" int prb_atmosphere_band_fluxes(prb_engine *e, int32_t n_mu, const dou
     if (band_down)
         CK(cudaMemcpyAsync(band_down, e->band_out.p + per_dir, sizeof(double) * per_dir, cudaMemcpyDeviceToHost, e->stream));
     CK(cudaStreamSynchronize(e->stream));
+    return PRB_OK;
+}
+
+extern "C" int prb_set_flux_boundaries(prb_engine *e, int64_t n_table, const double *table_nu,
+                                       const double *table_emissivity, int32_t reflection, double t_top) {
+    if (!e) return fail(PRB_ERR_ARG, "null engine");
+    if (n_table < 0 || (n_table > 0 && (!table_nu || !table_emissivity)))
+        return fail(PRB_ERR_ARG, "prb_set_flux_boundaries: need n_table >= 0 and both tables when n_table > 0");
+    for (int64_t i = 0; i < n_table; ++i) {
+        if (!std::isfinite(table_nu[i]) || (i > 0 && !(table_nu[i] > table_nu[i - 1])))
+            return fail(PRB_ERR_ARG, "prb_set_flux_boundaries: table_nu must be finite and strictly ascending");
+        if (!(table_emissivity[i] >= 0 && table_emissivity[i] <= 1))
+            return fail(PRB_ERR_ARG, "prb_set_flux_boundaries: every emissivity must lie in [0, 1]");
+    }
+    if (reflection != PRB_REFLECT_LAMBERTIAN && reflection != PRB_REFLECT_SPECULAR)
+        return fail(PRB_ERR_ARG, "prb_set_flux_boundaries: reflection must be PRB_REFLECT_LAMBERTIAN or PRB_REFLECT_SPECULAR");
+    if (!(std::isfinite(t_top) && t_top >= 0))
+        return fail(PRB_ERR_ARG, "prb_set_flux_boundaries: t_top must be finite and >= 0");
+    e->bnd_tab.assign(table_nu, table_nu + n_table);
+    e->bnd_tab.insert(e->bnd_tab.end(), table_emissivity, table_emissivity + n_table);
+    e->bnd_reflection = reflection;
+    e->bnd_t_top = t_top;
     return PRB_OK;
 }
 

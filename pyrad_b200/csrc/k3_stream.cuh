@@ -451,6 +451,12 @@ k3_fold_tma(const float *__restrict__ kmat, int64_t ld, int n_layers, const Fold
 // part[level][segment].  The CTA walks the host's list of strips that meet a band, and k3_flux_band_sum adds each band's
 // segments in position order with a tree whose shape depends only on their count: the result depends on the edges and
 // the span positions only, not on the launch grid.
+//
+// Boundaries (BOUND = true, prb_set_flux_boundaries): only the start values of the two passes change.  The downward pass
+// starts from B(nu, T_top) at level L (0 when T_top = 0) and adds that level's sum.  It runs first and writes its surface
+// rows.  The upward pass starts each strip from eps B(nu, T_s) + (1 - eps) S_i, S_i the radiance the surface reflects
+// along mu_i: Lambertian S = sum_j 2 w_j mu_j I_down_j(nu, 0) (FP32, node order), specular S_i = I_down_i(nu, 0).  Where
+// eps = 1 the start is B(nu, T_s) bit for bit, whatever comes down.  The layer loop is the fold's.
 struct FluxLayer {
     float c2_over_t;         // 100 h c / kB / T_layer
     float nd[4];             // -depth log2(e) / mu_i: T_i = exp2(k * nd[i])
@@ -472,6 +478,11 @@ struct K3FArgs {
     const K3FSpan *spans;    // per span of the chunk, 8 per strip (a ragged last strip padded with empty spans)
     const uint32_t *seg_range;   // per segment: its points within the span, [lo, hi) as lo | hi << 16 (0 <= lo < hi <= 128)
     int64_t ld_part;         // the number of segments
+    // boundaries only
+    const float *eps;        // upward pass: the surface emissivity on the chunk
+    const float *surf_down;  // upward pass: [NMU][ld_rows], the downward pass's radiance reaching the surface
+    int32_t specular;        // upward pass: 1 specular reflection, 0 Lambertian
+    float c2_over_ttop;      // downward pass: 100 h c / kB / T_top; 0: I = 0 at level L
 };
 
 constexpr int K3F_WARPS = K3T_THREADS / 32;
@@ -488,7 +499,7 @@ __host__ __device__ constexpr size_t k3f_smem_bytes(int n_layers) {
     return sizeof(K3FSmem) + sizeof(double) * K3F_WARPS * (size_t)(n_layers + 1);
 }
 
-template <int NMU, bool DOWN, bool BAND = false>
+template <int NMU, bool DOWN, bool BAND = false, bool BOUND = false>
 __global__ void __launch_bounds__(K3T_THREADS, k3f_minb(NMU))
 k3_flux_tma(const float *__restrict__ kmat, int64_t ld, int n_layers, const FluxLayer *__restrict__ layers,
             int64_t n_chunk, int64_t i_begin, int64_t n_total, double x0, double dx, double x_last,
@@ -611,6 +622,37 @@ k3_flux_tma(const float *__restrict__ kmat, int64_t ld, int n_layers, const Flux
         if constexpr (BAND) band_add(level);
         else level_add(partial(), level);
     };
+    // boundaries, upward pass: rad holds B(nu, T_s); make it eps B + (1 - eps) S_i (points outside the chunk keep B)
+    auto surface_start = [&]() {
+        float eps[4] = {1.f, 1.f, 1.f, 1.f}, dn[NMU][4];
+        if (n_valid == 4) {
+            const float4 e4 = *reinterpret_cast<const float4 *>(a.eps + i0);
+            eps[0] = e4.x; eps[1] = e4.y; eps[2] = e4.z; eps[3] = e4.w;
+#pragma unroll
+            for (int i = 0; i < NMU; ++i) {
+                const float4 d4 = *reinterpret_cast<const float4 *>(a.surf_down + (int64_t)i * a.ld_rows + i0);
+                dn[i][0] = d4.x; dn[i][1] = d4.y; dn[i][2] = d4.z; dn[i][3] = d4.w;
+            }
+        } else {
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+                if (q < n_valid) eps[q] = a.eps[i0 + q];
+#pragma unroll
+                for (int i = 0; i < NMU; ++i) dn[i][q] = q < n_valid ? a.surf_down[(int64_t)i * a.ld_rows + i0 + q] : 0.f;
+            }
+        }
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+            float s = 0.f;                             // Lambertian: F_down / pi = sum_j 2 w_j mu_j I_down_j
+#pragma unroll
+            for (int j = 0; j < NMU; ++j) s = fmaf(2.f * a.wmu[j], dn[j][q], s);
+#pragma unroll
+            for (int i = 0; i < NMU; ++i) {
+                const float sv = a.specular ? dn[i][q] : s;
+                rad[i][q] = eps[q] == 1.f ? rad[i][q] : fmaf(eps[q], rad[i][q], (1.f - eps[q]) * sv);
+            }
+        }
+    };
     for (int64_t step = 0; step < n_steps; ++step) {
         const int slot = (int)(step % K3T_SLOTS);
         const int g = group_of(step);
@@ -623,13 +665,16 @@ k3_flux_tma(const float *__restrict__ kmat, int64_t ld, int n_layers, const Flux
                 const double x = axis_value(i_begin + i0 + q, n_total, x0, dx, x_last);
                 nu[q] = (float)x;
                 a3[q] = (float)(2E8 * hPlanck * (cLight * cLight) * (x * x * x));
-                const float r0 = DOWN ? 0.f : planck_f32(a3[q], c2_over_tsurf * nu[q]);
+                float r0 = DOWN ? 0.f : planck_f32(a3[q], c2_over_tsurf * nu[q]);
+                if constexpr (BOUND && DOWN)
+                    if (a.c2_over_ttop > 0.f) r0 = planck_f32(a3[q], a.c2_over_ttop * nu[q]);   // B(nu, T_top)
 #pragma unroll
                 for (int i = 0; i < NMU; ++i) rad[i][q] = r0;
             }
+            if constexpr (BOUND && !DOWN) surface_start();
             interp = nu[0] >= nu_interp_min;
-            if (!DOWN) add_level(0);                   // (the downward pass starts from 0 at level L)
-            else if (BAND) add_level(n_layers);        // (whose segment slots must still be written: zeros)
+            if (!DOWN) add_level(0);                   // (the plain downward pass starts from 0 at level L,
+            else if (BAND || BOUND) add_level(n_layers);   // whose band segment slots must still be written: zeros)
         }
         if (tid == 0 && step + K3T_SLOTS - 1 < n_steps) issue(step + K3T_SLOTS - 1);
         mbar_wait(&sm.full[slot], (uint32_t)((step / K3T_SLOTS) & 1));
@@ -676,6 +721,15 @@ k3_flux_tma(const float *__restrict__ kmat, int64_t ld, int n_layers, const Flux
             a.part[(int64_t)blockIdx.x * n_levels + j] = s;
         }
     }
+}
+
+// Surface emissivity of the boundaries on the owned chunk: eps[i] = np.interp(x, table_nu, table_eps) in FP64 (numpy's
+// arithmetic), rounded to FP32; x the Planck axis of the fold.  tab = table_nu | table_eps, n_tab entries each.
+__global__ void __launch_bounds__(256)
+k3_flux_emissivity(int64_t n_chunk, int64_t i_begin, int64_t n_total, double x0, double dx, double x_last,
+                   const double *__restrict__ tab, int64_t n_tab, float *__restrict__ eps) {
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_chunk; i += (int64_t)gridDim.x * blockDim.x)
+        eps[i] = (float)np_interp(axis_value(i_begin + i, n_total, x0, dx, x_last), tab, tab + n_tab, n_tab);
 }
 
 // Band totals of the band pass: out[d][b][j] = scale * sum of band b's segments at level j of pass d (0 up, 1 down), for

@@ -12,6 +12,7 @@ OUT_F64, OUT_F32 = 0, 1
 K2_GENERAL, K2_CLASSED, K2_FARFIELD = 0, 1, 2
 OPT_BATCH_LAYERS, OPT_FUSE_SINGLE_LAYER, OPT_RECORD_BUDGET_MB, OPT_POINT_KERNEL, OPT_FOLD_TMA, OPT_SPLIT_TILES = 1, 2, 3, 4, 5, 6
 PEER_HANDLE_BYTES = 64
+REFLECTIONS = {"lambertian": 0, "specular": 1}       # PRB_REFLECT_LAMBERTIAN, PRB_REFLECT_SPECULAR
 
 
 def _f64(a):
@@ -120,6 +121,34 @@ def grid_len(range_min, range_max, res):
 def number_density_weight(conc, P, T):
     """absCoef factor conc * P / 1E4 / k / T, left to right (pyradClasses.py:583)."""
     return conc * P / 1E4 / K_BOLTZ / T
+
+
+def flux_boundary_args(emissivity=None, reflection="lambertian", t_top=0.0):
+    """Checked arguments of prb_set_flux_boundaries: (table_nu, table_emissivity, reflection code, t_top).
+
+    emissivity: None (a black surface: an empty table), a scalar (a one-entry table: a constant), or a pair (nu, eps) of
+    1-d arrays of one length, nu in cm-1 finite and strictly ascending; every emissivity finite and in [0, 1].
+    reflection: "lambertian" or "specular"; t_top: the top's temperature in K, finite and >= 0.  ValueError otherwise."""
+    if emissivity is None:
+        nu, eps = np.zeros(0), np.zeros(0)
+    elif np.ndim(emissivity) == 0:
+        nu, eps = np.zeros(1), np.array([float(emissivity)])
+    else:
+        if len(emissivity) != 2:
+            raise ValueError("emissivity must be None, a scalar or a pair (nu, eps)")
+        nu, eps = _f64(emissivity[0]), _f64(emissivity[1])
+        if nu.ndim != 1 or nu.shape != eps.shape or nu.size < 1:
+            raise ValueError("emissivity: nu and eps must be 1-d arrays of one length, at least one entry")
+        if not np.all(np.isfinite(nu)) or not np.all(np.diff(nu) > 0):
+            raise ValueError("emissivity: nu must be finite and strictly ascending")
+    if not np.all((eps >= 0) & (eps <= 1)):
+        raise ValueError("emissivity must be finite and in [0, 1]")
+    if not isinstance(reflection, str) or reflection not in REFLECTIONS:
+        raise ValueError("reflection must be one of %s" % sorted(REFLECTIONS))
+    t_top = float(t_top)
+    if not (np.isfinite(t_top) and t_top >= 0):
+        raise ValueError("t_top must be finite and >= 0")
+    return nu, eps, REFLECTIONS[reflection], t_top
 
 
 class Engine:
@@ -487,6 +516,16 @@ class Engine:
         _lib.check(self._lib.prb_atmosphere_band_fluxes(self._h, m.size, _dp(m), _dp(w), ed.size - 1, _dp(ed),
                                                         _dp(up) if up.size else None, _dp(down) if down.size else None))
         return up, down
+
+    def set_flux_boundaries(self, emissivity=None, reflection="lambertian", t_top=0.0):
+        """The surface and top boundaries of every later atmosphere_fluxes / atmosphere_band_fluxes call
+        (prb_set_flux_boundaries; arguments as flux_boundary_args).  The surface emits eps(nu) B(nu, T_surface) and
+        reflects 1 - eps(nu) of the sky's radiance, diffusely (Lambertian) or along the same mu (specular); eps is
+        np.interp over the table on the column's grid.  The top sends B(nu, t_top) down.  No arguments: a black surface
+        and nothing from the top again.  The column's own radiance (atmosphere_read) is not affected."""
+        nu, eps, refl, t_top = flux_boundary_args(emissivity, reflection, t_top)
+        _lib.check(self._lib.prb_set_flux_boundaries(self._h, nu.size, _dp(nu) if nu.size else None,
+                                                     _dp(eps) if eps.size else None, refl, t_top))
 
     def set_result_host(self, rad=None, tr=None):
         """Register pinned float32 host arrays that every following atmosphere() fills directly from the device

@@ -7,8 +7,11 @@ launches and the copy of the level fluxes), warm-up first, then --reps calls.  A
 k matrix read once per pass, L N 4 bytes, two passes) and their rate against prb_measure_peaks' copy bandwidth, and the
 device name and power limit read in the same run.  Then times prb_atmosphere_band_fluxes with 3 nodes on the same
 k matrix, for four band sets -- one band over the whole grid, RRTMG's 16 longwave bands, 5000 bands of 1 cm-1 and the
-single band 630-700 cm-1 -- and reports each beside the 3-node total call of the same run.  Prints one JSON line;
-writes nothing.
+single band 630-700 cm-1 -- and reports each beside the 3-node total call of the same run.  Last, with the flux
+boundaries set (prb_set_flux_boundaries: emissivity 0.98 with a linear dip to 0.75 over 1080-1180 cm-1, the 2.725 K
+cosmic background at the top, Lambertian and specular reflection), times the 3-node total call and the 16-band call as
+ratios to the plain calls timed right before them, and reports the OLR and the net flux at the surface with and
+without the surface.  Prints one JSON line; writes nothing.
 
     python scripts/flux_bench.py [--reps 30] [--warmup 3]
 """
@@ -114,6 +117,30 @@ def main():
             "bands": name, "n_bands": len(edges) - 1, "n_mu": 3, "ms_median": med,
             "ms_p10_p90": [float(np.percentile(ms, 10)), float(np.percentile(ms, 90))], "reps": args.reps,
             "ratio_to_total_call": med / total_ms, "olr_w_m2": float(bu[:, -1].sum())})
+    # boundaries: a grey surface with a reststrahlen-like dip and the cosmic background at the top
+    eps_table = ([1080.0, 1130.0, 1180.0], [0.98, 0.75, 0.98])
+    rrtmg = np.asarray(band_sets["rrtmg_lw_16"], dtype=np.float64)
+    calls = {"total": lambda: e.atmosphere_fluxes(mu, wt), "rrtmg_lw_16": lambda: e.atmosphere_band_fluxes(mu, wt, rrtmg)}
+    e.set_flux_boundaries()
+    plain_ms = {k: float(np.median(timed(stream, f, args.warmup, args.reps))) for k, f in calls.items()}
+    up0, down0 = e.atmosphere_fluxes(mu, wt)
+    out["boundaries"] = {"emissivity_table": eps_table, "t_top_k": 2.725, "n_mu": 3, "plain_ms_median": plain_ms,
+                         "plain_olr_w_m2": float(up0[-1]), "plain_surface_net_w_m2": float(up0[0] - down0[0]),
+                         "runs": []}
+    try:
+        for reflection in ("lambertian", "specular"):
+            e.set_flux_boundaries(eps_table, reflection, 2.725)
+            run = {"reflection": reflection}
+            for k, f in calls.items():
+                ms = timed(stream, f, args.warmup, args.reps)
+                med = float(np.median(ms))
+                run[k] = {"ms_median": med, "ms_p10_p90": [float(np.percentile(ms, 10)), float(np.percentile(ms, 90))],
+                          "reps": args.reps, "ratio_to_plain_call": med / plain_ms[k]}
+            up, down = e.atmosphere_fluxes(mu, wt)
+            run.update(olr_w_m2=float(up[-1]), surface_net_w_m2=float(up[0] - down[0]), top_down_w_m2=float(down[-1]))
+            out["boundaries"]["runs"].append(run)
+    finally:
+        e.set_flux_boundaries()
     e.close()
     print(json.dumps(out))
 
