@@ -23,6 +23,7 @@
  *   (absent upstream) hemispheric fluxes, downwelling and slant radiances of the column -> prb_atmosphere_fluxes
  *   (absent upstream) the column's fluxes per wavenumber band, at every level      -> prb_atmosphere_band_fluxes
  *   (absent upstream) a grey or spectral surface and a warm top for both flux calls -> prb_set_flux_boundaries
+ *   (absent upstream) an absorbed, reflected solar beam for both flux calls        -> prb_set_solar_source
  *
  * Conventions: every entry point is extern "C", returns int (0 = PRB_OK, < 0 = error) unless
  * noted, takes plain pointers and sizes.  Pointers named *_host / unmarked are caller-owned host
@@ -264,7 +265,8 @@ int prb_atmosphere_launches(prb_engine *e);              /* kernels launched by 
 /* Hemispheric fluxes and slant radiances of the last column (prb_atmosphere or prb_gas_cell_host), on the owned chunk,
  * from its device-resident k matrix.  For every node i of an angular quadrature (mu[i] in (0, 1], weight[i] > 0,
  * 1 <= n_mu <= 4) the fold I <- T I + (1 - T) B(nu, t[l]), T = exp(-k_l depth_l / mu[i]), runs up from B(nu, t_surface)
- * and down from 0 (a black surface, nothing from above, no solar source; prb_set_flux_boundaries changes the first two).
+ * and down from 0 (a black surface, nothing from above, no solar source; prb_set_flux_boundaries changes the first two,
+ * prb_set_solar_source adds the Sun's beam to flux_down, and its reflection to flux_up).
  * Level j is the boundary below layer j: 0 = surface, L = top.
  * flux_up / flux_down: L+1 doubles each, F[j] = 2 pi sum_i weight[i] mu[i] sum_nu I_i(nu, level j) res over this chunk
  * (NaN -- the 0 cm^-1 point -- counts as 0, as in integrateSpectrum, and so does +-inf: next to 0 cm^-1 the reference's
@@ -298,6 +300,21 @@ int prb_atmosphere_band_fluxes(prb_engine *e, int32_t n_mu, const double *mu, co
 #define PRB_REFLECT_SPECULAR   1
 int prb_set_flux_boundaries(prb_engine *e, int64_t n_table, const double *table_nu, const double *table_emissivity,
                             int32_t reflection, double t_top);
+/* The Sun of every later prb_atmosphere_fluxes and prb_atmosphere_band_fluxes call, until changed (independent of the
+ * grid; prb_atmosphere keeps it, and its own nadir radiance is not affected).  A collimated beam along mu_sun =
+ * cos(solar zenith), absorbed and neither emitted into nor scattered: E(nu, L) = S(nu), E <- E exp(-k_l depth_l / mu_sun)
+ * through every layer going down.  S(x) = np.interp(x, table_nu, table_irradiance, left=0, right=0) on the Planck axis x
+ * (FP64, rounded to FP32), in W m^-2 (cm^-1)^-1 on a plane normal to the beam.  flux_down[j] and band_down gain
+ * mu_sun sum_nu E(nu, j) res at every level.  The surface reflects 1 - eps(nu) of the beam (eps of
+ * prb_set_flux_boundaries; none set: eps = 1, nothing reflected): PRB_REFLECT_LAMBERTIAN adds (1 - eps) mu_sun E(nu, 0) / pi
+ * to every node's upward start (so rad_up_top includes it); PRB_REFLECT_SPECULAR sends a beam (1 - eps) E(nu, 0) up
+ * along mu_sun through the same layer factors, and flux_up and band_up gain mu_sun sum E_up res at every level.  Neither
+ * beam is a node: rad_down_surface never changes.  n_table = 0 clears the Sun (the pointers may be NULL, mu_sun is
+ * ignored); n_table >= 2 sets it, with table_nu finite and strictly ascending, every irradiance finite and >= 0, and
+ * mu_sun in (0, 1]; otherwise PRB_ERR_ARG and the previous setting stays.  An all-zero table gives the results without
+ * the Sun bit for bit. */
+int prb_set_solar_source(prb_engine *e, int64_t n_table, const double *table_nu, const double *table_irradiance,
+                         double mu_sun);
 int prb_set_option(prb_engine *e, int option, int64_t value);
 
 /* ---- section 8(f) rows beside the hot path -------------------------------------------------------

@@ -81,6 +81,7 @@ PROTOTYPES = {
     "prb_atmosphere_fluxes": (C.c_int, [_vp, _i32, _dp, _dp, _dp, _dp, C.POINTER(C.c_float), C.POINTER(C.c_float)]),
     "prb_atmosphere_band_fluxes": (C.c_int, [_vp, _i32, _dp, _dp, _i32, _dp, _dp, _dp]),
     "prb_set_flux_boundaries": (C.c_int, [_vp, _i64, _dp, _dp, _i32, _d]),
+    "prb_set_solar_source": (C.c_int, [_vp, _i64, _dp, _dp, _d]),
     "prb_set_option": (C.c_int, [_vp, C.c_int, _i64]),
     "prb_line_survey": (C.c_int, [_vp, _i64, _dp]),
     "prb_integrate_spectrum": (C.c_int, [_vp, _i64, _dp, _d, _d, _dp]),

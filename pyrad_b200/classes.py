@@ -869,11 +869,11 @@ class Atmosphere(list):
         return self._column(surfaceTemperature, lambda e: e.atmosphere_read())
 
     def columnFluxes(self, surfaceTemperature, mu=None, weights=None, bands=None, surfaceEmissivity=None,
-                     reflection="lambertian", topTemperature=0.0):
+                     reflection="lambertian", topTemperature=0.0, solarIrradiance=None, solarMu=1.0):
         """Hemispheric fluxes, heating rates and slant radiances of the column (prb_atmosphere, then
         prb_atmosphere_fluxes on its device-resident k matrix; same requirements on the layers as columnSpectrum).
         For every node mu_i of the angular quadrature (default: 3-node Gauss-Legendre on [0, 1]; at most 4 nodes) the
-        fold runs up from B(nu, surfaceTemperature) and down from 0 (no cosmic background, no sun) with
+        fold runs up from B(nu, surfaceTemperature) and down from 0 (by default no cosmic background, no sun) with
         T = exp(-k_l depth_l / mu_i); level j is the boundary below layer j (0 = surface, len(self) = top), and
         F[j] = 2 pi sum_i w_i mu_i integrateSpectrum(I_i(level j), 1, res).  A column with opaque bands is not
         isotropic, so F_up at the top differs from the pi x nadir radiance of integrateSpectrum(columnSpectrum(...)[0]).
@@ -888,8 +888,16 @@ class Atmosphere(list):
         surfaceEmissivity is None (black), a scalar, or a pair (nu, eps) of 1-d arrays interpolated onto the grid (np.interp);
         the surface then emits eps B(nu, surfaceTemperature) and reflects 1 - eps of the downward radiance, diffusely
         ("lambertian") or along the same mu ("specular").  topTemperature > 0 sends B(nu, topTemperature) down from the top
-        (2.725 for the cosmic background).  The defaults give the result described above, bit for bit."""
+        (2.725 for the cosmic background).
+        solarIrradiance, solarMu: the Sun for this call (Engine.set_solar_source).  solarIrradiance is None (no Sun) or a
+        pair (nu, S) of 1-d arrays, S the irradiance at the top in W m-2 (cm-1)-1 normal to the beam, interpolated onto
+        the grid (np.interp, 0 outside the table); solarMu is the cosine of the solar zenith angle, in (0, 1].  The beam is
+        absorbed on its way down and 1 - eps of it is reflected as the surface says; flux_down, net, heating_rate and the
+        band arrays then include it (and flux_up its reflection).  The sunlight's share of any of them is the result with
+        the Sun minus the result without it: the column is linear in its sources.
+        The defaults give the result described above, bit for bit."""
         _eng.flux_boundary_args(surfaceEmissivity, reflection, topTemperature)      # ValueError before the column runs
+        _eng.solar_source_args(solarIrradiance, solarMu)
         if mu is None and weights is None:
             x, w = np.polynomial.legendre.leggauss(3)
             mu, weights = (x + 1) / 2, w / 2
@@ -904,9 +912,11 @@ class Atmosphere(list):
         def result(e):
             e.set_flux_boundaries(surfaceEmissivity, reflection, topTemperature)
             try:
+                e.set_solar_source(solarIrradiance, solarMu)
                 return (e.atmosphere_fluxes(mu, weights, rows=True),
                         e.atmosphere_band_fluxes(mu, weights, bands) if bands is not None else None)
             finally:
+                e.set_solar_source()
                 e.set_flux_boundaries()
 
         (up, down, ru, rd), band = self._column(surfaceTemperature, result)

@@ -225,6 +225,11 @@ struct prb_engine {
     double bnd_t_top = 0;
     DevBuf<double> bnd_tab_dev;
     DevBuf<float> flux_eps;                           // the emissivity on the owned chunk
+    // the flux calls' solar beam (prb_set_solar_source); an empty table: no Sun
+    std::vector<double> sun_tab;                      // table_nu | table_irradiance
+    double sun_mu = 1;
+    DevBuf<double> sun_tab_dev;
+    DevBuf<float> sun_nd;                             // -depth_l log2(e) / mu_sun per layer
     // optional stage timing of prb_atmosphere (CUDA events on the engine stream)
     bool timing = false;
     std::vector<cudaEvent_t> ev;
@@ -322,6 +327,7 @@ extern "C" int prb_destroy(prb_engine *e) {
     e->flux_layers.release(); e->flux_part.release(); e->flux_out.release(); e->flux_rows.release();
     e->band_part.release(); e->band_out.release(); e->band_tab.release();
     e->bnd_tab_dev.release(); e->flux_eps.release();
+    e->sun_tab_dev.release(); e->sun_nd.release();
     e->k2tab.release(); e->ring_d.release(); e->peer_err.release();
     if (e->blk_h) cudaFreeHost(e->blk_h);
     if (e->read_stage) cudaFreeHost(e->read_stage);
@@ -1807,9 +1813,9 @@ extern "C" int prb_atmosphere_read_f32(prb_engine *e, float *radiance_host, floa
 }
 
 // One flux pass (k3_flux_tma) over the resident k matrix; its level sums (per CTA, or per segment for BAND) go to a.part.
-template <int NMU, bool DOWN, bool BAND = false, bool BOUND = false>
+template <int NMU, bool DOWN, bool BAND = false, bool BOUND = false, int SUN = K3F_NO_SUN>
 static cudaError_t launch_flux(prb_engine *e, int grid, size_t smem, double dx, const K3FArgs &a) {
-    const auto fn = k3_flux_tma<NMU, DOWN, BAND, BOUND>;
+    const auto fn = k3_flux_tma<NMU, DOWN, BAND, BOUND, SUN>;
     cudaError_t ce = cudaFuncSetAttribute((const void *)fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (ce != cudaSuccess) return ce;
     const double c2 = 100 * hPlanck * cLight / kBoltz;
@@ -1819,35 +1825,48 @@ static cudaError_t launch_flux(prb_engine *e, int grid, size_t smem, double dx, 
     return cudaGetLastError();
 }
 
-template <int NMU, bool BAND = false, bool BOUND = false>
+// SUN: the upward pass's solar variant (K3F_NO_SUN, K3F_SUN or K3F_SUN_SPECULAR); the downward pass carries the beam
+// whenever there is one.
+template <int NMU, bool BAND = false, bool BOUND = false, int SUN = K3F_NO_SUN>
 static cudaError_t launch_flux_pair(prb_engine *e, int grid, size_t smem, double dx, const K3FArgs &up, const K3FArgs &down) {
     if constexpr (BOUND) {                             // the upward pass reflects the downward pass's surface rows
-        cudaError_t ce = launch_flux<NMU, true, BAND, true>(e, grid, smem, dx, down);
-        return ce != cudaSuccess ? ce : launch_flux<NMU, false, BAND, true>(e, grid, smem, dx, up);
+        constexpr int SUN_DOWN = SUN == K3F_NO_SUN ? K3F_NO_SUN : K3F_SUN;
+        cudaError_t ce = launch_flux<NMU, true, BAND, true, SUN_DOWN>(e, grid, smem, dx, down);
+        return ce != cudaSuccess ? ce : launch_flux<NMU, false, BAND, true, SUN>(e, grid, smem, dx, up);
     }
     cudaError_t ce = launch_flux<NMU, false, BAND>(e, grid, smem, dx, up);
     return ce != cudaSuccess ? ce : launch_flux<NMU, true, BAND>(e, grid, smem, dx, down);
 }
 
-template <bool BAND, bool BOUND>
+template <bool BAND, bool BOUND, int SUN = K3F_NO_SUN>
 static cudaError_t launch_flux_nodes(prb_engine *e, int n_mu, int grid, size_t smem, double dx, const K3FArgs &up,
                                      const K3FArgs &down) {
     switch (n_mu) {
-        case 1: return launch_flux_pair<1, BAND, BOUND>(e, grid, smem, dx, up, down);
-        case 2: return launch_flux_pair<2, BAND, BOUND>(e, grid, smem, dx, up, down);
-        case 3: return launch_flux_pair<3, BAND, BOUND>(e, grid, smem, dx, up, down);
-        default: return launch_flux_pair<4, BAND, BOUND>(e, grid, smem, dx, up, down);
+        case 1: return launch_flux_pair<1, BAND, BOUND, SUN>(e, grid, smem, dx, up, down);
+        case 2: return launch_flux_pair<2, BAND, BOUND, SUN>(e, grid, smem, dx, up, down);
+        case 3: return launch_flux_pair<3, BAND, BOUND, SUN>(e, grid, smem, dx, up, down);
+        default: return launch_flux_pair<4, BAND, BOUND, SUN>(e, grid, smem, dx, up, down);
     }
 }
 
-// A black surface and nothing from the top: the plain passes.
-static bool flux_bounded(const prb_engine *e) { return !e->bnd_tab.empty() || e->bnd_t_top > 0; }
+// A black surface, nothing from the top and no Sun: the plain passes.  A Sun takes the boundary passes.
+static bool flux_bounded(const prb_engine *e) { return !e->bnd_tab.empty() || e->bnd_t_top > 0 || !e->sun_tab.empty(); }
 
 template <bool BAND>
 static cudaError_t launch_flux_passes(prb_engine *e, int n_mu, int grid, size_t smem, double dx, const K3FArgs &up,
                                       const K3FArgs &down) {
+    if (!e->sun_tab.empty())
+        return e->bnd_reflection == PRB_REFLECT_SPECULAR
+                   ? launch_flux_nodes<BAND, true, K3F_SUN_SPECULAR>(e, n_mu, grid, smem, dx, up, down)
+                   : launch_flux_nodes<BAND, true, K3F_SUN>(e, n_mu, grid, smem, dx, up, down);
     return flux_bounded(e) ? launch_flux_nodes<BAND, true>(e, n_mu, grid, smem, dx, up, down)
                            : launch_flux_nodes<BAND, false>(e, n_mu, grid, smem, dx, up, down);
+}
+
+// The radiance rows of the flux calls: up [0, 4), down [4, 8) and, with a Sun, the beam's row (8): S(nu) at the top,
+// which the downward pass replaces with the beam at the surface.
+static cudaError_t flux_rows_ensure(prb_engine *e) {
+    return e->flux_rows.ensure((size_t)(e->sun_tab.empty() ? 8 : 9) * e->kmat_ld);
 }
 
 // With boundaries set: the emissivity on the chunk (k3_flux_emissivity, every call: the table is tiny), the downward
@@ -1859,7 +1878,7 @@ static cudaError_t flux_boundaries_prepare(prb_engine *e, double dx, K3FArgs &up
     const std::vector<double> &tab = e->bnd_tab.empty() ? black : e->bnd_tab;
     const int64_t n_tab = (int64_t)tab.size() / 2;
     cudaError_t ce;
-    if ((ce = e->flux_rows.ensure((size_t)2 * 4 * e->kmat_ld)) != cudaSuccess) return ce;
+    if ((ce = flux_rows_ensure(e)) != cudaSuccess) return ce;
     if ((ce = e->flux_eps.ensure((size_t)e->kmat_ld)) != cudaSuccess) return ce;
     if ((ce = e->bnd_tab_dev.ensure(tab.size())) != cudaSuccess) return ce;
     ce = cudaMemcpyAsync(e->bnd_tab_dev.p, tab.data(), sizeof(double) * tab.size(), cudaMemcpyHostToDevice, e->stream);
@@ -1874,6 +1893,28 @@ static cudaError_t flux_boundaries_prepare(prb_engine *e, double dx, K3FArgs &up
     up.eps = e->flux_eps.p;
     up.surf_down = down.rows;
     up.specular = e->bnd_reflection == PRB_REFLECT_SPECULAR;
+    if (e->sun_tab.empty()) return cudaSuccess;
+    // the Sun: S on the chunk in the beam's row (k3_flux_solar, every call), and the beam's per-layer factors
+    const int L = e->atm_layers;
+    const int64_t n_sun = (int64_t)e->sun_tab.size() / 2;
+    std::vector<float> nd(L);
+    for (int l = 0; l < L; ++l) nd[l] = (float)(-e->atm_depth[l] * 1.4426950408889634 / e->sun_mu);
+    if ((ce = e->sun_tab_dev.ensure(e->sun_tab.size())) != cudaSuccess) return ce;
+    if ((ce = e->sun_nd.ensure((size_t)L)) != cudaSuccess) return ce;
+    ce = cudaMemcpyAsync(e->sun_tab_dev.p, e->sun_tab.data(), sizeof(double) * e->sun_tab.size(), cudaMemcpyHostToDevice,
+                         e->stream);
+    if (ce != cudaSuccess) return ce;
+    ce = cudaMemcpyAsync(e->sun_nd.p, nd.data(), sizeof(float) * L, cudaMemcpyHostToDevice, e->stream);
+    if (ce != cudaSuccess) return ce;
+    float *sun_row = e->flux_rows.p + (size_t)8 * e->kmat_ld;
+    k3_flux_solar<<<blocks, 256, 0, e->stream>>>(nc, e->i_begin, e->n_total, e->range_min, dx, e->atm_range_max,
+                                                 e->sun_tab_dev.p, n_sun, sun_row);
+    if ((ce = cudaGetLastError()) != cudaSuccess) return ce;
+    for (K3FArgs *a : {&up, &down}) {
+        a->sun_nd = e->sun_nd.p;
+        a->sun_w = (float)(e->sun_mu / (2 * 3.141592653589793));
+    }
+    up.sun_mu_over_pi = (float)(e->sun_mu / 3.141592653589793);
     return cudaSuccess;
 }
 
@@ -1931,7 +1972,7 @@ extern "C" int prb_atmosphere_fluxes(prb_engine *e, int32_t n_mu, const double *
     const bool rows = rad_up_top || rad_down_surface;
     CK(e->flux_part.ensure((size_t)2 * grid * n_levels));
     CK(e->flux_out.ensure((size_t)2 * n_levels));
-    if (rows) CK(e->flux_rows.ensure((size_t)2 * 4 * e->kmat_ld));
+    if (rows) CK(flux_rows_ensure(e));
     up.ld_rows = down.ld_rows = e->kmat_ld;
     up.rows = rows ? e->flux_rows.p : nullptr;
     down.rows = rows ? e->flux_rows.p + (size_t)4 * e->kmat_ld : nullptr;
@@ -2091,6 +2132,28 @@ extern "C" int prb_set_flux_boundaries(prb_engine *e, int64_t n_table, const dou
     e->bnd_tab.insert(e->bnd_tab.end(), table_emissivity, table_emissivity + n_table);
     e->bnd_reflection = reflection;
     e->bnd_t_top = t_top;
+    return PRB_OK;
+}
+
+extern "C" int prb_set_solar_source(prb_engine *e, int64_t n_table, const double *table_nu,
+                                    const double *table_irradiance, double mu_sun) {
+    if (!e) return fail(PRB_ERR_ARG, "null engine");
+    if (n_table == 0) {
+        e->sun_tab.clear();
+        return PRB_OK;
+    }
+    if (n_table < 2 || !table_nu || !table_irradiance)
+        return fail(PRB_ERR_ARG, "prb_set_solar_source: need n_table = 0, or n_table >= 2 and both tables");
+    for (int64_t i = 0; i < n_table; ++i) {
+        if (!std::isfinite(table_nu[i]) || (i > 0 && !(table_nu[i] > table_nu[i - 1])))
+            return fail(PRB_ERR_ARG, "prb_set_solar_source: table_nu must be finite and strictly ascending");
+        if (!(std::isfinite(table_irradiance[i]) && table_irradiance[i] >= 0))
+            return fail(PRB_ERR_ARG, "prb_set_solar_source: every irradiance must be finite and >= 0");
+    }
+    if (!(mu_sun > 0 && mu_sun <= 1)) return fail(PRB_ERR_ARG, "prb_set_solar_source: mu_sun must lie in (0, 1]");
+    e->sun_tab.assign(table_nu, table_nu + n_table);
+    e->sun_tab.insert(e->sun_tab.end(), table_irradiance, table_irradiance + n_table);
+    e->sun_mu = mu_sun;
     return PRB_OK;
 }
 

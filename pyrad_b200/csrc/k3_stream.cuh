@@ -457,6 +457,18 @@ k3_fold_tma(const float *__restrict__ kmat, int64_t ld, int n_layers, const Fold
 // rows.  The upward pass starts each strip from eps B(nu, T_s) + (1 - eps) S_i, S_i the radiance the surface reflects
 // along mu_i: Lambertian S = sum_j 2 w_j mu_j I_down_j(nu, 0) (FP32, node order), specular S_i = I_down_i(nu, 0).  Where
 // eps = 1 the start is B(nu, T_s) bit for bit, whatever comes down.  The layer loop is the fold's.
+//
+// Solar beam (SUN != K3F_NO_SUN, prb_set_solar_source; always with BOUND): a collimated beam E along mu_sun that nothing
+// emits into or scatters.  The downward pass (SUN = K3F_SUN) carries E next to the nodes from E = S(nu) at level L,
+// E <- E exp2(k sun_nd[l]) per layer, adds mu_sun sum E res to every level (E enters partial() with weight
+// mu_sun / (2 pi), under the same non-finite rule).  The beam's row is the one four rows past the downward pass's first
+// (row 8 of flux_rows): the pass reads S there and writes E at the surface over it, point by point, and the upward pass
+// reads that row at each strip's start.  Lambertian (K3F_SUN): 1 - eps of it joins the diffuse term, S_i + mu_sun E / pi
+// (added last, FP32).  Specular (K3F_SUN_SPECULAR): the reflected beam E_up = (1 - eps) E rises along mu_sun through
+// the same layer factors and joins the level sums as above.  Where eps = 1, or E is not > 0 (an E of 0 times an FP32
+// transmittance overflow next to 0 cm^-1 is NaN), nothing is reflected: a select, so the bits are those without the Sun.
+constexpr int K3F_NO_SUN = 0, K3F_SUN = 1, K3F_SUN_SPECULAR = 2;
+
 struct FluxLayer {
     float c2_over_t;         // 100 h c / kB / T_layer
     float nd[4];             // -depth log2(e) / mu_i: T_i = exp2(k * nd[i])
@@ -483,7 +495,12 @@ struct K3FArgs {
     const float *surf_down;  // upward pass: [NMU][ld_rows], the downward pass's radiance reaching the surface
     int32_t specular;        // upward pass: 1 specular reflection, 0 Lambertian
     float c2_over_ttop;      // downward pass: 100 h c / kB / T_top; 0: I = 0 at level L
+    // solar beam only (K3FArgs stays within 128 bytes: a larger one changes the code of every instantiation)
+    const float *sun_nd;     // [n_layers] -depth log2(e) / mu_sun: the beam's T = exp2(k * sun_nd[l])
+    float sun_w;             // mu_sun / (2 pi): the beam's weight in partial() (the sums are scaled by 2 pi res)
+    float sun_mu_over_pi;    // upward pass, Lambertian: mu_sun / pi, the diffuse radiance of a reflected unit beam
 };
+static_assert(sizeof(K3FArgs) <= 128, "K3FArgs above 128 bytes changes the compiled k3_flux_tma");
 
 constexpr int K3F_WARPS = K3T_THREADS / 32;
 struct K3FSmem {
@@ -499,11 +516,14 @@ __host__ __device__ constexpr size_t k3f_smem_bytes(int n_layers) {
     return sizeof(K3FSmem) + sizeof(double) * K3F_WARPS * (size_t)(n_layers + 1);
 }
 
-template <int NMU, bool DOWN, bool BAND = false, bool BOUND = false>
+template <int NMU, bool DOWN, bool BAND = false, bool BOUND = false, int SUN = K3F_NO_SUN>
 __global__ void __launch_bounds__(K3T_THREADS, k3f_minb(NMU))
 k3_flux_tma(const float *__restrict__ kmat, int64_t ld, int n_layers, const FluxLayer *__restrict__ layers,
             int64_t n_chunk, int64_t i_begin, int64_t n_total, double x0, double dx, double x_last,
             float c2_over_tsurf, float nu_interp_min, const K3FArgs a) {
+    static_assert(SUN == K3F_NO_SUN || BOUND, "the solar beam takes the boundary path");
+    static_assert(!(DOWN && SUN == K3F_SUN_SPECULAR), "the downward beam does not depend on the reflection");
+    constexpr bool BEAM = SUN != K3F_NO_SUN && (DOWN || SUN == K3F_SUN_SPECULAR);   // the pass carries a beam
     extern __shared__ __align__(128) unsigned char k3_smem_raw[];
     K3FSmem &sm = *reinterpret_cast<K3FSmem *>(k3_smem_raw);
     double *acc = reinterpret_cast<double *>(k3_smem_raw + sizeof(K3FSmem));
@@ -542,6 +562,7 @@ k3_flux_tma(const float *__restrict__ kmat, int64_t ld, int n_layers, const Flux
         for (int64_t s = 0; s < min(n_steps, (int64_t)(K3T_SLOTS - 1)); ++s) issue(s);
 
     float nu[4], a3[4], rad[NMU][4];
+    float beam[4] = {0.f, 0.f, 0.f, 0.f};              // BEAM: the solar beam at the thread's four points
     bool interp = false;
     int n_valid = 0;                                   // of the thread's four points, those inside the chunk
     int64_t i0 = 0;
@@ -568,6 +589,20 @@ k3_flux_tma(const float *__restrict__ kmat, int64_t ld, int n_layers, const Flux
                     if (q < n_valid && isfinite(rad[i][q])) t += rad[i][q];
                 s = fmaf(a.wmu[i], t, s);
             }
+        }
+        if constexpr (BEAM) {                          // + mu_sun / (2 pi) sum_q E(nu_q), the same non-finite rule
+            float e = 0.f;
+            if (n_valid == 4) {
+                const float2 p = __fadd2_rn(make_float2(beam[0], beam[1]), make_float2(beam[2], beam[3]));
+                e = p.x + p.y;
+            }
+            if (n_valid < 4 || !isfinite(e)) {
+                e = 0.f;
+#pragma unroll
+                for (int q = 0; q < 4; ++q)
+                    if (q < n_valid && isfinite(beam[q])) e += beam[q];
+            }
+            s = fmaf(a.sun_w, e, s);
         }
         return s;
     };
@@ -596,6 +631,8 @@ k3_flux_tma(const float *__restrict__ kmat, int64_t ld, int n_layers, const Flux
 #pragma unroll
                 for (int i = 0; i < NMU; ++i)
                     if (isfinite(rad[i][q])) v[q] = fmaf(a.wmu[i], rad[i][q], v[q]);
+                if constexpr (BEAM)
+                    if (isfinite(beam[q])) v[q] = fmaf(a.sun_w, beam[q], v[q]);
             }
             for (int s = 0; s < sp.nseg; s += 2) {
                 const uint32_t r0 = a.seg_range[sp.seg0 + s], r1 = s + 1 < sp.nseg ? a.seg_range[sp.seg0 + s + 1] : 0u;
@@ -622,6 +659,16 @@ k3_flux_tma(const float *__restrict__ kmat, int64_t ld, int n_layers, const Flux
         if constexpr (BAND) band_add(level);
         else level_add(partial(), level);
     };
+    // v[q] = p[i0 + q] for the thread's points inside the chunk, 0 outside (solar beam only)
+    auto chunk_load4 = [&](const float *p, float (&v)[4]) {
+        if (n_valid == 4) {
+            const float4 v4 = *reinterpret_cast<const float4 *>(p + i0);
+            v[0] = v4.x; v[1] = v4.y; v[2] = v4.z; v[3] = v4.w;
+        } else {
+#pragma unroll
+            for (int q = 0; q < 4; ++q) v[q] = q < n_valid ? p[i0 + q] : 0.f;
+        }
+    };
     // boundaries, upward pass: rad holds B(nu, T_s); make it eps B + (1 - eps) S_i (points outside the chunk keep B)
     auto surface_start = [&]() {
         float eps[4] = {1.f, 1.f, 1.f, 1.f}, dn[NMU][4];
@@ -641,14 +688,20 @@ k3_flux_tma(const float *__restrict__ kmat, int64_t ld, int n_layers, const Flux
                 for (int i = 0; i < NMU; ++i) dn[i][q] = q < n_valid ? a.surf_down[(int64_t)i * a.ld_rows + i0 + q] : 0.f;
             }
         }
+        float es[4] = {0.f, 0.f, 0.f, 0.f};           // the solar beam reaching the surface
+        if constexpr (SUN != K3F_NO_SUN) chunk_load4(a.surf_down + (int64_t)4 * a.ld_rows, es);
 #pragma unroll
         for (int q = 0; q < 4; ++q) {
             float s = 0.f;                             // Lambertian: F_down / pi = sum_j 2 w_j mu_j I_down_j
 #pragma unroll
             for (int j = 0; j < NMU; ++j) s = fmaf(2.f * a.wmu[j], dn[j][q], s);
+            if constexpr (SUN == K3F_SUN)              // + mu_sun E / pi
+                if (es[q] > 0.f) s = fmaf(a.sun_mu_over_pi, es[q], s);
+            if constexpr (SUN == K3F_SUN_SPECULAR)     // the reflected beam
+                beam[q] = eps[q] == 1.f || !(es[q] > 0.f) ? 0.f : (1.f - eps[q]) * es[q];
 #pragma unroll
             for (int i = 0; i < NMU; ++i) {
-                const float sv = a.specular ? dn[i][q] : s;
+                const float sv = (SUN == K3F_NO_SUN ? a.specular != 0 : SUN == K3F_SUN_SPECULAR) ? dn[i][q] : s;
                 rad[i][q] = eps[q] == 1.f ? rad[i][q] : fmaf(eps[q], rad[i][q], (1.f - eps[q]) * sv);
             }
         }
@@ -658,7 +711,13 @@ k3_flux_tma(const float *__restrict__ kmat, int64_t ld, int n_layers, const Flux
         const int g = group_of(step);
         if (step % groups == 0) {                      // a new strip: the boundary radiance of the pass
             const int64_t strip = strip_of(step);
-            i0 = strip * K3T_STRIP + 4 * tid;
+            if constexpr (SUN != K3F_NO_SUN) {          // (read again: 4 tid held over the strips would spill)
+                uint32_t t;
+                asm volatile("mov.u32 %0, %%tid.x;" : "=r"(t));
+                i0 = strip * K3T_STRIP + 4 * (int)t;
+            } else {
+                i0 = strip * K3T_STRIP + 4 * tid;
+            }
             n_valid = (int)max((int64_t)0, min((int64_t)4, n_chunk - i0));
 #pragma unroll
             for (int q = 0; q < 4; ++q) {
@@ -672,6 +731,7 @@ k3_flux_tma(const float *__restrict__ kmat, int64_t ld, int n_layers, const Flux
                 for (int i = 0; i < NMU; ++i) rad[i][q] = r0;
             }
             if constexpr (BOUND && !DOWN) surface_start();
+            if constexpr (BEAM && DOWN) chunk_load4(a.rows + (int64_t)4 * a.ld_rows, beam);   // E = S(nu) at level L
             interp = nu[0] >= nu_interp_min;
             if (!DOWN) add_level(0);                   // (the plain downward pass starts from 0 at level L,
             else if (BAND || BOUND) add_level(n_layers);   // whose band segment slots must still be written: zeros)
@@ -697,6 +757,14 @@ k3_flux_tma(const float *__restrict__ kmat, int64_t ld, int n_layers, const Flux
                     const float2 r23 = k3_fold_step2(make_float2(rad[i][2], rad[i][3]), e23, b23);
                     rad[i][0] = r01.x; rad[i][1] = r01.y; rad[i][2] = r23.x; rad[i][3] = r23.y;
                 }
+                if constexpr (BEAM) {                  // E <- E exp(-k depth / mu_sun): no emission, no scattering
+                    const float2 nd = make_float2(a.sun_nd[l], a.sun_nd[l]);
+                    const float2 e01 = __fmul2_rn(make_float2(k4.x, k4.y), nd), e23 = __fmul2_rn(make_float2(k4.z, k4.w), nd);
+                    const float2 t01 = make_float2(k3_ex2(e01.x), k3_ex2(e01.y)), t23 = make_float2(k3_ex2(e23.x), k3_ex2(e23.y));
+                    const float2 b01 = __fmul2_rn(make_float2(beam[0], beam[1]), t01);
+                    const float2 b23 = __fmul2_rn(make_float2(beam[2], beam[3]), t23);
+                    beam[0] = b01.x; beam[1] = b01.y; beam[2] = b23.x; beam[3] = b23.y;
+                }
                 add_level(DOWN ? l : l + 1);
             }
         }
@@ -710,6 +778,16 @@ k3_flux_tma(const float *__restrict__ kmat, int64_t ld, int n_layers, const Flux
 #pragma unroll
                     for (int q = 0; q < 4; ++q)
                         if (q < n_valid) dst[q] = rad[i][q];
+            }
+        }
+        if constexpr (BEAM && DOWN) {                  // the beam at the surface, for the upward pass
+            if (step % groups == groups - 1 && n_valid > 0) {
+                float *dst = a.rows + (int64_t)4 * a.ld_rows + i0;
+                if (n_valid == 4) *reinterpret_cast<float4 *>(dst) = make_float4(beam[0], beam[1], beam[2], beam[3]);
+                else
+#pragma unroll
+                    for (int q = 0; q < 4; ++q)
+                        if (q < n_valid) dst[q] = beam[q];
             }
         }
     }
@@ -730,6 +808,17 @@ k3_flux_emissivity(int64_t n_chunk, int64_t i_begin, int64_t n_total, double x0,
                    const double *__restrict__ tab, int64_t n_tab, float *__restrict__ eps) {
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_chunk; i += (int64_t)gridDim.x * blockDim.x)
         eps[i] = (float)np_interp(axis_value(i_begin + i, n_total, x0, dx, x_last), tab, tab + n_tab, n_tab);
+}
+
+// Solar irradiance at the top on the owned chunk: s[i] = np.interp(x, table_nu, table_s, left=0, right=0) in FP64,
+// rounded to FP32; x the Planck axis of the fold.  tab = table_nu | table_s, n_tab >= 2 entries each.
+__global__ void __launch_bounds__(256)
+k3_flux_solar(int64_t n_chunk, int64_t i_begin, int64_t n_total, double x0, double dx, double x_last,
+              const double *__restrict__ tab, int64_t n_tab, float *__restrict__ s) {
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_chunk; i += (int64_t)gridDim.x * blockDim.x) {
+        const double x = axis_value(i_begin + i, n_total, x0, dx, x_last);
+        s[i] = x < tab[0] || x > tab[n_tab - 1] ? 0.f : (float)np_interp(x, tab, tab + n_tab, n_tab);
+    }
 }
 
 // Band totals of the band pass: out[d][b][j] = scale * sum of band b's segments at level j of pass d (0 up, 1 down), for

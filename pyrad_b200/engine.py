@@ -151,6 +151,29 @@ def flux_boundary_args(emissivity=None, reflection="lambertian", t_top=0.0):
     return nu, eps, REFLECTIONS[reflection], t_top
 
 
+def solar_source_args(irradiance=None, mu_sun=1.0):
+    """Checked arguments of prb_set_solar_source: (table_nu, table_irradiance, mu_sun).
+
+    irradiance: None (no Sun: an empty table) or a pair (nu, S) of 1-d arrays of one length, at least two entries; nu in
+    cm-1 finite and strictly ascending, S in W m-2 (cm-1)-1 on a plane normal to the beam, finite and >= 0.  mu_sun: the
+    cosine of the solar zenith angle, in (0, 1]; ignored without a Sun.  ValueError otherwise."""
+    if irradiance is None:
+        return np.zeros(0), np.zeros(0), 1.0
+    if not hasattr(irradiance, "__len__") or len(irradiance) != 2:
+        raise ValueError("irradiance must be None or a pair (nu, S)")
+    nu, s = _f64(irradiance[0]), _f64(irradiance[1])
+    if nu.ndim != 1 or nu.shape != s.shape or nu.size < 2:
+        raise ValueError("irradiance: nu and S must be 1-d arrays of one length, at least two entries")
+    if not np.all(np.isfinite(nu)) or not np.all(np.diff(nu) > 0):
+        raise ValueError("irradiance: nu must be finite and strictly ascending")
+    if not np.all(np.isfinite(s) & (s >= 0)):
+        raise ValueError("irradiance: S must be finite and >= 0")
+    mu_sun = float(mu_sun)
+    if not (mu_sun > 0 and mu_sun <= 1):
+        raise ValueError("mu_sun must lie in (0, 1]")
+    return nu, s, mu_sun
+
+
 class Engine:
     """One engine per process per device (the C ABI's contract)."""
 
@@ -526,6 +549,16 @@ class Engine:
         nu, eps, refl, t_top = flux_boundary_args(emissivity, reflection, t_top)
         _lib.check(self._lib.prb_set_flux_boundaries(self._h, nu.size, _dp(nu) if nu.size else None,
                                                      _dp(eps) if eps.size else None, refl, t_top))
+
+    def set_solar_source(self, irradiance=None, mu_sun=1.0):
+        """The Sun of every later atmosphere_fluxes / atmosphere_band_fluxes call (prb_set_solar_source; arguments as
+        solar_source_args): a beam along mu_sun with irradiance S(nu) at the top, np.interp over the table on the
+        column's grid and 0 outside it, absorbed on its way down and reflected by the surface of set_flux_boundaries
+        (1 - eps of it, as that call's reflection says).  flux_down includes the beam, and flux_up its reflection.  No
+        arguments: no Sun again.  The column's own radiance (atmosphere_read) is not affected."""
+        nu, s, mu_sun = solar_source_args(irradiance, mu_sun)
+        _lib.check(self._lib.prb_set_solar_source(self._h, nu.size, _dp(nu) if nu.size else None,
+                                                  _dp(s) if s.size else None, mu_sun))
 
     def set_result_host(self, rad=None, tr=None):
         """Register pinned float32 host arrays that every following atmosphere() fills directly from the device

@@ -11,7 +11,11 @@ single band 630-700 cm-1 -- and reports each beside the 3-node total call of the
 boundaries set (prb_set_flux_boundaries: emissivity 0.98 with a linear dip to 0.75 over 1080-1180 cm-1, the 2.725 K
 cosmic background at the top, Lambertian and specular reflection), times the 3-node total call and the 16-band call as
 ratios to the plain calls timed right before them, and reports the OLR and the net flux at the surface with and
-without the surface.  Prints one JSON line; writes nothing.
+without the surface.  Then, on the same surface and top, adds a 5772 K blackbody Sun scaled to 1361 W m-2 in total at
+mu_sun = 0.5 (prb_set_solar_source, both reflections), times the same two calls as ratios to the sunless boundary calls
+timed right before them, and reports the sunlight at the top (mu_sun sum S res), the beam at the surface, the sunlight
+leaving the top and the largest solar heating rate with its layer, each as the result with the Sun minus the result
+without it.  Prints one JSON line; writes nothing.
 
     python scripts/flux_bench.py [--reps 30] [--warmup 3]
 """
@@ -50,6 +54,49 @@ def timed(stream, fn, warmup, reps):
         b.synchronize()
         ms.append(a.elapsed_time(b))
     return ms
+
+
+def blackbody_sun(nu_t, t_sun=5772.0, total=1361.0):
+    """A blackbody Sun scaled to `total` W m-2 over all wavenumbers, as an irradiance table (nu, S) on nu_t."""
+    from oracle import physics as ph
+    fine = np.arange(1.0, 100000.0, 1.0)
+    scale = total / (ph.pi * np.sum(ph.planck_wavenumber(fine, t_sun)))
+    return nu_t, ph.pi * np.nan_to_num(ph.planck_wavenumber(nu_t, t_sun)) * scale
+
+
+def solar_section(e, stream, args, w, mu, wt, calls, eps_table):
+    """The Sun on cfg4's surface (eps_table, 2.725 K top): both reflections, each timed right after the same sunless
+    boundary calls."""
+    from pyrad_b200.classes import heatingRate
+    sun, mu_sun = blackbody_sun(np.arange(0.0, 5011.0)), 0.5
+    res = {"t_sun_k": 5772.0, "total_w_m2": 1361.0, "mu_sun": mu_sun, "n_mu": 3, "runs": []}
+
+    def heating(up, down):
+        return heatingRate(up, down, w["depth_cm"], w["T"], w["P"])
+
+    try:
+        for reflection in ("lambertian", "specular"):
+            e.set_flux_boundaries(eps_table, reflection, 2.725)
+            e.set_solar_source()
+            dark_ms = {k: float(np.median(timed(stream, f, args.warmup, args.reps))) for k, f in calls.items()}
+            up0, down0 = e.atmosphere_fluxes(mu, wt)
+            e.set_solar_source(sun, mu_sun)
+            run = {"reflection": reflection, "sunless_ms_median": dark_ms}
+            for k, f in calls.items():
+                ms = timed(stream, f, args.warmup, args.reps)
+                med = float(np.median(ms))
+                run[k] = {"ms_median": med, "ms_p10_p90": [float(np.percentile(ms, 10)), float(np.percentile(ms, 90))],
+                          "reps": args.reps, "ratio_to_sunless_call": med / dark_ms[k]}
+            up, down = e.atmosphere_fluxes(mu, wt)
+            dq = heating(up, down) - heating(up0, down0)
+            run.update(sun_top_w_m2=float(down[-1] - down0[-1]), beam_surface_w_m2=float(down[0] - down0[0]),
+                       sun_leaving_top_w_m2=float(up[-1] - up0[-1]), max_solar_heating_k_day=float(dq.max()),
+                       max_solar_heating_layer=int(dq.argmax()), max_solar_heating_p_hpa=float(w["P"][int(dq.argmax())]))
+            res["runs"].append(run)
+    finally:
+        e.set_solar_source()
+        e.set_flux_boundaries()
+    return res
 
 
 def main():
@@ -141,6 +188,7 @@ def main():
             out["boundaries"]["runs"].append(run)
     finally:
         e.set_flux_boundaries()
+    out["solar"] = solar_section(e, stream, args, w, mu, wt, calls, eps_table)
     e.close()
     print(json.dumps(out))
 
