@@ -24,6 +24,7 @@
  *   (absent upstream) the column's fluxes per wavenumber band, at every level      -> prb_atmosphere_band_fluxes
  *   (absent upstream) a grey or spectral surface and a warm top for both flux calls -> prb_set_flux_boundaries
  *   (absent upstream) an absorbed, reflected solar beam for both flux calls        -> prb_set_solar_source
+ *   (absent upstream) a water-vapour continuum in the column's k matrix            -> prb_set_continuum
  *
  * Conventions: every entry point is extern "C", returns int (0 = PRB_OK, < 0 = error) unless
  * noted, takes plain pointers and sizes.  Pointers named *_host / unmarked are caller-owned host
@@ -215,6 +216,23 @@ int prb_xsc_resident(prb_engine *e, int32_t slot, int64_t n_out, int64_t dst0, i
                      int64_t n_file, const double *file_x, const double *file_y);
 int prb_set_xsc_conc(prb_engine *e, int32_t n_layers, int32_t n_xsc, const double *conc);
 int prb_xsc_clear(prb_engine *e);
+/* A water-vapour continuum in MT_CKD's form for every later prb_atmosphere and prb_gas_cell_host call with n_layers
+ * layers, until changed (grid changes keep it).  For layer l (T_l in K, P_l in hPa, x_l = mole_fraction[l] of the
+ * continuum's gas) and every point nu of the Planck axis, row l of the k matrix gains, before the fold,
+ *   k_c,l(nu) = n_l rho_l R(nu, T_l) [x_l (t_ref/T_l)^n(nu) C_s(nu) + (1 - x_l) C_f(nu)]   in cm^-1,
+ *   n_l = x_l P_l / 1e4 / kB / T_l (molecules cm^-3),  rho_l = (P_l / p_ref)(t_ref / T_l),  R(nu, T) = nu tanh(c2 nu / 2T),
+ * C_s, C_f = np.interp(nu, table_nu, c_self / c_foreign, left=0, right=0) in cm^2 molecule^-1 (cm^-1)^-1 and
+ * n = np.interp(nu, table_nu, t_exp) (clamped at the ends).  Layers with x_l = 0 are left alone.  The table must match
+ * the line shape: MT_CKD's coefficients belong to lines cut at 25 cm^-1 with the 25 cm^-1 value subtracted, while this
+ * path cuts the lines at 5 P/p0 cm^-1 and adds whatever table it is given.  n_table = 0 clears the continuum (the
+ * pointers may then be NULL); otherwise n_table >= 2, table_nu finite and strictly ascending, c_self and c_foreign finite
+ * and >= 0, t_exp finite, t_ref and p_ref finite and > 0, n_layers >= 1 and every mole fraction in [0, 1], or PRB_ERR_ARG
+ * and the previous setting stays.  A column of another layer count gets PRB_ERR_ARG.  With a continuum, one layer takes
+ * the separate fold instead of K2's fused epilogue, and prb_gas_cell_host takes its separate calls; without one, every
+ * result is what it was before. */
+int prb_set_continuum(prb_engine *e, int64_t n_table, const double *table_nu, const double *c_self,
+                      const double *c_foreign, const double *t_exp, double t_ref, double p_ref, int32_t n_layers,
+                      const double *mole_fraction);
 
 /* ---- per-layer line ranges.  The reference loads every layer's lines from that layer's own effective range, strictly
  * inside (Isotope.getData -> gatherData(effectiveRangeMin, effectiveRangeMax), pyradClasses.py:350-352,

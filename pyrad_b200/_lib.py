@@ -64,6 +64,7 @@ PROTOTYPES = {
     "prb_xsc_place": (C.c_int, [_vp, _i64, _i64, _i64, _i64, C.c_int, _d, _d, _i64, _dp, _dp, _dp]),
     "prb_xsc_resident": (C.c_int, [_vp, _i32, _i64, _i64, _i64, _i64, C.c_int, _d, _d, _i64, _dp, _dp]),
     "prb_set_xsc_conc": (C.c_int, [_vp, _i32, _i32, _dp]),
+    "prb_set_continuum": (C.c_int, [_vp, _i64, _dp, _dp, _dp, _dp, _d, _d, _i32, _dp]),
     "prb_set_layer_line_range": (C.c_int, [_vp, _i32, _dp, _dp]),
     "prb_xsc_clear": (C.c_int, [_vp]),
     "prb_atmosphere": (C.c_int, [_vp, _i32, _i32, _dp, _dp, _dp, _dp, _dp, _dp, _dp, _lp, _d, _d]),

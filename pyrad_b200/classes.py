@@ -859,17 +859,22 @@ class Atmosphere(list):
             spectrum = layer.transmission(spectrum)
         return spectrum
 
-    def columnSpectrum(self, surfaceTemperature):
+    def columnSpectrum(self, surfaceTemperature, continuum=None):
         """The whole column on the device in ONE engine call (prb_atmosphere): K1 for every layer, the batched line
         sums, and the fold  I <- T_l I + (1 - T_l) B(nu, T_l)  starting from I_0 = B(nu, surfaceTemperature).
         Returns (radiance, total transmittance) on the layers' common grid.  Same physics as ``transmission`` above,
         without one host round trip per layer and isotope; needs layers that share range and base resolution and carry
         the same line-by-line molecules in the same order.  xsc molecules (up to eight distinct tables over the column)
-        stay resident on the device and enter every layer's k(nu) inside the line-sum kernel (prb_xsc_resident)."""
-        return self._column(surfaceTemperature, lambda e: e.atmosphere_read())
+        stay resident on the device and enter every layer's k(nu) inside the line-sum kernel (prb_xsc_resident).
+        continuum: None, or a water-vapour continuum table in MT_CKD's form for this call (Engine.set_continuum: a dict
+        with nu, self, foreign, texp and optional t_ref, p_ref); its mole fraction in a layer is the summed concentration
+        of the layer's line-by-line H2O (HITRAN id 1), 0 without one.  The continuum is an extension of the column path:
+        ``transmission``, getTransmittance(layer) and Layer.transmission stay the reference's physics, without it.  The
+        default gives the result described above, bit for bit."""
+        return self._column(surfaceTemperature, lambda e: e.atmosphere_read(), continuum)
 
     def columnFluxes(self, surfaceTemperature, mu=None, weights=None, bands=None, surfaceEmissivity=None,
-                     reflection="lambertian", topTemperature=0.0, solarIrradiance=None, solarMu=1.0):
+                     reflection="lambertian", topTemperature=0.0, solarIrradiance=None, solarMu=1.0, continuum=None):
         """Hemispheric fluxes, heating rates and slant radiances of the column (prb_atmosphere, then
         prb_atmosphere_fluxes on its device-resident k matrix; same requirements on the layers as columnSpectrum).
         For every node mu_i of the angular quadrature (default: 3-node Gauss-Legendre on [0, 1]; at most 4 nodes) the
@@ -895,6 +900,7 @@ class Atmosphere(list):
         absorbed on its way down and 1 - eps of it is reflected as the surface says; flux_down, net, heating_rate and the
         band arrays then include it (and flux_up its reflection).  The sunlight's share of any of them is the result with
         the Sun minus the result without it: the column is linear in its sources.
+        continuum: a water-vapour continuum in the column's k matrix for this call, as in columnSpectrum.
         The defaults give the result described above, bit for bit."""
         _eng.flux_boundary_args(surfaceEmissivity, reflection, topTemperature)      # ValueError before the column runs
         _eng.solar_source_args(solarIrradiance, solarMu)
@@ -919,7 +925,7 @@ class Atmosphere(list):
                 e.set_solar_source()
                 e.set_flux_boundaries()
 
-        (up, down, ru, rd), band = self._column(surfaceTemperature, result)
+        (up, down, ru, rd), band = self._column(surfaceTemperature, result, continuum)
         layers = list(self)
         depth, T, P = [l.depth for l in layers], [l.T for l in layers], [l.P for l in layers]
         out = {"flux_up": up, "flux_down": down, "net": up - down, "heating_rate": heatingRate(up, down, depth, T, P),
@@ -930,11 +936,15 @@ class Atmosphere(list):
                        band_heating_rate=np.array([heatingRate(u, d, depth, T, P) for u, d in zip(bu, bd)]))
         return out
 
-    def _column(self, surfaceTemperature, result):
+    def _column(self, surfaceTemperature, result, continuum=None):
         """Run the column on the device (prb_atmosphere) and return result(engine) while its state is in place."""
         layers = list(self)
         if not layers:
             raise ValueError("atmosphere has no layers")
+        # the continuum's gas is the layers' line-by-line H2O (HITRAN id 1); ValueError before the column runs
+        h2o = [sum(m.concentration for m in l if not m.exotic and m.ID == 1) for l in layers] if continuum is not None \
+            else None
+        _eng.continuum_args(continuum, h2o)
         ref = layers[0]
         for l in layers:
             if (l.rangeMin, l.rangeMax) != (ref.rangeMin, ref.rangeMax) or l.resolution != BASE_RESOLUTION:
@@ -986,6 +996,7 @@ class Atmosphere(list):
             if any((l.effectiveRangeMin, l.effectiveRangeMax) != (widest.effectiveRangeMin, widest.effectiveRangeMax)
                    for l in layers):
                 e.set_layer_line_range([l.effectiveRangeMin for l in layers], [l.effectiveRangeMax for l in layers])
+            e.set_continuum(continuum, h2o)
             e.atmosphere([l.depth for l in layers], [l.T for l in layers], [l.P for l in layers], conc,
                          [iso.molmass for iso in isos] or [1.0], q_t, [iso.q296 for iso in isos] or [1.0], window,
                          surfaceTemperature, ref.rangeMax)
@@ -993,6 +1004,7 @@ class Atmosphere(list):
         finally:
             e.xsc_clear()
             e.set_layer_line_range()
+            e.set_continuum()
 
 
 #: dry air: molar mass (kg/mol), isobaric specific heat (J kg-1 K-1); molar gas constant (J mol-1 K-1, CODATA 2018 exact)

@@ -195,6 +195,15 @@ struct prb_engine {
     std::vector<double> xsc_conc;                     // [xsc_conc_layers][n_xsc]
     int xsc_conc_layers = 0;
     std::vector<double> line_lo, line_hi;             // per-layer line ranges of the next prb_atmosphere calls (may be empty)
+    // the water-vapour continuum of the next prb_atmosphere / prb_gas_cell_host calls (prb_set_continuum); empty: none
+    std::vector<double> cont_tab;                     // table_nu | c_self | c_foreign | t_exp
+    double cont_t_ref = 0, cont_p_ref = 0;
+    std::vector<double> cont_x;                       // mole fraction per layer
+    DevBuf<double> cont_tab_dev;
+    DevBuf<float> cont_rows;                          // [3][kmat_ld]: C_s, C_f, n on the owned chunk
+    std::vector<double> cont_rows_tab;                // the table the rows hold (kept when the continuum is cleared)
+    double cont_sig[5] = {};                          // (i_begin, i_end, n_total, range_min, range_max) of the rows
+    DevBuf<ContLayer> cont_layers;
 
     // outputs / scratch
     DevBuf<double> out64;
@@ -1380,6 +1389,61 @@ static int ensure_xsc_rows(prb_engine *e) {
     return PRB_OK;
 }
 
+extern "C" int prb_set_continuum(prb_engine *e, int64_t n_table, const double *table_nu, const double *c_self,
+                                 const double *c_foreign, const double *t_exp, double t_ref, double p_ref,
+                                 int32_t n_layers, const double *mole_fraction) {
+    if (!e) return fail(PRB_ERR_ARG, "null engine");
+    if (n_table == 0) {
+        e->cont_tab.clear();
+        e->cont_x.clear();
+        return PRB_OK;
+    }
+    if (n_table < 2 || !table_nu || !c_self || !c_foreign || !t_exp)
+        return fail(PRB_ERR_ARG, "prb_set_continuum: need n_table = 0, or n_table >= 2 and all four tables");
+    for (int64_t i = 0; i < n_table; ++i) {
+        if (!std::isfinite(table_nu[i]) || (i > 0 && !(table_nu[i] > table_nu[i - 1])))
+            return fail(PRB_ERR_ARG, "prb_set_continuum: table_nu must be finite and strictly ascending");
+        if (!(std::isfinite(c_self[i]) && c_self[i] >= 0 && std::isfinite(c_foreign[i]) && c_foreign[i] >= 0))
+            return fail(PRB_ERR_ARG, "prb_set_continuum: every c_self and c_foreign must be finite and >= 0");
+        if (!std::isfinite(t_exp[i])) return fail(PRB_ERR_ARG, "prb_set_continuum: every t_exp must be finite");
+    }
+    if (!(std::isfinite(t_ref) && t_ref > 0 && std::isfinite(p_ref) && p_ref > 0))
+        return fail(PRB_ERR_ARG, "prb_set_continuum: t_ref and p_ref must be finite and > 0");
+    if (n_layers < 1 || !mole_fraction) return fail(PRB_ERR_ARG, "prb_set_continuum: need n_layers >= 1 and mole_fraction");
+    for (int l = 0; l < n_layers; ++l)
+        if (!(mole_fraction[l] >= 0 && mole_fraction[l] <= 1))
+            return fail(PRB_ERR_ARG, "prb_set_continuum: every mole fraction must lie in [0, 1]");
+    e->cont_tab.assign(table_nu, table_nu + n_table);
+    for (const double *p : {c_self, c_foreign, t_exp}) e->cont_tab.insert(e->cont_tab.end(), p, p + n_table);
+    e->cont_t_ref = t_ref;
+    e->cont_p_ref = p_ref;
+    e->cont_x.assign(mole_fraction, mole_fraction + n_layers);
+    return PRB_OK;
+}
+
+// The continuum table resampled onto the owned chunk (k3_continuum_rows; rebuilt when the grid or the table changed,
+// so a caller that sets and clears the same table around every column resamples it once), after kmat_ld is set for
+// the call.  Enqueue only; *launches counts a rebuild.
+static int ensure_continuum_rows(prb_engine *e, double range_max, int *launches) {
+    const int64_t nc = chunk_len(e);
+    const double sig[5] = {(double)e->i_begin, (double)e->i_end, (double)e->n_total, e->range_min, range_max};
+    if (e->cont_rows_tab == e->cont_tab && std::equal(sig, sig + 5, e->cont_sig)) return PRB_OK;
+    const int64_t n_tab = (int64_t)e->cont_tab.size() / 4;
+    CK(e->cont_tab_dev.ensure(e->cont_tab.size()));
+    CK(cudaMemcpyAsync(e->cont_tab_dev.p, e->cont_tab.data(), sizeof(double) * e->cont_tab.size(), cudaMemcpyHostToDevice,
+                       e->stream));
+    CK(e->cont_rows.ensure((size_t)3 * std::max<int64_t>(e->kmat_ld, 4)));
+    const double dx = e->n_total > 1 ? (range_max - e->range_min) / (double)(e->n_total - 1) : 0.0;
+    k3_continuum_rows<<<stream_grid(e, e->kmat_ld), 256, 0, e->stream>>>(nc, e->kmat_ld, e->i_begin, e->n_total,
+                                                                        e->range_min, dx, range_max, e->cont_tab_dev.p,
+                                                                        n_tab, e->cont_rows.p);
+    CK(cudaGetLastError());
+    ++*launches;
+    e->cont_rows_tab = e->cont_tab;
+    std::copy(sig, sig + 5, e->cont_sig);
+    return PRB_OK;
+}
+
 static void xsc_args(const prb_engine *e, K2Args &a) {
     a.n_xsc = e->n_xsc;
     a.xsc_sigma = e->xsc_rows.p;
@@ -1439,6 +1503,10 @@ static int atmosphere_impl(prb_engine *e, int32_t n_layers, int32_t n_groups, co
     if (!e->line_lo.empty() && (int)e->line_lo.size() != n_layers)
         return fail(PRB_ERR_ARG, "prb_atmosphere: the per-layer line ranges were set for another number of layers "
                                  "(prb_set_layer_line_range with the same n_layers, or with 0 to clear)");
+    const bool continuum = !e->cont_tab.empty();
+    if (continuum && (int)e->cont_x.size() != n_layers)
+        return fail(PRB_ERR_ARG, "prb_atmosphere: the continuum's mole fractions were set for another number of layers "
+                                 "(prb_set_continuum with the same n_layers, or with n_table = 0 to clear)");
     const int xsc_before = e->xsc_build_launches;
     if ((rc = ensure_xsc_rows(e))) return rc;
     const int xsc_launches = e->xsc_build_launches - xsc_before;   // table resamplings this call had to enqueue
@@ -1564,7 +1632,8 @@ static int atmosphere_impl(prb_engine *e, int32_t n_layers, int32_t n_groups, co
         ++dst.n;
     }
     const double dx = e->n_total > 1 ? (range_max - e->range_min) / (double)(e->n_total - 1) : 0.0;
-    const bool fused = n_layers == 1 && e->fuse_single && !jobs[0].narrow && k2_classed(e);
+    // a continuum is added to the k matrix between K2 and the fold, so it needs the separate fold
+    const bool fused = n_layers == 1 && e->fuse_single && !jobs[0].narrow && k2_classed(e) && !continuum;
     K2Fuse fuse{};
     if (fused) {
         fuse.enabled = 1;
@@ -1682,6 +1751,28 @@ static int atmosphere_impl(prb_engine *e, int32_t n_layers, int32_t n_groups, co
         if (e->timing) CK(cudaEventRecord(e->ev[3 * bi + 2], e->stream));
     }
     if (e->timing) CK(cudaEventRecord(e->ev[3 * n_batches], e->stream));
+    if (continuum && nc > 0) {
+        // the continuum on the finished k matrix: the layers with x > 0, their constants formed in FP64
+        if ((rc = ensure_continuum_rows(e, range_max, &launches))) return rc;
+        std::vector<ContLayer> cl;
+        for (int l = 0; l < n_layers; ++l) {
+            const double x = e->cont_x[l];
+            if (!(x > 0)) continue;
+            const double n_rho = x * p_layer[l] / 1E4 / kBoltz / t_layer[l] * (p_layer[l] / e->cont_p_ref) *
+                                 (e->cont_t_ref / t_layer[l]);
+            cl.push_back(ContLayer{(float)(n_rho * x), (float)(n_rho * (1 - x)), (float)std::log2(e->cont_t_ref / t_layer[l]),
+                                   (float)(c2 / (2 * t_layer[l])), l, 0});
+        }
+        if (!cl.empty()) {
+            CK(e->cont_layers.ensure(cl.size()));
+            CK(cudaMemcpyAsync(e->cont_layers.p, cl.data(), sizeof(ContLayer) * cl.size(), cudaMemcpyHostToDevice, e->stream));
+            k3_continuum_add<<<stream_grid(e, e->kmat_ld, 4), 256, 0, e->stream>>>(
+                e->kmat.p, e->kmat_ld, e->cont_layers.p, (int)cl.size(), e->cont_rows.p, e->i_begin, e->n_total,
+                e->range_min, dx, range_max);
+            CK(cudaGetLastError());
+            ++launches;
+        }
+    }
     if (nc > 0 && !fused) {
         if (e->k3_tma && n_layers >= K3T_LAYERS) {
             const int64_t n_strips = (nc + K3T_STRIP - 1) / K3T_STRIP;
@@ -2655,8 +2746,9 @@ extern "C" int prb_gas_cell_host(prb_engine *e, int64_t n, const double *nu0, co
     const int wave = waves_per_piece * wave1;
     const int first = std::min(n_tiles, PRB_PIPE_FIRST_WAVES * wave1);
     const int S = (first > 0 ? 1 : 0) + (n_tiles - first + wave - 1) / wave;
-    // (per-layer line ranges: the separate calls apply them)
-    const bool pipelined = k2_classed(e) && e->fuse_single && wm >= e->narrow_wm && S >= 2 && n >= 4096 && e->line_lo.empty();
+    // (per-layer line ranges and a continuum: the separate calls apply them)
+    const bool pipelined = k2_classed(e) && e->fuse_single && wm >= e->narrow_wm && S >= 2 && n >= 4096 && e->line_lo.empty() &&
+                           e->cont_tab.empty();
     if (!pipelined) {
         int rc = prb_upload_lines(e, n, nu0, s296, gamma_air, gamma_self, elower, n_air, delta_air, group, n_groups);
         if (rc) return rc;

@@ -821,6 +821,102 @@ k3_flux_solar(int64_t n_chunk, int64_t i_begin, int64_t n_total, double x0, doub
     }
 }
 
+// ---- water-vapour continuum (prb_set_continuum), added to the k matrix before the fold -----------------------------
+//   k_c,l(nu) = n_l rho_l R(nu, T_l) [x_l (t_ref/T_l)^n(nu) C_s(nu) + (1 - x_l) C_f(nu)]
+//   n_l = x_l P_l / 1e4 / kB / T_l,  rho_l = (P_l / p_ref)(t_ref / T_l),  R(nu, T) = nu tanh(c2 nu / 2T)
+// in MT_CKD's form.  MT_CKD's coefficients are defined against lines cut at 25 cm^-1 with the 25 cm^-1 value subtracted;
+// this path cuts at 5 P/p0 cm^-1 and adds whatever table it is given: matching the two is the caller's job.
+
+// The table on the owned chunk, once per (grid, table): rows [0, ld) C_s, [ld, 2 ld) C_f, [2 ld, 3 ld) n, each
+// np.interp in FP64 (numpy's arithmetic) rounded to FP32; C_s and C_f are 0 outside the table, n is clamped there.  Points
+// from n_chunk up to ld (the row padding) get 0 in all three.  tab = table_nu | c_self | c_foreign | t_exp, n_tab each.
+__global__ void __launch_bounds__(256)
+k3_continuum_rows(int64_t n_chunk, int64_t ld, int64_t i_begin, int64_t n_total, double x0, double dx, double x_last,
+                  const double *__restrict__ tab, int64_t n_tab, float *__restrict__ rows) {
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < ld; i += (int64_t)gridDim.x * blockDim.x) {
+        float cs = 0.f, cf = 0.f, n = 0.f;
+        if (i < n_chunk) {
+            const double x = axis_value(i_begin + i, n_total, x0, dx, x_last);
+            const bool inside = !(x < tab[0] || x > tab[n_tab - 1]);
+            cs = inside ? (float)np_interp(x, tab, tab + n_tab, n_tab) : 0.f;
+            cf = inside ? (float)np_interp(x, tab, tab + 2 * n_tab, n_tab) : 0.f;
+            n = (float)np_interp(x, tab, tab + 3 * n_tab, n_tab);
+        }
+        rows[i] = cs;
+        rows[ld + i] = cf;
+        rows[2 * ld + i] = n;
+    }
+}
+
+// A layer of the add, formed on the host in FP64 and rounded once: the products n rho x and n rho (1 - x) never leave
+// the normal FP32 range, where x C_s alone (1e-6 x 1e-30 in the stratosphere) would reach the flush-to-zero range.
+struct ContLayer {
+    float a;                 // n_l rho_l x_l
+    float b;                 // n_l rho_l (1 - x_l)
+    float log2_tref_t;       // log2(t_ref / T_l)
+    float c2_over_2t;        // c2 / (2 T_l)
+    int row;                 // the layer's row of the k matrix
+    int pad;
+};
+
+// tanh(y) for y >= 0, to a few FP32 ulp relative everywhere: next to 0 cm^-1, y = c2 nu / 2T is ~3e-6, where
+// (1 - e^-2y) / (1 + e^-2y) would lose every digit to cancellation.  Below 1/4 the odd series to y^9 (truncation < 1e-8
+// relative), above it that quotient with e^-2y <= 0.61 (one ex2, one rcp).
+__device__ __forceinline__ float k3_cont_tanh(float y) {
+    if (y < 0.25f) {
+        const float y2 = y * y;
+        float p = fmaf(y2, 2.1869488536e-2f, -5.3968253968e-2f);      // 62/2835, -17/315
+        p = fmaf(y2, p, 1.3333333333e-1f);                             // 2/15
+        p = fmaf(y2, p, -3.3333333333e-1f);                            // -1/3
+        return fmaf(y * y2, p, y);
+    }
+    const float t = k3_ex2(y * -2.8853900817779268f);                // e^-2y
+    return (1.f - t) * k3_rcp(1.f + t);
+}
+
+// k[row][i] += k_c(nu_i) for the listed layers (those with x_l > 0; no other row is read or written), on the owned chunk.
+// A thread owns four points (one float4: ld is a multiple of 4), loads their C_s, C_f, n once and walks the layers,
+// K3_CONT_UNROLL rows' loads in flight before their math.  A pointwise function of the chunk: no atomics, and
+// tile-aligned chunks give the rows of the whole grid bit for bit.
+constexpr int K3_CONT_UNROLL = 4;
+__global__ void __launch_bounds__(256)
+k3_continuum_add(float *__restrict__ kmat, int64_t ld, const ContLayer *__restrict__ layers, int n_list,
+                 const float *__restrict__ rows, int64_t i_begin, int64_t n_total, double x0, double dx, double x_last) {
+    const int64_t nvec = ld >> 2;
+    for (int64_t v = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; v < nvec; v += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t i0 = v << 2;
+        const float4 cs4 = *reinterpret_cast<const float4 *>(rows + i0);
+        const float4 cf4 = *reinterpret_cast<const float4 *>(rows + ld + i0);
+        const float4 n4 = *reinterpret_cast<const float4 *>(rows + 2 * ld + i0);
+        const float cs[4] = {cs4.x, cs4.y, cs4.z, cs4.w}, cf[4] = {cf4.x, cf4.y, cf4.z, cf4.w};
+        const float nn[4] = {n4.x, n4.y, n4.z, n4.w};
+        float nu[4];
+#pragma unroll
+        for (int q = 0; q < 4; ++q) nu[q] = (float)axis_value(i_begin + i0 + q, n_total, x0, dx, x_last);
+        for (int j0 = 0; j0 < n_list; j0 += K3_CONT_UNROLL) {
+            float4 k4[K3_CONT_UNROLL];
+#pragma unroll
+            for (int j = 0; j < K3_CONT_UNROLL; ++j)
+                if (j0 + j < n_list) k4[j] = *reinterpret_cast<const float4 *>(kmat + (int64_t)layers[j0 + j].row * ld + i0);
+#pragma unroll
+            for (int j = 0; j < K3_CONT_UNROLL; ++j) {
+                if (j0 + j < n_list) {
+                    const ContLayer c = layers[j0 + j];
+                    float kk[4] = {k4[j].x, k4[j].y, k4[j].z, k4[j].w};
+#pragma unroll
+                    for (int q = 0; q < 4; ++q) {
+                        // (t_ref/T)^n as one ex2; the clamp keeps it finite, so a zero coefficient gives exactly 0
+                        const float tn = k3_ex2(fminf(nn[q] * c.log2_tref_t, 126.f));
+                        const float r = nu[q] * k3_cont_tanh(c.c2_over_2t * nu[q]);
+                        kk[q] += r * fmaf(c.a, tn * cs[q], c.b * cf[q]);
+                    }
+                    *reinterpret_cast<float4 *>(kmat + (int64_t)c.row * ld + i0) = make_float4(kk[0], kk[1], kk[2], kk[3]);
+                }
+            }
+        }
+    }
+}
+
 // Band totals of the band pass: out[d][b][j] = scale * sum of band b's segments at level j of pass d (0 up, 1 down), for
 // the bands list[0 .. n_list).  G threads take one (d, b, j): thread t adds segments t, t + G, ... in order, then a fixed
 // xor butterfly over the warp and, for G = 256, the eight warps' values in a fixed tree.  The host picks G from the

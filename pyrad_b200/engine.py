@@ -174,6 +174,50 @@ def solar_source_args(irradiance=None, mu_sun=1.0):
     return nu, s, mu_sun
 
 
+CONTINUUM_KEYS = ("nu", "self", "foreign", "texp")
+
+
+def continuum_args(table=None, mole_fraction=None):
+    """Checked arguments of prb_set_continuum: (table_nu, c_self, c_foreign, t_exp, t_ref, p_ref, mole_fraction).
+
+    table: None (no continuum: empty arrays) or a dict in MT_CKD's form with the 1-d arrays "nu" (cm-1, finite and strictly
+    ascending, at least two entries), "self" and "foreign" (cm2 molecule-1 (cm-1)-1, finite and >= 0) and "texp" (the
+    self coefficient's temperature exponent, finite), all of one length, and optional "t_ref" (K, default 296.0) and
+    "p_ref" (hPa, default 1013.0), finite and > 0.  mole_fraction: the continuum gas's mole fraction per layer, a
+    non-empty 1-d array with every entry in [0, 1]; ignored without a table.  ValueError otherwise."""
+    if table is None:
+        z = np.zeros(0)
+        return z, z, z, z, 296.0, 1013.0, z
+    if not isinstance(table, dict):
+        raise ValueError("continuum table must be None or a dict with keys %s" % (CONTINUUM_KEYS,))
+    missing = [k for k in CONTINUUM_KEYS if k not in table]
+    if missing:
+        raise ValueError("continuum table lacks %s" % missing)
+    unknown = sorted(set(table) - set(CONTINUUM_KEYS) - {"t_ref", "p_ref"})
+    if unknown:
+        raise ValueError("continuum table: unknown keys %s" % unknown)
+    nu, cs, cf, tx = (_f64(table[k]) for k in CONTINUUM_KEYS)
+    if nu.ndim != 1 or nu.size < 2 or not (nu.shape == cs.shape == cf.shape == tx.shape):
+        raise ValueError("continuum table: nu, self, foreign and texp must be 1-d arrays of one length, at least two entries")
+    if not np.all(np.isfinite(nu)) or not np.all(np.diff(nu) > 0):
+        raise ValueError("continuum table: nu must be finite and strictly ascending")
+    if not np.all(np.isfinite(cs) & (cs >= 0) & np.isfinite(cf) & (cf >= 0)):
+        raise ValueError("continuum table: self and foreign must be finite and >= 0")
+    if not np.all(np.isfinite(tx)):
+        raise ValueError("continuum table: texp must be finite")
+    t_ref, p_ref = float(table.get("t_ref", 296.0)), float(table.get("p_ref", 1013.0))
+    if not (np.isfinite(t_ref) and t_ref > 0 and np.isfinite(p_ref) and p_ref > 0):
+        raise ValueError("continuum table: t_ref and p_ref must be finite and > 0")
+    if mole_fraction is None:
+        raise ValueError("a continuum needs the mole fraction of its gas per layer")
+    x = _f64(mole_fraction)
+    if x.ndim != 1 or x.size < 1:
+        raise ValueError("mole_fraction must be a non-empty 1-d array, one entry per layer")
+    if not np.all((x >= 0) & (x <= 1)):
+        raise ValueError("every mole fraction must be finite and in [0, 1]")
+    return nu, cs, cf, tx, t_ref, p_ref, x
+
+
 class Engine:
     """One engine per process per device (the C ABI's contract)."""
 
@@ -427,6 +471,19 @@ class Engine:
 
     def xsc_clear(self):
         _lib.check(self._lib.prb_xsc_clear(self._h))
+
+    def set_continuum(self, table=None, mole_fraction=None):
+        """A water-vapour continuum in MT_CKD's form for every later atmosphere() / gas cell with len(mole_fraction)
+        layers (prb_set_continuum; arguments as continuum_args).  Row l of the k matrix gains, before the fold,
+        n_l rho_l R(nu, T_l) [x_l (t_ref/T_l)^texp C_self + (1 - x_l) C_foreign], the table interpolated onto the grid
+        (0 outside it for the coefficients).  The table must suit the line shape: MT_CKD's belongs to lines cut at
+        25 cm-1 with the 25 cm-1 value subtracted, this path cuts at 5 P/p0 cm-1.  No arguments: no continuum again."""
+        nu, cs, cf, tx, t_ref, p_ref, x = continuum_args(table, mole_fraction)
+        if not nu.size:
+            _lib.check(self._lib.prb_set_continuum(self._h, 0, None, None, None, None, t_ref, p_ref, 0, None))
+            return
+        _lib.check(self._lib.prb_set_continuum(self._h, nu.size, _dp(nu), _dp(cs), _dp(cf), _dp(tx), t_ref, p_ref,
+                                               x.size, _dp(x)))
 
     def atmosphere_call(self, depth_cm, t_layer, p_layer, conc, molmass, q_t, q_296, window, t_surface, range_max):
         """The prb_atmosphere call with its arguments marshalled ONCE: returns a zero-argument callable for callers that

@@ -15,7 +15,11 @@ without the surface.  Then, on the same surface and top, adds a 5772 K blackbody
 mu_sun = 0.5 (prb_set_solar_source, both reflections), times the same two calls as ratios to the sunless boundary calls
 timed right before them, and reports the sunlight at the top (mu_sun sum S res), the beam at the surface, the sunlight
 leaving the top and the largest solar heating rate with its layer, each as the result with the Sun minus the result
-without it.  Prints one JSON line; writes nothing.
+without it.  Last, a water-vapour continuum (prb_set_continuum) from a SYNTHETIC table in MT_CKD's form (seeded,
+log-uniform coefficients, not MT_CKD's values) with cfg4's H2O profile: the column itself (prb_atmosphere) timed five
+times without and five times with it, alternating, the median difference against the add kernel's algorithmic bytes
+(the k matrix read and written once, 2 L N 4) and the copy bandwidth, and the change it makes to the OLR, the surface
+down flux and RRTMG's 16 band fluxes (3 nodes).  Prints one JSON line; writes nothing.
 
     python scripts/flux_bench.py [--reps 30] [--warmup 3]
 """
@@ -97,6 +101,52 @@ def solar_section(e, stream, args, w, mu, wt, calls, eps_table):
         e.set_solar_source()
         e.set_flux_boundaries()
     return res
+
+
+def synthetic_continuum(seed=4, lo=0.0, hi=5000.0, spacing=10.0):
+    """A table in MT_CKD's form, NOT MT_CKD's values: coefficients log-uniform in [1e-27, 1e-21] cm2 molecule-1 (cm-1)-1,
+    exponents uniform in [0, 6], entries `spacing` cm-1 apart (tests/continuum_oracle.synthetic_table)."""
+    rng = np.random.default_rng(seed)
+    m = int(round((hi - lo) / spacing)) + 1
+    return {"nu": np.linspace(lo, hi, m), "self": 10.0 ** rng.uniform(-27, -21, m),
+            "foreign": 10.0 ** rng.uniform(-27, -21, m), "texp": rng.uniform(0.0, 6.0, m)}
+
+
+def continuum_section(e, stream, w, column, mu, wt, rrtmg, copy_bytes_per_s, runs=5):
+    """The column with and without the continuum, alternating; then what the continuum changes in the 3-node fluxes."""
+    table, x = synthetic_continuum(), np.asarray(w["conc"])[:, 0]
+    L, n = len(w["T"]), e.n_chunk
+
+    def fluxes():
+        up, down = e.atmosphere_fluxes(mu, wt)
+        bu, bd = e.atmosphere_band_fluxes(mu, wt, rrtmg)
+        return up, down, bu, bd
+
+    plain, wet = [], []
+    try:
+        for i in range(runs):
+            e.set_continuum()
+            plain += timed(stream, column, 1 if i == 0 else 0, 1)
+            e.set_continuum(table, x)
+            wet += timed(stream, column, 1 if i == 0 else 0, 1)
+        wet_f = fluxes()
+        e.set_continuum()
+        column()
+        dry_f = fluxes()
+    finally:
+        e.set_continuum()
+    diff = float(np.median(wet) - np.median(plain))
+    add_bytes = 2 * L * n * 4
+    return {"table": "synthetic (seeded, log-uniform 1e-27..1e-21, t_exp 0..6, 10 cm-1 spacing over 0-5000 cm-1; "
+                     "not MT_CKD)", "mole_fraction": "cfg4 H2O profile", "runs": runs,
+            "plain_ms": plain, "continuum_ms": wet, "plain_ms_median": float(np.median(plain)),
+            "continuum_ms_median": float(np.median(wet)), "median_difference_ms": diff,
+            "add_bytes": add_bytes, "add_ms_at_copy_bandwidth": add_bytes / copy_bytes_per_s * 1e3,
+            "olr_change_w_m2": float(wet_f[0][-1] - dry_f[0][-1]),
+            "surface_down_change_w_m2": float(wet_f[1][0] - dry_f[1][0]),
+            "rrtmg_band_edges": [float(v) for v in rrtmg],
+            "band_olr_change_w_m2": [float(v) for v in wet_f[2][:, -1] - dry_f[2][:, -1]],
+            "band_surface_down_change_w_m2": [float(v) for v in wet_f[3][:, 0] - dry_f[3][:, 0]]}
 
 
 def main():
@@ -189,6 +239,7 @@ def main():
     finally:
         e.set_flux_boundaries()
     out["solar"] = solar_section(e, stream, args, w, mu, wt, calls, eps_table)
+    out["continuum"] = continuum_section(e, stream, w, column, mu, wt, rrtmg, peaks["copy_bytes_per_s"])
     e.close()
     print(json.dumps(out))
 
