@@ -151,7 +151,13 @@ int     prb_debug_parse_double(const char *text, int64_t n_bytes, double *value)
 
 /* ---- grid (a10/a11): point i of the FULL grid sits at range_min + i*res, i in [0, n_total).
  * This engine (rank) owns the contiguous chunk [i_begin, i_end).  Computes every line's
- * arrayIndex = int((nu0 - range_min)/res) (FP64 divide, truncation toward zero) on the device. */
+ * arrayIndex = int((nu0 - range_min)/res) (FP64 divide, truncation toward zero) on the device.
+ * A grid change (this call, even with the same grid, or prb_gas_cell_host) drops the resident column: until the next
+ * prb_atmosphere succeeds, its readers (prb_atmosphere_read, _read_f32, _result_dev, _kmatrix_dev, _integrate, _fluxes,
+ * _band_fluxes) return PRB_ERR_STATE instead of reading the old k matrix on the new grid.  So do a prb_atmosphere that
+ * fails, a prb_gas_cell_host whose line list fails its check, and prb_peer_alloc / prb_peer_disconnect.  The flux
+ * boundaries, the Sun and the continuum are settings and stay.  (ABI version 3 holds: only a sequence whose result was
+ * undefined now fails.) */
 int prb_set_grid(prb_engine *e, double range_min, double res,
                  int64_t n_total, int64_t i_begin, int64_t i_end);
 

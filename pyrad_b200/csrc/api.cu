@@ -219,6 +219,10 @@ struct prb_engine {
     DevBuf<FoldLayer> fold;
     int64_t kmat_ld = 0;
     int atm_layers = 0;
+    // the resident column (k matrix, spectra, the flux calls' layer constants) belongs to the current grid: cleared by
+    // every grid change and by a prb_atmosphere that fails, so that no reader labels the old k with the new wavenumbers
+    // (atm_layers itself stays: prb_atmosphere zeroes the k matrix when it changes)
+    bool atm_valid = false;
     // the last column's layer constants and fold policy, for prb_atmosphere_fluxes
     std::vector<double> atm_depth, atm_t;
     double atm_t_surface = 0, atm_range_max = 0;
@@ -712,6 +716,7 @@ extern "C" int prb_set_grid(prb_engine *e, double range_min, double res, int64_t
     e->last.valid = false;
     e->xsc_rows_valid = false;
     e->group_rows_valid = false;
+    e->atm_valid = false;
     return PRB_OK;
 }
 
@@ -1477,6 +1482,7 @@ static int atmosphere_impl(prb_engine *e, int32_t n_layers, int32_t n_groups, co
                            const double *q_t, const double *q_296, const int64_t *window_len, double t_surface,
                            double range_max, const UploadPipe *pipe) {
     if (!e) return fail(PRB_ERR_ARG, "null engine");
+    e->atm_valid = false;                                       // a failed call leaves no column; set once this one is enqueued
     if (!e->grid_set && !pipe) return fail(PRB_ERR_STATE, "prb_atmosphere: set the grid first");
     if (!e->seg.empty() && !pipe)
         return fail(PRB_ERR_STATE, "prb_atmosphere: the line list was uploaded in groups (prb_upload_line_groups); the column "
@@ -1507,6 +1513,9 @@ static int atmosphere_impl(prb_engine *e, int32_t n_layers, int32_t n_groups, co
     if (continuum && (int)e->cont_x.size() != n_layers)
         return fail(PRB_ERR_ARG, "prb_atmosphere: the continuum's mole fractions were set for another number of layers "
                                  "(prb_set_continuum with the same n_layers, or with n_table = 0 to clear)");
+    // np.linspace(range_min, range_max, 1) is [range_min]: the only point of a one-point grid is its first, not range_max
+    // (axis_value returns x_last for the last point)
+    if (e->n_total == 1) range_max = e->range_min;
     const int xsc_before = e->xsc_build_launches;
     if ((rc = ensure_xsc_rows(e))) return rc;
     const int xsc_launches = e->xsc_build_launches - xsc_before;   // table resamplings this call had to enqueue
@@ -1833,6 +1842,7 @@ static int atmosphere_impl(prb_engine *e, int32_t n_layers, int32_t n_groups, co
         CK(cudaEventElapsedTime(&e->t_k3, e->ev[3 * n_batches], e->ev[3 * n_batches + 1]));
     }
     e->last.valid = false;
+    e->atm_valid = true;                                        // (a flag or peer error below still leaves it sized right)
     if (ps.connected) {
         unsigned int perr = 0;
         CK(cudaMemcpy(&perr, e->peer_err.p, sizeof perr, cudaMemcpyDeviceToHost));
@@ -1854,21 +1864,21 @@ extern "C" int prb_atmosphere(prb_engine *e, int32_t n_layers, int32_t n_groups,
 }
 
 extern "C" int prb_atmosphere_result_dev(prb_engine *e, void **radiance_dev, void **transmittance_dev) {
-    if (!e || !e->atm_layers) return fail(PRB_ERR_STATE, "prb_atmosphere_result_dev: run prb_atmosphere first");
+    if (!e || !e->atm_valid) return fail(PRB_ERR_STATE, "prb_atmosphere_result_dev: run prb_atmosphere on the current grid first");
     if (radiance_dev) *radiance_dev = e->res_rad;
     if (transmittance_dev) *transmittance_dev = e->res_trans;
     return PRB_OK;
 }
 
 extern "C" int prb_atmosphere_kmatrix_dev(prb_engine *e, void **kmat_dev, int64_t *ld) {
-    if (!e || !e->atm_layers) return fail(PRB_ERR_STATE, "prb_atmosphere_kmatrix_dev: run prb_atmosphere first");
+    if (!e || !e->atm_valid) return fail(PRB_ERR_STATE, "prb_atmosphere_kmatrix_dev: run prb_atmosphere on the current grid first");
     if (kmat_dev) *kmat_dev = e->kmat.p;
     if (ld) *ld = e->kmat_ld;
     return PRB_OK;
 }
 
 extern "C" int prb_atmosphere_read(prb_engine *e, double *radiance_host, double *transmittance_host) {
-    if (!e || !e->atm_layers) return fail(PRB_ERR_STATE, "prb_atmosphere_read: run prb_atmosphere first");
+    if (!e || !e->atm_valid) return fail(PRB_ERR_STATE, "prb_atmosphere_read: run prb_atmosphere on the current grid first");
     CK(cudaSetDevice(e->device));
     const int64_t nc = chunk_len(e);
     // both spectra cross PCIe into one pinned staging block (grown on demand, kept), then widen to the caller's doubles
@@ -1893,7 +1903,7 @@ extern "C" int prb_atmosphere_read(prb_engine *e, double *radiance_host, double 
 }
 
 extern "C" int prb_atmosphere_read_f32(prb_engine *e, float *radiance_host, float *transmittance_host) {
-    if (!e || !e->atm_layers) return fail(PRB_ERR_STATE, "prb_atmosphere_read_f32: run prb_atmosphere first");
+    if (!e || !e->atm_valid) return fail(PRB_ERR_STATE, "prb_atmosphere_read_f32: run prb_atmosphere on the current grid first");
     CK(cudaSetDevice(e->device));
     const int64_t nc = chunk_len(e);
     if (radiance_host) CK(cudaMemcpyAsync(radiance_host, e->res_rad, sizeof(float) * nc, cudaMemcpyDeviceToHost, e->stream));
@@ -2012,7 +2022,7 @@ static cudaError_t flux_boundaries_prepare(prb_engine *e, double dx, K3FArgs &up
 // The checks shared by the flux calls: a column on the device, a quadrature of 1 to 4 nodes with mu in (0, 1] and finite
 // weights > 0, and few enough layers for k3_flux_tma's per-level accumulators.
 static int flux_check(prb_engine *e, const char *fn, int32_t n_mu, const double *mu, const double *weight) {
-    if (!e || !e->atm_layers) return fail(PRB_ERR_STATE, std::string(fn) + ": run prb_atmosphere first");
+    if (!e || !e->atm_valid) return fail(PRB_ERR_STATE, std::string(fn) + ": run prb_atmosphere on the current grid first");
     if (n_mu < 1 || n_mu > 4 || !mu || !weight) return fail(PRB_ERR_ARG, std::string(fn) + ": need 1 <= n_mu <= 4, mu and weight");
     for (int i = 0; i < n_mu; ++i)
         if (!(mu[i] > 0 && mu[i] <= 1) || !(weight[i] > 0 && std::isfinite(weight[i])))
@@ -2309,6 +2319,7 @@ extern "C" int prb_peer_alloc(prb_engine *e, int rank, int world, int64_t max_ch
     CK(cudaSetDevice(e->device));
     CK(cudaStreamSynchronize(e->stream));
     peer_release(e);
+    e->atm_valid = false;                                       // the last column's spectra may have been in that buffer
     PeerState &ps = e->peer;
     ps.rank = rank; ps.world = world;
     ps.ld = (max_chunk_points + 63) & ~int64_t(63);
@@ -2354,6 +2365,7 @@ extern "C" int prb_peer_disconnect(prb_engine *e) {
     peer_release(e);
     e->res_rad = e->res_trans = nullptr;
     e->atm_layers = 0;
+    e->atm_valid = false;
     return PRB_OK;
 }
 
@@ -2417,8 +2429,8 @@ extern "C" int prb_integrate_spectrum(prb_engine *e, int64_t n, const double *sp
 
 extern "C" int prb_atmosphere_integrate(prb_engine *e, double unit_angle, double res, double *radiance_integral,
                                         double *transmittance_sum) {
-    if (!e || !e->atm_layers || !e->res_rad)
-        return fail(PRB_ERR_STATE, "prb_atmosphere_integrate: run prb_atmosphere first");
+    if (!e || !e->atm_valid || !e->res_rad)
+        return fail(PRB_ERR_STATE, "prb_atmosphere_integrate: run prb_atmosphere on the current grid first");
     CK(cudaSetDevice(e->device));
     const int64_t nc = chunk_len(e);
     int rc;
@@ -2772,6 +2784,7 @@ extern "C" int prb_gas_cell_host(prb_engine *e, int64_t n, const double *nu0, co
     e->lines_set = false;
     e->grid_set = false;
     e->last.valid = false;
+    e->atm_valid = false;                                       // the grid changes below, as in prb_set_grid
     int rc = alloc_line_storage(e, n);
     if (rc) return rc;
     e->n_lines = n;
@@ -2843,6 +2856,7 @@ extern "C" int prb_gas_cell_host(prb_engine *e, int64_t n, const double *nu0, co
     if (rc) return rc;                                          // a failed launch sequence: its own message stands
     memcpy(&e->s_max, e->pin_scal, sizeof(double));             // max|S296|, for the planning of later calls
     const unsigned int vf = (unsigned int)e->pin_scal[1];
+    if (vf & 3u) e->atm_valid = false;                          // a column from a list that fails the check is garbage
     if (vf & 1u) return fail(PRB_ERR_ARG, "prb_gas_cell_host: nu0 must be ascending");
     if (vf & 2u) return fail(PRB_ERR_ARG, "prb_gas_cell_host: group id out of range");
     e->lines_set = true;

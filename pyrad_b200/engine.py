@@ -710,7 +710,7 @@ class Engine:
 def linspace_axis(range_min, range_max, n):
     """(x0, dx, x_last, n) reproducing np.linspace(range_min, range_max, n, endpoint=True) bit for bit:
     numpy forms arange(n) * step + start and overwrites the last sample with stop (Layer.xAxis,
-    pyradClasses.py:703-705)."""
+    pyradClasses.py:703-705).  One point is [range_min]: numpy overwrites nothing then."""
     n = int(n)
     step = (range_max - range_min) / (n - 1) if n > 1 else 0.0
-    return float(range_min), float(step), float(range_max), n
+    return float(range_min), float(step), float(range_max if n > 1 else range_min), n

@@ -18,7 +18,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def test_linspace_axis_reproduces_numpy_bitwise():
-    for a, b, n in [(600.0, 700.0, 10000), (0.0, 3000.0, 3000000), (1000.0, 1008.0, 8000)]:
+    for a, b, n in [(600.0, 700.0, 10000), (0.0, 3000.0, 3000000), (1000.0, 1008.0, 8000), (600.0, 600.1, 1),
+                    (600.0, 600.1, 2)]:
         x0, dx, xl, n_ = eng.linspace_axis(a, b, n)
         ref = np.linspace(a, b, n, endpoint=True)
         mine = np.arange(n) * dx + x0
