@@ -25,6 +25,8 @@
  *   (absent upstream) a grey or spectral surface and a warm top for both flux calls -> prb_set_flux_boundaries
  *   (absent upstream) an absorbed, reflected solar beam for both flux calls        -> prb_set_solar_source
  *   (absent upstream) a water-vapour continuum in the column's k matrix            -> prb_set_continuum
+ *   (absent upstream) per-layer radiative kernels of the outgoing and surface fluxes -> prb_atmosphere_save_base,
+ *                                                                                    prb_atmosphere_layer_kernels
  *
  * Conventions: every entry point is extern "C", returns int (0 = PRB_OK, < 0 = error) unless
  * noted, takes plain pointers and sizes.  Pointers named *_host / unmarked are caller-owned host
@@ -339,6 +341,29 @@ int prb_set_flux_boundaries(prb_engine *e, int64_t n_table, const double *table_
  * the Sun bit for bit. */
 int prb_set_solar_source(prb_engine *e, int64_t n_table, const double *table_nu, const double *table_irradiance,
                          double mu_sun);
+/* Keep a copy of the current column on the device as the base of prb_atmosphere_layer_kernels: its k matrix, depths,
+ * layer and surface temperatures and Planck policy, and its optical depth S = sum_l k_l depth_l per point in FP64.  The
+ * current column stays readable.  A second call replaces the base.  The copy is an engine buffer the size of the k matrix
+ * (2 GB for 100 layers x 5 M points), held until prb_destroy.  Every grid or chunk change drops the base (prb_set_grid,
+ * even to the same grid; prb_gas_cell_host; prb_peer_alloc; prb_peer_disconnect); prb_atmosphere keeps it, failed or
+ * not.  PRB_ERR_STATE without a valid column. */
+int prb_atmosphere_save_base(prb_engine *e);
+/* Radiative kernels of the base column against the current one (the last prb_atmosphere or prb_gas_cell_host on the
+ * grid the base was saved on, with as many layers): the exact change of the flux leaving the top and of the flux reaching
+ * the surface when layer l alone of the base takes the current column's state (row k_l, depth_l, T_l).  toa_up and
+ * surf_down: [n_bands][L+1] doubles each, this chunk's share, either may be NULL; bands, edge rules, quadrature rules and
+ * the non-finite rule as prb_atmosphere_band_fluxes.  Entry l + 1 is layer l's kernel,
+ *   toa_up[b][l+1] = F_up,top[base, l := current] - F_up,top[base],  surf_down[b][l+1] = F_down,sfc[...] - F_down,sfc[base];
+ * entry 0 of toa_up is the surface temperature's, F_up,top[base, T_s := T'_s] - F_up,top[base], and entry 0 of surf_down
+ * is 0 (a black surface's temperature does not reach its own downward flux).  Both are formed per layer from the base
+ * radiance, the two columns' transmittances and Planck terms (differences formed without cancellation) and the base
+ * transmittance of the other layers (from the FP64 S): no subtraction of two flux calls.  A layer whose row, depth and
+ * temperature are bit-identical in both columns contributes exactly 0.  A warm top (prb_set_flux_boundaries with
+ * n_table = 0, t_top > 0) is the same downward start for both columns and is allowed; a surface emissivity table or a
+ * Sun gives PRB_ERR_STATE, as do no base, no valid current column and different layer counts.  Deterministic; under a
+ * peer connection the call stays local. */
+int prb_atmosphere_layer_kernels(prb_engine *e, int32_t n_mu, const double *mu, const double *weight, int32_t n_bands,
+                                 const double *edges, double *toa_up, double *surf_down);
 int prb_set_option(prb_engine *e, int option, int64_t value);
 
 /* ---- section 8(f) rows beside the hot path -------------------------------------------------------

@@ -936,8 +936,67 @@ class Atmosphere(list):
                        band_heating_rate=np.array([heatingRate(u, d, depth, T, P) for u, d in zip(bu, bd)]))
         return out
 
-    def _column(self, surfaceTemperature, result, continuum=None):
-        """Run the column on the device (prb_atmosphere) and return result(engine) while its state is in place."""
+    def columnKernels(self, surfaceTemperature, perturbed, perturbedSurfaceTemperature=None, mu=None, weights=None,
+                      bands=None, topTemperature=0.0, continuum=None):
+        """Radiative kernels of this column against ``perturbed`` (prb_atmosphere_save_base, then
+        prb_atmosphere_layer_kernels): the exact change of the upward flux at the top and of the downward flux at the
+        surface when layer l alone of this column takes the state of perturbed's layer l (its k row, depth and
+        temperature).  perturbed is another Atmosphere with as many layers on the same grid and with the same line list
+        (the same isotopologues and loaded line range); both columns run here, this one first, with the same continuum
+        setting.  perturbedSurfaceTemperature (default: surfaceTemperature) gives the surface's entry.  Quadrature
+        (default 3-node Gauss-Legendre on [0, 1]) and bands as in columnFluxes; without bands, one band holds every point.
+        The surface is black; topTemperature > 0 sends B(nu, topTemperature) down from the top of both columns.
+        Returns a dict: band_edges; toa_up and surface_down, (n_bands, L) in W m-2 -- entry l is layer l's kernel;
+        toa_up_surface, (n_bands,), the surface temperature's entry; mu and weights.  The entries are exact single-layer
+        differences, not linearisations, and the k(T) dependence is included.  The kernels shard like the fluxes
+        (distributed.sum_over_ranks adds the ranks' shares).
+
+        The temperature kernel of the OLR, per kelvin (the reference's Q tables are tabulated at integer temperatures,
+        so a 1 K step is natural)::
+
+            warm = Atmosphere("warm")             # the same layers, every one 1 K warmer
+            ...
+            k = base.columnKernels(288.0, warm, perturbedSurfaceTemperature=289.0)
+            olr_kernel = k["toa_up"].sum(axis=0)  # W m-2 K-1 per layer
+        """
+        _eng.flux_boundary_args(None, "lambertian", topTemperature)               # ValueError before the columns run
+        if not isinstance(perturbed, Atmosphere):
+            raise ValueError("columnKernels: perturbed must be an Atmosphere")
+        layers, other = list(self), list(perturbed)
+        if not layers or len(layers) != len(other):
+            raise ValueError(f"columnKernels needs two columns with as many layers ({len(layers)} and {len(other)})")
+        if (layers[0].rangeMin, layers[0].rangeMax, layers[0].resolution) != \
+                (other[0].rangeMin, other[0].rangeMax, other[0].resolution):
+            raise ValueError("columnKernels needs the perturbed column on the same grid")
+        if mu is None and weights is None:
+            x, w = np.polynomial.legendre.leggauss(3)
+            mu, weights = (x + 1) / 2, w / 2
+        mu, weights = np.atleast_1d(np.asarray(mu, dtype=np.float64)), np.atleast_1d(np.asarray(weights, dtype=np.float64))
+        if mu.shape != weights.shape or not 1 <= mu.size <= 4:
+            raise ValueError("columnKernels needs 1 to 4 quadrature nodes, as many weights as mu")
+        if bands is None:
+            bands = np.array([layers[0].rangeMin, layers[0].rangeMax + BASE_RESOLUTION])
+        bands = np.asarray(bands, dtype=np.float64)
+        if bands.ndim != 1 or bands.size < 2 or not np.all(np.isfinite(bands)) or not np.all(np.diff(bands) > 0):
+            raise ValueError("columnKernels: bands must be a 1-d array of at least 2 finite, strictly ascending edges")
+        t_pert = surfaceTemperature if perturbedSurfaceTemperature is None else perturbedSurfaceTemperature
+
+        def kernels(e):
+            e.set_flux_boundaries(None, "lambertian", topTemperature)
+            try:
+                return e.atmosphere_layer_kernels(mu, weights, bands)
+            finally:
+                e.set_flux_boundaries()
+
+        base_lines = self._column(surfaceTemperature, lambda e: (e.save_column_base(), e._column_lines)[1], continuum)
+        up, down = perturbed._column(t_pert, kernels, continuum, resident_lines=base_lines)
+        return {"band_edges": bands, "toa_up": up[:, 1:], "surface_down": down[:, 1:], "toa_up_surface": up[:, 0],
+                "mu": mu, "weights": weights}
+
+    def _column(self, surfaceTemperature, result, continuum=None, resident_lines=None):
+        """Run the column on the device (prb_atmosphere) and return result(engine) while its state is in place.
+        resident_lines: the line list the engine holds on this grid (a previous _column's), which must be this column's
+        too; the column then runs without a new upload or grid (which would drop a saved base)."""
         layers = list(self)
         if not layers:
             raise ValueError("atmosphere has no layers")
@@ -978,8 +1037,13 @@ class Atmosphere(list):
         global _RESIDENT_KEY
         _RESIDENT_KEY = None
         e = engine()
-        e.upload_lines(lines, n_groups=max(len(isos), 1))
-        e.set_grid(ref.rangeMin, BASE_RESOLUTION, n)
+        if resident_lines is None:
+            e.upload_lines(lines, n_groups=max(len(isos), 1))
+            e.set_grid(ref.rangeMin, BASE_RESOLUTION, n)
+            e._column_lines = lines
+        elif set(lines) != set(resident_lines) or not all(np.array_equal(lines[k], resident_lines[k]) for k in lines):
+            raise ValueError("columnKernels needs the perturbed column with the same line list (the same isotopologues "
+                             "and loaded line range)")
         conc = [[m.concentration for m in l if not m.exotic for _ in m] for l in layers]
         q_t = [[iso.q[l.T] for m in l if not m.exotic for iso in m] for l in layers]   # KeyError on a non-tabulated T
         window = [_eng.window_len(l.distanceFromCenter, BASE_RESOLUTION) for l in layers]

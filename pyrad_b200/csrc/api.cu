@@ -232,6 +232,16 @@ struct prb_engine {
     DevBuf<float> flux_rows;
     DevBuf<double> band_part, band_out;               // prb_atmosphere_band_fluxes: per-segment level sums, band totals
     DevBuf<int32_t> band_tab;                         // its span, segment, band and strip tables
+    // the base column of prb_atmosphere_layer_kernels (prb_atmosphere_save_base): a copy of a column's k matrix, its FP64
+    // optical depth per point and its layer constants; dropped by every grid or chunk change, kept by prb_atmosphere
+    bool base_valid = false;
+    int base_layers = 0;
+    DevBuf<float> base_kmat;                          // [base_layers][kmat_ld]
+    DevBuf<double> base_s, base_depth_dev;            // [kmat_ld] S = sum_l k_l depth_l; [base_layers] depth_l
+    std::vector<double> base_depth, base_t;
+    double base_t_surface = 0, base_range_max = 0;
+    float base_nu_interp_min = 1e30f;
+    DevBuf<KernLayer> kern_layers;
     // the flux calls' boundaries (prb_set_flux_boundaries); an empty table and t_top = 0: a black surface, 0 at the top
     std::vector<double> bnd_tab;                      // table_nu | table_emissivity
     int bnd_reflection = PRB_REFLECT_LAMBERTIAN;
@@ -339,6 +349,7 @@ extern "C" int prb_destroy(prb_engine *e) {
     e->kmat.release(); e->rad.release(); e->trans.release(); e->fold.release();
     e->flux_layers.release(); e->flux_part.release(); e->flux_out.release(); e->flux_rows.release();
     e->band_part.release(); e->band_out.release(); e->band_tab.release();
+    e->base_kmat.release(); e->base_s.release(); e->base_depth_dev.release(); e->kern_layers.release();
     e->bnd_tab_dev.release(); e->flux_eps.release();
     e->sun_tab_dev.release(); e->sun_nd.release();
     e->k2tab.release(); e->ring_d.release(); e->peer_err.release();
@@ -717,6 +728,7 @@ extern "C" int prb_set_grid(prb_engine *e, double range_min, double res, int64_t
     e->xsc_rows_valid = false;
     e->group_rows_valid = false;
     e->atm_valid = false;
+    e->base_valid = false;
     return PRB_OK;
 }
 
@@ -2114,33 +2126,32 @@ static int64_t first_point_at_or_above(double v, int64_t n, double x0, double dx
     return lo;
 }
 
-extern "C" int prb_atmosphere_band_fluxes(prb_engine *e, int32_t n_mu, const double *mu, const double *weight,
-                                          int32_t n_bands, const double *edges, double *band_up, double *band_down) {
-    if (int rc = flux_check(e, "prb_atmosphere_band_fluxes", n_mu, mu, weight)) return rc;
-    if (n_bands < 1 || !edges) return fail(PRB_ERR_ARG, "prb_atmosphere_band_fluxes: need n_bands >= 1 and n_bands + 1 edges");
+// The band tables of the band passes (k3_flux_tma's BAND pass, k3_kernel_tma) on the owned chunk, uploaded to e->band_tab.
+struct BandPlan {
+    int64_t n_spans = 0, n_seg = 0;
+    std::vector<int32_t> strips, small, big;          // the strips that meet a band; the bands by the size of their sum
+    size_t o_band = 0, o_strips = 0, o_small = 0, o_big = 0;   // offsets into e->band_tab
+};
+
+// Checks the edges (PRB_ERR_ARG) and builds the plan; bp.strips stays empty when no band meets the chunk (nothing is
+// uploaded then).  Band b holds the points with edges[b] <= x_i < edges[b+1], x the Planck axis of the fold.
+static int band_plan(prb_engine *e, const char *fn, int32_t n_bands, const double *edges, double x_last, BandPlan &bp) {
+    if (n_bands < 1 || !edges) return fail(PRB_ERR_ARG, std::string(fn) + ": need n_bands >= 1 and n_bands + 1 edges");
     for (int b = 0; b <= n_bands; ++b)
         if (!std::isfinite(edges[b]) || (b > 0 && !(edges[b] > edges[b - 1])))
-            return fail(PRB_ERR_ARG, "prb_atmosphere_band_fluxes: the edges must be finite and strictly ascending");
-    CK(cudaSetDevice(e->device));
-    const int L = e->atm_layers, n_levels = L + 1;
+            return fail(PRB_ERR_ARG, std::string(fn) + ": the edges must be finite and strictly ascending");
     const int64_t nc = chunk_len(e);
-    const size_t per_dir = (size_t)n_bands * n_levels;
-    auto zeros = [&]() {
-        if (band_up) std::fill(band_up, band_up + per_dir, 0.0);
-        if (band_down) std::fill(band_down, band_down + per_dir, 0.0);
-        return PRB_OK;
-    };
-    if (nc == 0) return zeros();                                // an empty chunk contributes nothing
+    if (nc == 0) return PRB_OK;
     constexpr int SPAN = 128;                                   // points per warp
     const int64_t n_strips = (nc + K3T_STRIP - 1) / K3T_STRIP, n_spans = n_strips * K3F_WARPS;
-    if (n_spans + n_bands + 1 > INT32_MAX) return fail(PRB_ERR_RANGE, "prb_atmosphere_band_fluxes: chunk too long");
-    // Band b holds the points with edges[b] <= x_i < edges[b+1], x the Planck axis of the fold: the chunk-local points
-    // [p[b], p[b+1]), each p the first point at or above its edge by the device's own formula (exact at grid values).
-    const double dx = flux_dx(e);
+    if (n_spans + n_bands + 1 > INT32_MAX) return fail(PRB_ERR_RANGE, std::string(fn) + ": chunk too long");
+    // the chunk-local points [p[b], p[b+1]) of band b, each p the first point at or above its edge by the device's own
+    // formula (exact at grid values)
+    const double dx = e->n_total > 1 ? (x_last - e->range_min) / (double)(e->n_total - 1) : 0.0;
     std::vector<int64_t> p(n_bands + 1);
     for (int b = 0; b <= n_bands; ++b)
-        p[b] = std::clamp<int64_t>(first_point_at_or_above(edges[b], e->n_total, e->range_min, dx, e->atm_range_max) -
-                                   e->i_begin, 0, nc);
+        p[b] = std::clamp<int64_t>(first_point_at_or_above(edges[b], e->n_total, e->range_min, dx, x_last) - e->i_begin,
+                                   0, nc);
     // Segments (span x band) in position order; a band's segments are consecutive: band_seg[b] .. band_seg[b+1].
     std::vector<K3FSpan> spans(n_spans, K3FSpan{0, 0});
     std::vector<uint32_t> seg_range;
@@ -2161,55 +2172,198 @@ extern "C" int prb_atmosphere_band_fluxes(prb_engine *e, int32_t n_mu, const dou
     for (int64_t s = 0; s < n_spans; ++s)                       // one band over all of the span's points: the plain sum
         if (spans[s].nseg == 1 && seg_range[spans[s].seg0] == (uint32_t)(std::min<int64_t>(SPAN, nc - s * SPAN) << 16))
             spans[s].nseg = -1;
-    // the strips that meet a band, and the bands by the size of their sum (k3_flux_band_sum)
-    std::vector<int32_t> strips, small, big;
     for (int64_t t = 0; t < n_strips; ++t)
         for (int w = 0; w < K3F_WARPS; ++w)
-            if (spans[t * K3F_WARPS + w].nseg != 0) { strips.push_back((int32_t)t); break; }
-    if (strips.empty()) return zeros();                         // no band meets the chunk
-    for (int b = 0; b < n_bands; ++b) (band_seg[b + 1] - band_seg[b] > K3F_BAND_WARP_MAX ? big : small).push_back(b);
+            if (spans[t * K3F_WARPS + w].nseg != 0) { bp.strips.push_back((int32_t)t); break; }
+    if (bp.strips.empty()) return PRB_OK;                       // no band meets the chunk
+    for (int b = 0; b < n_bands; ++b) (band_seg[b + 1] - band_seg[b] > K3F_BAND_WARP_MAX ? bp.big : bp.small).push_back(b);
     // one upload: spans | seg_range | band_seg | strips | small | big
     std::vector<int32_t> tab(2 * n_spans + n_seg);
     std::memcpy(tab.data(), spans.data(), sizeof(K3FSpan) * n_spans);
     std::memcpy(tab.data() + 2 * n_spans, seg_range.data(), sizeof(uint32_t) * n_seg);
-    const size_t o_band = tab.size(), o_strips = o_band + band_seg.size(), o_small = o_strips + strips.size(),
-                 o_big = o_small + small.size();
-    for (const auto *v : {&band_seg, &strips, &small, &big}) tab.insert(tab.end(), v->begin(), v->end());
+    bp.o_band = tab.size();
+    bp.o_strips = bp.o_band + band_seg.size();
+    bp.o_small = bp.o_strips + bp.strips.size();
+    bp.o_big = bp.o_small + bp.small.size();
+    for (const auto *v : {&band_seg, &bp.strips, &bp.small, &bp.big}) tab.insert(tab.end(), v->begin(), v->end());
+    bp.n_spans = n_spans;
+    bp.n_seg = n_seg;
+    CK(e->band_tab.ensure(tab.size()));
+    CK(cudaMemcpyAsync(e->band_tab.p, tab.data(), sizeof(int32_t) * tab.size(), cudaMemcpyHostToDevice, e->stream));
+    return PRB_OK;
+}
+
+// out[d][b][j] = scale * sum of band b's segments at level j of pass d (k3_flux_band_sum), part as the band passes left it.
+static cudaError_t band_sums(prb_engine *e, const BandPlan &bp, int n_levels, int32_t n_bands, double scale, double *out) {
+    const int32_t *d_tab = e->band_tab.p;
+    if (!bp.small.empty()) {
+        const int64_t items = 2 * (int64_t)bp.small.size() * n_levels;
+        k3_flux_band_sum<32><<<(unsigned)((items + 7) / 8), 256, 0, e->stream>>>(
+            e->band_part.p, bp.n_seg, n_levels, d_tab + bp.o_small, (int)bp.small.size(), d_tab + bp.o_band, n_bands, scale,
+            out);
+    }
+    if (!bp.big.empty())
+        k3_flux_band_sum<256><<<(unsigned)(2 * bp.big.size() * n_levels), 256, 0, e->stream>>>(
+            e->band_part.p, bp.n_seg, n_levels, d_tab + bp.o_big, (int)bp.big.size(), d_tab + bp.o_band, n_bands, scale, out);
+    return cudaGetLastError();
+}
+
+extern "C" int prb_atmosphere_band_fluxes(prb_engine *e, int32_t n_mu, const double *mu, const double *weight,
+                                          int32_t n_bands, const double *edges, double *band_up, double *band_down) {
+    if (int rc = flux_check(e, "prb_atmosphere_band_fluxes", n_mu, mu, weight)) return rc;
+    CK(cudaSetDevice(e->device));
+    BandPlan bp;
+    if (int rc = band_plan(e, "prb_atmosphere_band_fluxes", n_bands, edges, e->atm_range_max, bp)) return rc;
+    const int L = e->atm_layers, n_levels = L + 1;
+    const size_t per_dir = (size_t)n_bands * n_levels;
+    if (bp.strips.empty()) {                                    // an empty chunk, or no band meets it: nothing
+        if (band_up) std::fill(band_up, band_up + per_dir, 0.0);
+        if (band_down) std::fill(band_down, band_down + per_dir, 0.0);
+        return PRB_OK;
+    }
+    const double dx = flux_dx(e);
     std::vector<FluxLayer> hl;
     K3FArgs up{}, down{};
     CK(flux_layers_upload(e, n_mu, mu, weight, hl, up, down));
-    CK(e->band_tab.ensure(tab.size()));
-    CK(cudaMemcpyAsync(e->band_tab.p, tab.data(), sizeof(int32_t) * tab.size(), cudaMemcpyHostToDevice, e->stream));
-    CK(e->band_part.ensure((size_t)2 * n_levels * n_seg));
+    CK(e->band_part.ensure((size_t)2 * n_levels * bp.n_seg));
     CK(e->band_out.ensure(2 * per_dir));
     const int32_t *d_tab = e->band_tab.p;
     for (K3FArgs *a : {&up, &down}) {
-        a->strips = d_tab + o_strips;
-        a->n_list = (int64_t)strips.size();
+        a->strips = d_tab + bp.o_strips;
+        a->n_list = (int64_t)bp.strips.size();
         a->spans = reinterpret_cast<const K3FSpan *>(d_tab);
-        a->seg_range = reinterpret_cast<const uint32_t *>(d_tab + 2 * n_spans);
-        a->ld_part = n_seg;
+        a->seg_range = reinterpret_cast<const uint32_t *>(d_tab + 2 * bp.n_spans);
+        a->ld_part = bp.n_seg;
     }
     up.part = e->band_part.p;
-    down.part = e->band_part.p + (size_t)n_levels * n_seg;
+    down.part = e->band_part.p + (size_t)n_levels * bp.n_seg;
     CK(flux_boundaries_prepare(e, dx, up, down));
-    const int grid = (int)std::min<int64_t>((int64_t)strips.size(), k3f_minb(n_mu) * (int64_t)e->prop.multiProcessorCount);
+    const int grid = (int)std::min<int64_t>((int64_t)bp.strips.size(), k3f_minb(n_mu) * (int64_t)e->prop.multiProcessorCount);
     const cudaError_t ce = launch_flux_passes<true>(e, n_mu, grid, sizeof(K3FSmem), dx, up, down);
     if (ce != cudaSuccess) return fail(PRB_ERR_CUDA, std::string("k3_flux_tma launch failed: ") + cudaGetErrorString(ce));
     // F_b[j] = 2 pi sum_i w_i mu_i sum_{nu in band b} I_i(nu, j) res
-    const double scale = 2 * 3.141592653589793 * e->res;
-    if (!small.empty()) {
-        const int64_t items = 2 * (int64_t)small.size() * n_levels;
-        k3_flux_band_sum<32><<<(unsigned)((items + 7) / 8), 256, 0, e->stream>>>(
-            e->band_part.p, n_seg, n_levels, d_tab + o_small, (int)small.size(), d_tab + o_band, n_bands, scale, e->band_out.p);
-    }
-    if (!big.empty())
-        k3_flux_band_sum<256><<<(unsigned)(2 * big.size() * n_levels), 256, 0, e->stream>>>(
-            e->band_part.p, n_seg, n_levels, d_tab + o_big, (int)big.size(), d_tab + o_band, n_bands, scale, e->band_out.p);
-    CK(cudaGetLastError());
+    CK(band_sums(e, bp, n_levels, n_bands, 2 * 3.141592653589793 * e->res, e->band_out.p));
     if (band_up) CK(cudaMemcpyAsync(band_up, e->band_out.p, sizeof(double) * per_dir, cudaMemcpyDeviceToHost, e->stream));
     if (band_down)
         CK(cudaMemcpyAsync(band_down, e->band_out.p + per_dir, sizeof(double) * per_dir, cudaMemcpyDeviceToHost, e->stream));
+    CK(cudaStreamSynchronize(e->stream));
+    return PRB_OK;
+}
+
+extern "C" int prb_atmosphere_save_base(prb_engine *e) {
+    if (!e || !e->atm_valid) return fail(PRB_ERR_STATE, "prb_atmosphere_save_base: run prb_atmosphere on the current grid first");
+    CK(cudaSetDevice(e->device));
+    const int L = e->atm_layers;
+    e->base_valid = false;                                      // until the copy below is enqueued
+    CK(e->base_kmat.ensure((size_t)L * std::max<int64_t>(e->kmat_ld, 4)));
+    CK(e->base_s.ensure((size_t)std::max<int64_t>(e->kmat_ld, 4)));
+    CK(e->base_depth_dev.ensure((size_t)L));
+    CK(cudaMemcpyAsync(e->base_depth_dev.p, e->atm_depth.data(), sizeof(double) * L, cudaMemcpyHostToDevice, e->stream));
+    if (e->kmat_ld > 0) {
+        k3_kernel_base<<<stream_grid(e, e->kmat_ld, 4), 256, 0, e->stream>>>(e->kmat.p, e->base_kmat.p, e->kmat_ld, L,
+                                                                             e->base_depth_dev.p, e->base_s.p);
+        CK(cudaGetLastError());
+    }
+    CK(cudaStreamSynchronize(e->stream));                       // (the depths' host copy is pageable)
+    e->base_layers = L;
+    e->base_depth = e->atm_depth;
+    e->base_t = e->atm_t;
+    e->base_t_surface = e->atm_t_surface;
+    e->base_range_max = e->atm_range_max;
+    e->base_nu_interp_min = e->atm_nu_interp_min;
+    e->base_valid = true;
+    return PRB_OK;
+}
+
+template <int NMU>
+static cudaError_t launch_kernel_pair(prb_engine *e, int grid, double dx, const K3KArgs &up, const K3KArgs &down) {
+    const auto fu = k3_kernel_tma<NMU, false>, fd = k3_kernel_tma<NMU, true>;
+    for (const auto &[fn, a] : {std::pair{fu, &up}, std::pair{fd, &down}}) {
+        fn<<<grid, K3T_THREADS, sizeof(K3KSmem), e->stream>>>(e->kmat.p, e->kmat_ld, e->atm_layers, chunk_len(e), e->i_begin,
+                                                              e->n_total, e->range_min, dx, e->base_range_max,
+                                                              e->base_nu_interp_min, *a);
+        const cudaError_t ce = cudaGetLastError();
+        if (ce != cudaSuccess) return ce;
+    }
+    return cudaSuccess;
+}
+
+extern "C" int prb_atmosphere_layer_kernels(prb_engine *e, int32_t n_mu, const double *mu, const double *weight,
+                                            int32_t n_bands, const double *edges, double *toa_up, double *surf_down) {
+    const char *fn = "prb_atmosphere_layer_kernels";
+    if (int rc = flux_check(e, fn, n_mu, mu, weight)) return rc;
+    if (!e->base_valid) return fail(PRB_ERR_STATE, std::string(fn) + ": save a base column on the current grid first "
+                                                                      "(prb_atmosphere_save_base)");
+    if (e->base_layers != e->atm_layers)
+        return fail(PRB_ERR_STATE, std::string(fn) + ": the base and the current column have different layer counts");
+    if (!e->bnd_tab.empty() || !e->sun_tab.empty())
+        return fail(PRB_ERR_STATE, std::string(fn) + ": a surface emissivity table or a Sun is set; the layer kernels take "
+                                                     "a black surface and no Sun (a warm top is allowed)");
+    CK(cudaSetDevice(e->device));
+    BandPlan bp;
+    if (int rc = band_plan(e, fn, n_bands, edges, e->base_range_max, bp)) return rc;
+    const int L = e->atm_layers, n_levels = L + 1;
+    const size_t per_dir = (size_t)n_bands * n_levels;
+    if (bp.strips.empty()) {                                    // an empty chunk, or no band meets it: zeros
+        if (toa_up) std::fill(toa_up, toa_up + per_dir, 0.0);
+        if (surf_down) std::fill(surf_down, surf_down + per_dir, 0.0);
+        return PRB_OK;
+    }
+    // per layer, the base's and the current column's constants; differences of temperature formed in FP64
+    const double c2 = 100 * hPlanck * cLight / kBoltz, log2e = 1.4426950408889634;
+    std::vector<KernLayer> hl(L);
+    for (int l = 0; l < L; ++l) {
+        KernLayer &k = hl[l];
+        k.depth = e->base_depth[l];
+        k.c2_over_t = (float)(c2 / e->base_t[l]);
+        k.dx2 = (float)((c2 / e->base_t[l] - c2 / e->atm_t[l]) * log2e);
+        k.x2_cur = (float)(c2 / e->atm_t[l] * log2e);
+        k.pad = 0.f;
+        for (int i = 0; i < 4; ++i) {
+            k.nd[i] = i < n_mu ? (float)(-e->base_depth[l] * log2e / mu[i]) : 0.f;
+            k.dnd[i] = i < n_mu ? (float)(-(e->atm_depth[l] - e->base_depth[l]) * log2e / mu[i]) : 0.f;
+        }
+    }
+    CK(e->kern_layers.ensure(L));
+    CK(cudaMemcpyAsync(e->kern_layers.p, hl.data(), sizeof(KernLayer) * L, cudaMemcpyHostToDevice, e->stream));
+    CK(e->band_part.ensure((size_t)2 * n_levels * bp.n_seg));
+    CK(e->band_out.ensure(2 * per_dir));
+    const int32_t *d_tab = e->band_tab.p;
+    K3KArgs up{};
+    up.base = e->base_kmat.p;
+    up.s = e->base_s.p;
+    up.layers = e->kern_layers.p;
+    for (int i = 0; i < n_mu; ++i) {
+        up.wmu[i] = (float)(weight[i] * mu[i]);
+        up.cu[i] = (float)(-log2e / mu[i]);
+    }
+    up.c2_over_ts = (float)(c2 / e->base_t_surface);
+    up.ts_dx2 = (float)((c2 / e->base_t_surface - c2 / e->atm_t_surface) * log2e);
+    up.ts_x2_cur = (float)(c2 / e->atm_t_surface * log2e);
+    up.strips = d_tab + bp.o_strips;
+    up.n_list = (int64_t)bp.strips.size();
+    up.spans = reinterpret_cast<const K3FSpan *>(d_tab);
+    up.seg_range = reinterpret_cast<const uint32_t *>(d_tab + 2 * bp.n_spans);
+    up.ld_part = bp.n_seg;
+    K3KArgs down = up;
+    up.part = e->band_part.p;
+    down.part = e->band_part.p + (size_t)n_levels * bp.n_seg;
+    down.c2_over_ttop = e->bnd_t_top > 0 ? (float)(c2 / e->bnd_t_top) : 0.f;   // the same start for both columns
+    const double dx = e->n_total > 1 ? (e->base_range_max - e->range_min) / (double)(e->n_total - 1) : 0.0;
+    const int grid = (int)std::min<int64_t>((int64_t)bp.strips.size(), k3k_minb(n_mu) * (int64_t)e->prop.multiProcessorCount);
+    cudaError_t ce;
+    switch (n_mu) {
+        case 1: ce = launch_kernel_pair<1>(e, grid, dx, up, down); break;
+        case 2: ce = launch_kernel_pair<2>(e, grid, dx, up, down); break;
+        case 3: ce = launch_kernel_pair<3>(e, grid, dx, up, down); break;
+        default: ce = launch_kernel_pair<4>(e, grid, dx, up, down); break;
+    }
+    if (ce != cudaSuccess) return fail(PRB_ERR_CUDA, std::string("k3_kernel_tma launch failed: ") + cudaGetErrorString(ce));
+    // K_b[j] = 2 pi sum_i w_i mu_i sum_{nu in band b} dI_i(nu, j) res
+    CK(band_sums(e, bp, n_levels, n_bands, 2 * 3.141592653589793 * e->res, e->band_out.p));
+    if (toa_up) CK(cudaMemcpyAsync(toa_up, e->band_out.p, sizeof(double) * per_dir, cudaMemcpyDeviceToHost, e->stream));
+    if (surf_down)
+        CK(cudaMemcpyAsync(surf_down, e->band_out.p + per_dir, sizeof(double) * per_dir, cudaMemcpyDeviceToHost, e->stream));
     CK(cudaStreamSynchronize(e->stream));
     return PRB_OK;
 }
@@ -2320,6 +2474,7 @@ extern "C" int prb_peer_alloc(prb_engine *e, int rank, int world, int64_t max_ch
     CK(cudaStreamSynchronize(e->stream));
     peer_release(e);
     e->atm_valid = false;                                       // the last column's spectra may have been in that buffer
+    e->base_valid = false;
     PeerState &ps = e->peer;
     ps.rank = rank; ps.world = world;
     ps.ld = (max_chunk_points + 63) & ~int64_t(63);
@@ -2366,6 +2521,7 @@ extern "C" int prb_peer_disconnect(prb_engine *e) {
     e->res_rad = e->res_trans = nullptr;
     e->atm_layers = 0;
     e->atm_valid = false;
+    e->base_valid = false;
     return PRB_OK;
 }
 
@@ -2785,6 +2941,7 @@ extern "C" int prb_gas_cell_host(prb_engine *e, int64_t n, const double *nu0, co
     e->grid_set = false;
     e->last.valid = false;
     e->atm_valid = false;                                       // the grid changes below, as in prb_set_grid
+    e->base_valid = false;
     int rc = alloc_line_storage(e, n);
     if (rc) return rc;
     e->n_lines = n;

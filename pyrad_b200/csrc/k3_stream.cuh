@@ -958,6 +958,276 @@ k3_flux_sum(const double *__restrict__ part, int n_parts, int n_levels, double s
     }
 }
 
+// ---- layer kernels: the change of the outgoing and surface fluxes when one layer's state is swapped ------------------
+// prb_atmosphere_save_base keeps a copy of the column (the base) and its FP64 optical depth S = sum_l k_l d_l per point;
+// prb_atmosphere_layer_kernels compares it with the current column layer by layer.  With T_l = exp(-k_l d_l / mu) and the
+// primed values those of the current column, swapping layer l alone changes the radiance leaving it by
+//   up:   dI_{l+1} = (1 - T'_l)(B'_l - B_l) + (T'_l - T_l)(I_l - B_l)        I_l the base radiance entering from below
+//   down: dI_l     = (1 - T'_l)(B'_l - B_l) + (T'_l - T_l)(I_{l+1} - B_l)    I_{l+1} the base radiance entering from above
+// and the fold is linear in what enters, so that change reaches the top (the surface) multiplied by the base
+// transmittance of the layers above (below): exp(-rem / mu), rem = S minus the depths of layer l and those before it in
+// the pass's order, formed in FP64 by subtracting k_l d_l from S layer by layer (rem is small exactly where the kernels
+// live, the top layers of an opaque band, while S itself may be 1e6).  Both differences are formed without cancellation:
+//   T'_l - T_l = T_l (2^de - 1) for small de, else T'_l - T_l directly (k3_dtrans); de = k' nd' - k nd is formed as
+//   (k' - k) nd + k' (nd' - nd), nd' - nd on the host in FP64, so neither a row change nor a depth change cancels (and
+//   de = 0 exactly for equal rows and depths);
+//   B'_l - B_l = B_l (e^(x - x') - 1) / (1 - e^-x'), x = c2 nu / T, x - x' formed on the host in FP64 (exactly 0 for
+//   equal temperatures).
+// So a layer whose row, depth and temperature are bit-identical in both columns adds exactly 0.  B_l follows the base
+// column's Planck policy (k3_planck4 above its nu_interp_min), and B'_l - B_l is interpolated the same way.  The upward
+// pass adds the surface entry exp(-S / mu)(B(T'_s) - B(T_s)) at level 0; the downward pass writes 0 there.  Sums as the
+// band pass: per point sum_i w_i mu_i (...) (a term that is not finite counts as 0), per segment of the warp's span an
+// FP32 butterfly and one FP64 store, then k3_flux_band_sum over "levels" 0..L.  No atomics.
+constexpr int K3K_LAYERS = 2;                          // layers per ring slot: two rows each (base, current), 16 KB
+constexpr int K3K_SLOTS = 2;
+
+struct KernLayer {
+    double depth;            // base depth_l (cm), for rem
+    float c2_over_t;         // base 100 h c / kB / T_l
+    float dx2;               // (c2 / T_l - c2 / T'_l) log2(e): x - x' in log2 units per cm-1
+    float x2_cur;            // c2 / T'_l log2(e)
+    float pad;
+    float nd[4];             // base -depth_l log2(e) / mu_i
+    float dnd[4];            // -(depth'_l - depth_l) log2(e) / mu_i, formed in FP64 (exactly 0 for equal depths)
+};
+
+struct K3KArgs {
+    const float *base;       // [n_layers][ld] the base k matrix
+    const double *s;         // [ld] the base optical depth
+    const KernLayer *layers;
+    float wmu[4];            // w_i mu_i
+    float cu[4];             // -log2(e) / mu_i: exp(-rem / mu_i) = 2^(rem cu[i])
+    float c2_over_ttop;      // downward pass: 100 h c / kB / T_top; 0: I = 0 at level L
+    float c2_over_ts;        // upward pass, the surface: base 100 h c / kB / T_s
+    float ts_dx2, ts_x2_cur; // ... and its dx2, x2_cur as KernLayer's
+    double *part;            // [n_levels][ld_part] per-segment sums of the pass
+    const int32_t *strips;   // the n_list strips that meet a band, ascending
+    int64_t n_list;
+    const K3FSpan *spans;    // as K3FArgs
+    const uint32_t *seg_range;
+    int64_t ld_part;
+};
+
+struct K3KSmem {
+    float k[K3K_SLOTS][K3K_LAYERS][2][K3T_STRIP];
+    uint64_t full[K3K_SLOTS];
+};
+
+// Resident CTAs per SM the registers allow without spills (-Xptxas -v, 256 threads): one node fits 80 registers
+// (3 CTAs), two to four take 116-123 (2 CTAs; two nodes spill at 80).
+__host__ __device__ constexpr int k3k_minb(int nmu) { return nmu == 1 ? 3 : 2; }
+
+// 2^e - 1 to a few FP32 ulp relative: the fold's five-term series below |e| = 1/8 (exactly 0 at e = 0), else ex2 - 1.
+__device__ __forceinline__ float k3_exp2m1(float e) {
+    float p = fmaf(e, 1.3333558146e-3f, 9.6181291076e-3f);
+    p = fmaf(e, p, 5.5504108665e-2f);
+    p = fmaf(e, p, 2.4022650696e-1f);
+    p = fmaf(e, p, 6.9314718056e-1f);
+    return fabsf(e) < 0.125f ? e * p : k3_ex2(e) - 1.0f;
+}
+
+// T' - T = 2^(e + de) - 2^e: 2^e (2^de - 1) by the series below |de| = 1/8 (exactly 0 at de = 0), else the plain
+// difference, which cancels little there and stays finite where 2^e underflows and 2^de overflows (an opaque layer).
+__device__ __forceinline__ float k3_dtrans(float e, float de) {
+    float p = fmaf(de, 1.3333558146e-3f, 9.6181291076e-3f);
+    p = fmaf(de, p, 5.5504108665e-2f);
+    p = fmaf(de, p, 2.4022650696e-1f);
+    p = fmaf(de, p, 6.9314718056e-1f);
+    return fabsf(de) < 0.125f ? k3_ex2(e) * (de * p) : k3_ex2(e + de) - k3_ex2(e);
+}
+
+// B(T') - B(T) from b = B(T): b (e^(x - x') - 1) / (1 - e^-x'), with dx2 = (x - x') log2(e), x2c = x' log2(e).
+__device__ __forceinline__ float k3_dplanck(float b, float x2c, float dx2) {
+    return b * k3_exp2m1(dx2) / -k3_exp2m1(-x2c);
+}
+
+template <int NMU, bool DOWN>
+__global__ void __launch_bounds__(K3T_THREADS, k3k_minb(NMU))
+k3_kernel_tma(const float *__restrict__ kmat, int64_t ld, int n_layers, int64_t n_chunk, int64_t i_begin, int64_t n_total,
+              double x0, double dx, double x_last, float nu_interp_min, const K3KArgs a) {
+    extern __shared__ __align__(128) unsigned char k3_smem_raw[];
+    K3KSmem &sm = *reinterpret_cast<K3KSmem *>(k3_smem_raw);
+    const int tid = threadIdx.x, lane = tid & 31;
+    const int groups = (n_layers + K3K_LAYERS - 1) / K3K_LAYERS;
+    const int64_t my_strips = blockIdx.x < a.n_list ? (a.n_list - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
+    const int64_t n_steps = my_strips * groups;
+    if (tid == 0) {
+        for (int s = 0; s < K3K_SLOTS; ++s) mbar_init(&sm.full[s], 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    }
+    __syncthreads();
+    auto group_of = [&](int64_t step) { const int g = (int)(step % groups); return DOWN ? groups - 1 - g : g; };
+    auto strip_of = [&](int64_t step) { return (int64_t)a.strips[blockIdx.x + (step / groups) * gridDim.x]; };
+    auto issue = [&](int64_t step) {                   // thread 0 only: both rows of every layer of the group
+        const int slot = (int)(step % K3K_SLOTS);
+        const int g = group_of(step);
+        const int64_t p0 = strip_of(step) * K3T_STRIP;
+        const int64_t pts = min((int64_t)K3T_STRIP, ((n_chunk - p0) + 3) & ~int64_t(3));
+        const int rows = min(K3K_LAYERS, n_layers - g * K3K_LAYERS);
+        mbar_expect_tx(&sm.full[slot], (uint32_t)(2 * rows * pts * 4));
+        for (int r = 0; r < rows; ++r) {
+            const int64_t off = (int64_t)(g * K3K_LAYERS + r) * ld + p0;
+            tma_bulk_g2s(sm.k[slot][r][0], a.base + off, (uint32_t)(pts * 4), &sm.full[slot]);
+            tma_bulk_g2s(sm.k[slot][r][1], kmat + off, (uint32_t)(pts * 4), &sm.full[slot]);
+        }
+    };
+    if (tid == 0)
+        for (int64_t s = 0; s < min(n_steps, (int64_t)(K3K_SLOTS - 1)); ++s) issue(s);
+
+    float nu[4], a3[4], rad[NMU][4];
+    double rem[4];
+    bool interp = false;
+    int n_valid = 0;
+    int64_t i0 = 0;
+    // the per-point values v of one level into its segments: a masked FP32 sum per segment, an xor butterfly, one FP64
+    // store by lane 0 (points outside the chunk hold v = 0)
+    auto seg_add = [&](const float (&v)[4], int level) {
+        const K3FSpan sp = a.spans[i0 >> 7];
+        if (sp.nseg == 0) return;
+        const int nseg = sp.nseg < 0 ? 1 : sp.nseg;
+        double *dst = a.part + (int64_t)level * a.ld_part + sp.seg0;
+        for (int s = 0; s < nseg; s += 2) {
+            const uint32_t r0 = sp.nseg < 0 ? 128u << 16 : a.seg_range[sp.seg0 + s];
+            const uint32_t r1 = s + 1 < nseg ? a.seg_range[sp.seg0 + s + 1] : 0u;
+            float t0 = 0.f, t1 = 0.f;
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+                const uint32_t p = 4 * lane + q;
+                if (p >= (r0 & 0xffffu) && p < (r0 >> 16)) t0 += v[q];
+                if (p >= (r1 & 0xffffu) && p < (r1 >> 16)) t1 += v[q];
+            }
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) {
+                t0 += __shfl_xor_sync(0xffffffffu, t0, o);
+                t1 += __shfl_xor_sync(0xffffffffu, t1, o);
+            }
+            if (lane == 0) {
+                dst[s] = (double)t0;
+                if (s + 1 < nseg) dst[s + 1] = (double)t1;
+            }
+        }
+    };
+    for (int64_t step = 0; step < n_steps; ++step) {
+        const int slot = (int)(step % K3K_SLOTS);
+        const int g = group_of(step);
+        if (step % groups == 0) {                      // a new strip: the boundary radiance of the pass, rem = S
+            i0 = strip_of(step) * K3T_STRIP + 4 * tid;
+            n_valid = (int)max((int64_t)0, min((int64_t)4, n_chunk - i0));
+            float v[4];
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+                const double x = axis_value(i_begin + i0 + q, n_total, x0, dx, x_last);
+                nu[q] = (float)x;
+                a3[q] = (float)(2E8 * hPlanck * (cLight * cLight) * (x * x * x));
+                rem[q] = q < n_valid ? a.s[i0 + q] : 0.0;
+                float r0 = 0.f;
+                if (!DOWN) r0 = planck_f32(a3[q], a.c2_over_ts * nu[q]);
+                else if (a.c2_over_ttop > 0.f) r0 = planck_f32(a3[q], a.c2_over_ttop * nu[q]);
+#pragma unroll
+                for (int i = 0; i < NMU; ++i) rad[i][q] = r0;
+                v[q] = 0.f;
+                if (!DOWN && q < n_valid) {            // the surface entry: exp(-S / mu_i) (B(T'_s) - B(T_s))
+                    const float db = k3_dplanck(r0, a.ts_x2_cur * nu[q], a.ts_dx2 * nu[q]);
+                    const float rf = (float)rem[q];
+#pragma unroll
+                    for (int i = 0; i < NMU; ++i) {
+                        const float c = k3_ex2(rf * a.cu[i]) * db;
+                        if (isfinite(c)) v[q] = fmaf(a.wmu[i], c, v[q]);
+                    }
+                }
+            }
+            interp = nu[0] >= nu_interp_min;
+            seg_add(v, 0);
+        }
+        if (tid == 0 && step + K3K_SLOTS - 1 < n_steps) issue(step + K3K_SLOTS - 1);
+        mbar_wait(&sm.full[slot], (uint32_t)((step / K3K_SLOTS) & 1));
+        const int rows = min(K3K_LAYERS, n_layers - g * K3K_LAYERS);
+#pragma unroll
+        for (int rr = 0; rr < K3K_LAYERS; ++rr) {
+            if (rr < rows) {
+                const int r = DOWN ? rows - 1 - rr : rr;
+                const int l = g * K3K_LAYERS + r;
+                // the rows are read from shared memory again for every node: held in registers they spill
+                const float4 *kb4 = reinterpret_cast<const float4 *>(&sm.k[slot][r][0][4 * tid]);
+                const float4 *kc4 = reinterpret_cast<const float4 *>(&sm.k[slot][r][1][4 * tid]);
+                const KernLayer &fl = a.layers[l];
+                float b[4], db[4], v[4];
+                k3_planck4(nu, a3, fl.c2_over_t, interp, b);
+                if (interp) {                          // B' - B at the first and last point, linear between
+                    const float da = k3_dplanck(b[0], fl.x2_cur * nu[0], fl.dx2 * nu[0]);
+                    const float dd = k3_dplanck(b[3], fl.x2_cur * nu[3], fl.dx2 * nu[3]);
+                    const float d = dd - da;
+                    db[0] = da; db[1] = fmaf(d, 1.0f / 3.0f, da); db[2] = fmaf(d, 2.0f / 3.0f, da); db[3] = dd;
+                } else {
+#pragma unroll
+                    for (int q = 0; q < 4; ++q) db[q] = k3_dplanck(b[q], fl.x2_cur * nu[q], fl.dx2 * nu[q]);
+                }
+                {
+                    const float4 k4 = *kb4;
+                    const double d = fl.depth;
+                    rem[0] = fma(-(double)k4.x, d, rem[0]); rem[1] = fma(-(double)k4.y, d, rem[1]);
+                    rem[2] = fma(-(double)k4.z, d, rem[2]); rem[3] = fma(-(double)k4.w, d, rem[3]);
+                }
+#pragma unroll
+                for (int q = 0; q < 4; ++q) v[q] = 0.f;
+#pragma unroll
+                for (int i = 0; i < NMU; ++i) {
+                    const float4 kb4i = *kb4, kc4i = *kc4;
+                    const float kb[4] = {kb4i.x, kb4i.y, kb4i.z, kb4i.w}, kc[4] = {kc4i.x, kc4i.y, kc4i.z, kc4i.w};
+#pragma unroll
+                    for (int q = 0; q < 4; ++q) {
+                        const float e = kb[q] * fl.nd[i];
+                        const float de = fmaf(kc[q] - kb[q], fl.nd[i], kc[q] * fl.dnd[i]);  // k' nd' - k nd
+                        const float dt = k3_dtrans(e, de);                                  // T' - T
+                        const float di = fmaf(-k3_exp2m1(e + de), db[q], dt * (rad[i][q] - b[q]));
+                        const float c = k3_ex2((float)rem[q] * a.cu[i]) * di;
+                        if (q < n_valid && isfinite(c)) v[q] = fmaf(a.wmu[i], c, v[q]);
+                    }
+                    const float2 nd = make_float2(fl.nd[i], fl.nd[i]);
+                    const float2 e01 = __fmul2_rn(make_float2(kb[0], kb[1]), nd), e23 = __fmul2_rn(make_float2(kb[2], kb[3]), nd);
+                    const float2 r01 = k3_fold_step2(make_float2(rad[i][0], rad[i][1]), e01, make_float2(b[0], b[1]));
+                    const float2 r23 = k3_fold_step2(make_float2(rad[i][2], rad[i][3]), e23, make_float2(b[2], b[3]));
+                    rad[i][0] = r01.x; rad[i][1] = r01.y; rad[i][2] = r23.x; rad[i][3] = r23.y;
+                }
+                seg_add(v, l + 1);
+            }
+        }
+        __syncthreads();                               // every thread is done with this slot: it may be refilled
+    }
+}
+
+// The base of the layer kernels: base = kmat row by row (streaming), and s[i] = sum_l k_l(i) depth_l in FP64, layer
+// order, over all ld points of a row (the padding too, so the kernel passes may read any point of a float4).
+__global__ void __launch_bounds__(256)
+k3_kernel_base(const float *__restrict__ kmat, float *__restrict__ base, int64_t ld, int n_layers,
+               const double *__restrict__ depth, double *__restrict__ s) {
+    const int64_t nvec = ld >> 2;
+    for (int64_t v = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; v < nvec; v += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t i0 = v << 2;
+        double acc[4] = {0.0, 0.0, 0.0, 0.0};
+        for (int l0 = 0; l0 < n_layers; l0 += K3_UNROLL) {
+            float4 k4[K3_UNROLL];
+#pragma unroll
+            for (int j = 0; j < K3_UNROLL; ++j)
+                if (l0 + j < n_layers) k4[j] = __ldcs(reinterpret_cast<const float4 *>(kmat + (int64_t)(l0 + j) * ld + i0));
+#pragma unroll
+            for (int j = 0; j < K3_UNROLL; ++j) {
+                if (l0 + j < n_layers) {
+                    __stcs(reinterpret_cast<float4 *>(base + (int64_t)(l0 + j) * ld + i0), k4[j]);
+                    const double d = depth[l0 + j];
+                    acc[0] = fma((double)k4[j].x, d, acc[0]);
+                    acc[1] = fma((double)k4[j].y, d, acc[1]);
+                    acc[2] = fma((double)k4[j].z, d, acc[2]);
+                    acc[3] = fma((double)k4[j].w, d, acc[3]);
+                }
+            }
+        }
+        *reinterpret_cast<double2 *>(s + i0) = make_double2(acc[0], acc[1]);
+        *reinterpret_cast<double2 *>(s + i0 + 2) = make_double2(acc[2], acc[3]);
+    }
+}
+
 // ---- cross-GPU completion barrier of one gather step ------------------------------------------------
 // Launched (one warp) after the kernel that stored this rank's spectra into every peer's gather buffer.
 // Lane p publishes "rank r finished epoch E" into peer p's flag block with a system-scope release, then

@@ -597,6 +597,32 @@ class Engine:
                                                         _dp(up) if up.size else None, _dp(down) if down.size else None))
         return up, down
 
+    def save_column_base(self):
+        """Keep the last column as the base of atmosphere_layer_kernels (prb_atmosphere_save_base): a device copy of its
+        k matrix and layer state, and its FP64 optical depth per point.  A grid change drops it; atmosphere keeps it."""
+        _lib.check(self._lib.prb_atmosphere_save_base(self._h))
+
+    def atmosphere_layer_kernels(self, mu, weights, edges):
+        """Radiative kernels of the saved base column against the last column (prb_atmosphere_layer_kernels): for the
+        quadrature (mu, weights) and the bands edges[b] <= nu < edges[b+1] (as atmosphere_band_fluxes), returns
+        (toa_up, surf_down), float64 W m-2 of shape (n_bands, L+1), this chunk's share.  Entry l+1 is the exact change of
+        the upward flux at the top (the downward flux at the surface) when layer l alone of the base takes the last
+        column's state; toa_up[:, 0] is the surface temperature's entry, surf_down[:, 0] is 0.  The kernels shard like
+        the fluxes: distributed.sum_over_ranks adds the ranks' shares."""
+        m, w, ed = _f64(np.atleast_1d(mu)), _f64(np.atleast_1d(weights)), _f64(np.atleast_1d(edges))
+        if m.ndim != 1 or m.shape != w.shape or not 1 <= m.size <= 4:
+            raise ValueError("atmosphere_layer_kernels: mu and weights must be 1-d arrays of one length, 1 to 4 nodes")
+        if not (np.all(m > 0) and np.all(m <= 1) and np.all(np.isfinite(w)) and np.all(w > 0)):
+            raise ValueError("atmosphere_layer_kernels: every mu must lie in (0, 1] and every weight be finite and > 0")
+        if ed.ndim != 1 or ed.size < 2 or not np.all(np.isfinite(ed)) or not np.all(np.diff(ed) > 0):
+            raise ValueError("atmosphere_layer_kernels: edges must be a 1-d array of at least 2 finite, strictly ascending "
+                             "values")
+        L = int(getattr(self, "atm_layers", 0))
+        up, down = np.zeros((ed.size - 1, L + 1)), np.zeros((ed.size - 1, L + 1))
+        _lib.check(self._lib.prb_atmosphere_layer_kernels(self._h, m.size, _dp(m), _dp(w), ed.size - 1, _dp(ed), _dp(up),
+                                                          _dp(down)))
+        return up, down
+
     def set_flux_boundaries(self, emissivity=None, reflection="lambertian", t_top=0.0):
         """The surface and top boundaries of every later atmosphere_fluxes / atmosphere_band_fluxes call
         (prb_set_flux_boundaries; arguments as flux_boundary_args).  The surface emits eps(nu) B(nu, T_surface) and

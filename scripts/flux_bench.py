@@ -19,7 +19,10 @@ without it.  Last, a water-vapour continuum (prb_set_continuum) from a SYNTHETIC
 log-uniform coefficients, not MT_CKD's values) with cfg4's H2O profile: the column itself (prb_atmosphere) timed five
 times without and five times with it, alternating, the median difference against the add kernel's algorithmic bytes
 (the k matrix read and written once, 2 L N 4) and the copy bandwidth, and the change it makes to the OLR, the surface
-down flux and RRTMG's 16 band fluxes (3 nodes).  Prints one JSON line; writes nothing.
+down flux and RRTMG's 16 band fluxes (3 nodes).  Last, the layer kernels: prb_atmosphere_save_base on the plain column and
+prb_atmosphere_layer_kernels (3 nodes, RRTMG's 16 bands) against a column 1 K warmer, each as a ratio to the 16-band
+flux call timed right before it, and the OLR temperature kernel's column sum beside the OLR difference of the two
+columns (they differ by the layers' non-additivity).  Prints one JSON line; writes nothing.
 
     python scripts/flux_bench.py [--reps 30] [--warmup 3]
 """
@@ -149,6 +152,44 @@ def continuum_section(e, stream, w, column, mu, wt, rrtmg, copy_bytes_per_s, run
             "band_surface_down_change_w_m2": [float(v) for v in wet_f[3][:, 0] - dry_f[3][:, 0]]}
 
 
+def kernels_section(e, stream, args, w, column, mu, wt, rrtmg):
+    """prb_atmosphere_save_base and prb_atmosphere_layer_kernels (3 nodes, RRTMG's 16 bands) on the plain column and a
+    column 1 K warmer in every layer and at the surface, each timed as a ratio to the 16-band flux call timed right before
+    it; then the OLR temperature kernel's column sum beside the OLR difference of the two columns."""
+    from pyrad_b200 import engine as eng
+    sp = w["species"]
+    win = [eng.window_len(c, w["res"]) for c in w["cutoff"]]
+    t_warm = np.asarray(w["T"]) + 1.0
+    warm = e.atmosphere_call(w["depth_cm"], t_warm, w["P"], w["conc"], [s.molmass for s in sp],
+                             np.array([[s.q(T) for s in sp] for T in t_warm]), [s.q296 for s in sp], win,
+                             w["t_surface"] + 1.0, w["range_max"])
+    band = lambda: e.atmosphere_band_fluxes(mu, wt, rrtmg)                      # noqa: E731
+    column()
+    up0, _ = e.atmosphere_fluxes(mu, wt)
+
+    def stats(ms):
+        return {"ms_median": float(np.median(ms)), "ms_p10_p90": [float(np.percentile(ms, 10)),
+                                                                  float(np.percentile(ms, 90))], "reps": args.reps}
+    band_a = stats(timed(stream, band, args.warmup, args.reps))
+    save = stats(timed(stream, e.save_column_base, args.warmup, args.reps))
+    warm()
+    up1, _ = e.atmosphere_fluxes(mu, wt)
+    band_b = stats(timed(stream, band, args.warmup, args.reps))
+    kern = stats(timed(stream, lambda: e.atmosphere_layer_kernels(mu, wt, rrtmg), args.warmup, args.reps))
+    toa, sfc = e.atmosphere_layer_kernels(mu, wt, rrtmg)
+    out = {"n_mu": 3, "bands": "rrtmg_lw_16", "perturbation": "+1 K in every layer and at the surface",
+           "band_call_before_save": band_a, "save_base": save,
+           "save_base_ratio_to_band_call": save["ms_median"] / band_a["ms_median"],
+           "band_call_before_kernels": band_b, "layer_kernels": kern,
+           "layer_kernels_ratio_to_band_call": kern["ms_median"] / band_b["ms_median"],
+           "olr_kernel_column_sum_w_m2": float(toa.sum()),
+           "olr_kernel_layers_w_m2": float(toa[:, 1:].sum()), "olr_kernel_surface_w_m2": float(toa[:, 0].sum()),
+           "olr_difference_of_the_columns_w_m2": float(up1[-1] - up0[-1]),
+           "surface_down_kernel_column_sum_w_m2": float(sfc.sum())}
+    column()
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--reps", type=int, default=30)
@@ -240,6 +281,7 @@ def main():
         e.set_flux_boundaries()
     out["solar"] = solar_section(e, stream, args, w, mu, wt, calls, eps_table)
     out["continuum"] = continuum_section(e, stream, w, column, mu, wt, rrtmg, peaks["copy_bytes_per_s"])
+    out["kernels"] = kernels_section(e, stream, args, w, column, mu, wt, rrtmg)
     e.close()
     print(json.dumps(out))
 
